@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one rank per GPU under torchrun)
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU path (oracle port), host cores
+    python bench.py --steps K --warmup W --dump-outputs bench_outputs   # + heights of the last timed step, .npy
 
 Headline metric (BASELINE.json): height-scan rays/s on cfg-2 -- 4096 envs x 961 rays per GPU on the synthetic
 200 m x 200 m / 2,000,000-triangle terrain.  A "step" is one height-scan pass over one batch of synthetic poses.
@@ -180,6 +181,14 @@ def time_steps(fn, steps, warmup, flush, stream):
     return np.array([a.elapsed_time(b) for a, b in ev])
 
 
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write each tensor as ``out_dir/<name>.npy`` (float32), so that two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.float().cpu().numpy())
+    log(f"outputs of the last timed step written to {out_dir}: {sorted(arrays)}")
+
+
 def guarded(name, out: dict, fn):
     """The headline number must survive a failure of the additional measurements."""
     try:
@@ -241,12 +250,15 @@ def run_ours(args):
     torch.cuda.synchronize()
     with ClockSampler(local) as clocks:
         ms = time_steps(scan_step, args.steps, max(args.warmup, 3), flush, stream)  # never fewer than 3 untimed steps
+        last_heights = out.clone() if args.dump_outputs else None  # the loop below overwrites `out`
         t_end = time.time() + 0.3  # keep the GPU busy long enough for a few clock samples
         while time.time() < t_end:
             scan_step(0)
         torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"height_scan": last_heights})
     total_ms = max_over_ranks([ms.sum()])[0]
     value = n_scan * N_RAYS * args.steps * world / (total_ms * 1e-3)
     t_launch = float(ms.mean()) * 1e-3
@@ -819,8 +831,8 @@ def cpu_reference(v, f, steps, warmup, n_envs, budget_s=None):
 
 def cpu_full_step(v, f, tables, mesh=None, warmup=20, steps=30):
     """cfg-1 (BASELINE.json configs[0], BASELINE.md section 3): one whole non-physics step of AAURoverEnv-v0 at 256 envs on
-    the host cores -- the reference's term functions as restated by the oracle (bit-identical to the imported reference:
-    tests/test_oracle_golden.py::test_live_reference_agrees_bitwise) + the raycast port; >= 20 warm-up + >= 30 timed steps
+    the host cores -- the reference's term functions as restated by the oracle (bit-identical to the reference's outputs:
+    tests/test_oracle_golden.py::test_reference_golden_agrees_bitwise) + the raycast port; >= 20 warm-up + >= 30 timed steps
     (SURVEY.md 8d "CPU baseline timing")."""
     from isaac_rover_orbit_b200 import synthetic
     from oracle import raycast as oracle_raycast
@@ -926,7 +938,13 @@ def main():
     ap.add_argument("--no-cfg1", action="store_true", help="reference arm: skip the cfg-1 full-step leg")
     ap.add_argument("--no-graph", action="store_true", help="launch the fused step kernel by kernel instead of replaying CUDA graphs")
     ap.add_argument("--init-on-cpu", action="store_true", help="build the init-time tables on the host (profiling)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the heights of the last timed height-scan step (rank 0, 4096 x 961 "
+                         "float32, -inf where a ray misses) as DIR/height_scan.npy; the poses are seeded, so runs with the "
+                         "same arguments scan the same inputs")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,13 +1,11 @@
 """TEST INFRASTRUCTURE ONLY -- CPU (torch, fp32) restatement of the reference's MDP term math.
 
 Every function takes plain tensors (no ``env`` object) and cites the reference lines it follows.
-Paths are relative to ``/root/reference``.  The restatement is pinned in two ways
-(``tests/test_oracle_golden.py::test_live_reference_agrees_bitwise`` / ``tests/golden/make_golden.py``):
-
-* in the build container the UNMODIFIED reference functions are imported through
-  :mod:`oracle.ref_loader` and must agree bit-for-bit with these on seeded inputs;
-* the outputs of the imported reference are committed as fixtures under ``tests/golden/`` so the
-  same check runs where ``/root/reference`` does not exist (the GPU box).
+Paths are relative to the reference's source tree.  The restatement is pinned by
+``tests/golden/make_golden.py``: it imports the UNMODIFIED reference functions through
+:mod:`oracle.ref_loader`, runs them on seeded inputs and commits their outputs as fixtures under
+``tests/golden/``, which these functions must reproduce bit for bit
+(``tests/test_oracle_golden.py::test_reference_golden_agrees_bitwise``).
 
 Only ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py``'s CPU-baseline / ``--impl reference``
 legs may import this module.  The product package never does.

@@ -28,21 +28,6 @@ def test_trainer_call_trace_equals_reference(golden_calls, name, mode, steps, he
     assert json.loads(json.dumps(log)) == golden_calls[name]  # same calls, order, arguments and tensor checksums
 
 
-def test_trainer_matches_reference_live():
-    """When the reference tree is present (build container), drive both trainers side by side."""
-    from oracle import ref_loader
-
-    if not ref_loader.available():
-        pytest.skip("reference tree not mounted")
-    ref = ref_loader.load("skrl_utils")
-    for mode in ("train", "eval"):
-        a, b = [], []
-        cfg = {"timesteps": 7, "disable_progressbar": True, "headless": True}
-        getattr(ref.SkrlSequentialLogTrainer(env=FakeEnv(a, 5), agents=FakeAgent(a), cfg=dict(cfg)), mode)()
-        getattr(SkrlSequentialLogTrainer(env=FakeEnv(b, 5), agents=FakeAgent(b), cfg=dict(cfg)), mode)()
-        assert a == b
-
-
 def test_log_episode_info_can_be_skipped():
     log = []
     SkrlSequentialLogTrainer(env=FakeEnv(log), agents=FakeAgent(log), cfg={"timesteps": 4}, log_episode_info=False).train()
