@@ -190,9 +190,8 @@ height_scan_paired_kernel(const float* __restrict__ pos_w, const float* __restri
     } else {
         // =============================== consumers ===============================
         // Work units (environment, chunk): chunk K of the CTA's run goes to warp K mod 15 (static deal).  With
-        // ROVER_PAIR_DYNAMIC they are handed out in order from a shared counter instead; the phase-aliasing argument above
-        // holds either way (at most 15 units are outstanding, so when a warp holds a chunk of environment E at least 17
-        // chunks of E-8 .. E-1 are finished, i.e. E-8 was issued and E-16 consumed).
+        // ROVER_PAIR_DYNAMIC they are handed out in order from a shared counter instead; the phase-aliasing argument in
+        // scan_paired.cuh holds either way.
 #if ROVER_PAIR_DYNAMIC
         int it = 0, c = 0;
         auto next_unit = [&]() {

@@ -29,6 +29,7 @@ constexpr int kStepMdpWarps = 4;      // batches of 32 envs are dealt to them ro
 constexpr int kStepThreads = 32 * (1 + kStepWorkerWarps);
 constexpr int kStepLead = 96;         // an MDP batch is started when the scan front is within this many envs of it
 static_assert(kStepThreads == 512, "16 warps x 128 registers = the register file");
+static_assert(kPairFullBars >= kStepWorkerWarps + kPairStages, "full barriers: phase-aliasing note in scan_paired.cuh");
 
 struct StepSmem {
     PairStage stage[kPairStages];

@@ -54,7 +54,7 @@ constexpr int kPairStages = 8;          // ring depth (data)
 #define ROVER_PAIR_EARLY 8
 #endif
 constexpr int kPairEarly = ROVER_PAIR_EARLY;  // windows whose TMA load is issued in the prologue (<= kPairStages)
-constexpr int kPairFullBars = 16;       // `full` barriers: two per stage, see the note on phase aliasing below
+constexpr int kPairFullBars = 32;       // `full` barriers: four per stage, see the note on phase aliasing below
 constexpr int kPairWin = 26;            // window cells per axis
 constexpr int kPairPitch = 27;          // cells per staged row: odd, so that consecutive rows shift by one 16-byte bank
                                         // group and a quarter-warp's LDS.128 of 8 neighbouring cells is conflict free
@@ -127,13 +127,18 @@ struct PairSmem {
     unsigned long long empty_bar[kPairStages];
     int next_chunk;  // dynamic hand-out of (environment, chunk) work units, in order
 };
-// Phase aliasing: a consumer warp visits only every 3rd..4th environment, so it may reach environment E while the
-// TMA load of E - 8 (same stage) is still in flight (loads complete out of order); with one `full` barrier per stage
-// its parity wait would then be satisfied by the phase of E - 16.  Environment E therefore signals on barrier E % 16
-// with parity (E / 16) & 1: the warp's previous chunk (environment >= E - 4) was issued after E - 8, which was issued
-// after E - 16 had been consumed (the producer issues strictly in order), so the barrier is never more than one phase
-// behind the waiter.
-static_assert(kPairFullBars == 2 * kPairStages, "full barriers: two per stage");
+// Phase aliasing: a consumer warp does not visit every environment, so it may reach environment E while the TMA load
+// of an earlier environment on the same barrier is still in flight (loads complete out of order, and an environment
+// whose window is not staged completes its barrier as soon as the header is published); a parity wait on a barrier
+// two phases behind would pass on a stale phase.  Environment E therefore signals on barrier E % F with parity
+// (E / F) & 1, F = kPairFullBars, and the wait is sound when E - F has completed.  With W = 15 consumer warps and
+// S = 8 stages: the warp's previous work unit is at most W units back, so its environment is >= E - W (one chunk per
+// environment, <= 256 rays, is the worst case); that environment was issued, the producer issues strictly in order
+// and issues environment X only after X - S was consumed, so every environment <= E - W - S was consumed.  F >= W + S
+// makes E - F one of them.  (F = 16 held only at >= 2 chunks per environment.)  The same bound holds for a dynamic
+// hand-out: of the W units handed out just before E's, at most W - 1 can still be held by the other warps.  Environments
+// E < F wait on a barrier's first phase, which only their own arrivals complete.
+static_assert(kPairFullBars >= kPairConsumerWarps + kPairStages, "full barriers: see the phase-aliasing note");
 
 static_assert(sizeof(PairSmem) <= 227 * 1024, "PairSmem exceeds the shared memory of one SM");
 __device__ __forceinline__ float sm_vz(const PairSmem& sm, int slot) { return sm.vz[slot]; }

@@ -14,7 +14,7 @@ import torch
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
 sys.path.insert(0, os.path.dirname(__file__))
 
-import scan_emulation as SE  # noqa: E402
+import scan_exact as SE  # noqa: E402
 
 from isaac_rover_orbit_b200 import _lib, ops  # noqa: E402
 from isaac_rover_orbit_b200 import terrain as TR  # noqa: E402
