@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define ROVER_B200_ABI_VERSION 3
+#define ROVER_B200_ABI_VERSION 4
 #define ROVER_MAX_LEVELS 12
 #define ROVER_NUM_REWARD_TERMS 7
 #define ROVER_NUM_TERMINATION_TERMS 4
@@ -91,6 +91,23 @@ int rover_height_scan(const float* pos_w, const float* quat_w, int32_t n_envs, c
                       int32_t n_rays, const float* pattern_box /* host */, const RoverScanGrid* grid /* host */,
                       const RoverPlaneCells* cells /* host */, float max_distance, float base_offset,
                       float* out_heights, int32_t out_stride, float* out_hits_w, int32_t variant, void* stream);
+
+/* The height scan with rays in any direction: ORBIT RayCasterCfg.attach_yaw_only and GridPatternCfg.direction honoured.
+ * Replaces the same reference lines as rover_height_scan (rover_env_cfg.py:78-86 + observations.py:35-45, via ORBIT
+ * RayCaster._update_buffers_impl), both branches of the frame:
+ *   attach_yaw_only != 0: starts_w = quat_apply_yaw(q, starts) + p (the vertical kernels' starts bit for bit), dirs_w = dirs;
+ *   attach_yaw_only == 0: starts_w = quat_apply(q, starts) + p, dirs_w = quat_apply(q, dirs), q as given (not normalised).
+ * ray_dirs_local [n_rays,3]: per-ray directions, used as given (not normalised): the hit is the first P(t) = S + t * D on
+ * the mesh with 0 <= t < max_distance, t in units of |D|; D == 0 misses.  Surfaces are double-sided.
+ * out_heights / out_hits_w / out_stride / base_offset as in rover_height_scan (hit = S + t * D, one rounding per component;
+ * a miss is -inf / +inf).  For D = (0, 0, -1) with attach_yaw_only the result equals variant 2 bit for bit.
+ * cells is required, and grid must hold the home grid when the table has general cells (the rule of variant 2).
+ * Deviation: faces with zero XY area (vertical walls) are in neither table, so a tilted ray passes through them where
+ * mesh_query_ray would hit (DESIGN.md section 2, (iii)); DEM lattices have no such faces. */
+int rover_ray_cast(const float* pos_w, const float* quat_w, int32_t n_envs, const float* ray_starts_local,
+                   const float* ray_dirs_local, int32_t n_rays, int32_t attach_yaw_only, const RoverScanGrid* grid /* host */,
+                   const RoverPlaneCells* cells /* host */, float max_distance, float base_offset, float* out_heights,
+                   int32_t out_stride, float* out_hits_w, void* stream);
 
 /* The height scan for a caller whose poses and heights live in HOST memory (a CPU-side simulator; bench.py's `e2e`):
  * pos_host [n_envs,3], quat_host [n_envs,4] and out_host [n_envs,out_stride] are host pointers (page-locked for the

@@ -67,7 +67,8 @@ class RayCaster:
     def __init__(self, env, cfg):
         self.cfg = cfg
         self._env = env
-        self.ray_pattern = ops.RayPattern.grid(env.device, cfg.pattern_cfg.resolution, cfg.pattern_cfg.size, cfg.offset_pos)
+        self.ray_pattern = ops.RayPattern.grid(env.device, cfg.pattern_cfg.resolution, cfg.pattern_cfg.size, cfg.offset_pos,
+                                               direction=cfg.pattern_cfg.direction)
         self.ray_starts = self.ray_pattern.starts
         outer = self
 
@@ -85,7 +86,7 @@ class RayCaster:
                 robot = outer._env.scene["robot"].data
                 _, hits = ops.height_scan(robot.root_pos_w, robot.root_quat_w, outer.ray_pattern, outer._env.scan_grid,
                                           outer.cfg.max_distance, outer._env.cfg.height_scan_base_offset,
-                                          return_hits=True)
+                                          return_hits=True, attach_yaw_only=outer.cfg.attach_yaw_only)
                 return hits
 
         self.data = _SensorData()
@@ -303,7 +304,8 @@ class RoverEnv:
         robot = self.scene["robot"].data
         sensor = self.scene.sensors["height_scanner"]
         ops.height_scan(robot.root_pos_w, robot.root_quat_w, sensor.ray_pattern, self.scan_grid,
-                        sensor.cfg.max_distance, self.cfg.height_scan_base_offset, out=self.obs_buf[:, 4:])
+                        sensor.cfg.max_distance, self.cfg.height_scan_base_offset, out=self.obs_buf[:, 4:],
+                        attach_yaw_only=sensor.cfg.attach_yaw_only)
 
     def episode_log(self) -> dict:
         """Host-side copy of the last episode log (synchronises): the values of ``extras["log"]`` + ``num_resets``."""

@@ -123,13 +123,34 @@ def grid_pattern(resolution: float = 0.1, size=(3.0, 3.0), offset_pos=(0.0, 0.0,
 
 
 class RayPattern:
-    """ORBIT ``RayCaster.ray_starts`` on the device + its host-side bounding box (the staged kernel's window)."""
+    """ORBIT ``RayCaster.ray_starts`` / ``ray_directions`` on the device + the starts' host-side bounding box (the staged
+    kernel's window).  ``directions``: ``[R,3]``, or one ``[3]`` row for every ray; default (0, 0, -1).  Directions are
+    used as given (not normalised): the hit is the first ``S + t * D`` with ``0 <= t < max_distance``.
+    ``vertical_down``: every direction is exactly (0, 0, -1) -- the configuration of the vertical kernels."""
 
-    def __init__(self, ray_starts_local: torch.Tensor, device):
+    def __init__(self, ray_starts_local: torch.Tensor, device, directions=None):
         cpu = ray_starts_local.detach().to("cpu", torch.float32).contiguous()
+        if cpu.dim() != 2 or cpu.shape[1] != 3:
+            raise RuntimeError(f"RayPattern: starts must be [R,3], got {list(cpu.shape)}")
         self.n_rays = cpu.shape[0]
         self.device = torch.device(device)
         self.starts = cpu.to(self.device)
+        if directions is None:
+            directions = (0.0, 0.0, -1.0)
+        if isinstance(directions, (tuple, list)):
+            d = torch.tensor(directions, dtype=torch.float64)
+        else:
+            d = torch.as_tensor(directions)
+            if d.dtype not in (torch.float32, torch.float64):
+                raise RuntimeError(f"RayPattern: directions must be fp32 or fp64, got {d.dtype}")
+        d = d.detach().to("cpu", torch.float32)
+        if d.shape == (3,):
+            d = d.expand(self.n_rays, 3)
+        if d.shape != (self.n_rays, 3):
+            raise RuntimeError(f"RayPattern: directions must be [R,3] or [3] for R = {self.n_rays}, got {list(d.shape)}")
+        d = d.contiguous()
+        self.vertical_down = bool(((d[:, 0] == 0) & (d[:, 1] == 0) & (d[:, 2] == -1)).all())
+        self.dirs = d.to(self.device)
         if self.n_rays:
             self.box = (C.c_float * 4)(float(cpu[:, 0].min()), float(cpu[:, 0].max()), float(cpu[:, 1].min()),
                                        float(cpu[:, 1].max()))
@@ -138,22 +159,44 @@ class RayPattern:
         self.box_t = torch.frombuffer(self.box, dtype=torch.float32)  # host tensor aliasing the box
 
     @classmethod
-    def grid(cls, device, resolution: float = 0.1, size=(3.0, 3.0), offset_pos=(0.0, 0.0, 10.0)) -> "RayPattern":
-        return cls(grid_pattern(resolution, size, offset_pos), device)
+    def grid(cls, device, resolution: float = 0.1, size=(3.0, 3.0), offset_pos=(0.0, 0.0, 10.0),
+             direction=(0.0, 0.0, -1.0)) -> "RayPattern":
+        """ORBIT ``grid_pattern``: every ray of the grid casts along ``direction`` (``GridPatternCfg.direction``)."""
+        return cls(grid_pattern(resolution, size, offset_pos), device, directions=direction)
+
+
+def require_vertical(what: str, rays: "RayPattern", attach_yaw_only: bool = True) -> None:
+    """The fused / bf16 / encoder / host / single-launch step paths cast vertical yaw-only rays only."""
+    if not attach_yaw_only or not rays.vertical_down:
+        raise RuntimeError(f"{what}: only vertical rays (direction (0, 0, -1), attach_yaw_only=True) are supported; this "
+                           f"pattern has attach_yaw_only={bool(attach_yaw_only)}, vertical_down={rays.vertical_down}: use "
+                           f"height_scan(..., attach_yaw_only=...)")
 
 
 DEFAULT_SCAN_VARIANT = 5
+RAY_CAST_VARIANT = 6  # rays in any direction (csrc/ray_cast.cu)
 
 
 def height_scan(pos_w: torch.Tensor, quat_w: torch.Tensor, rays, grid: ScanGridHandle,
                 max_distance: float = 100.0, base_offset: float = 0.26878, out: torch.Tensor | None = None,
-                return_hits: bool = False, variant: int | None = None):
+                return_hits: bool = False, variant: int | None = None, attach_yaw_only: bool = True):
     """``height_scan_rover`` over the CUDA raycaster.  ``out`` may be a ``[N, >=R]`` row-strided view (e.g. the
-    scan columns of the observation buffer).  Returns heights ``[N,R]`` (and ``ray_hits_w [N,R,3]``)."""
+    scan columns of the observation buffer).  Returns heights ``[N,R]`` (and ``ray_hits_w [N,R,3]``).
+    ``attach_yaw_only`` (ORBIT ``RayCasterCfg``): True rotates the ray starts by the yaw of ``quat_w`` only and leaves the
+    directions as they are; False rotates starts and directions by the full ``quat_w``.  Yaw-only with a ``vertical_down``
+    pattern runs the vertical kernels (variants 0 / 2 / 4 / 5, default 5); any other configuration runs variant 6, the
+    kernel of rays in any direction, which ``variant=6`` also forces for the vertical configuration."""
     if not isinstance(rays, RayPattern):
         rays = RayPattern(rays, pos_w.device)
     ray_starts_local = rays.starts
-    variant = DEFAULT_SCAN_VARIANT if variant is None else variant
+    general = not attach_yaw_only or not rays.vertical_down
+    if variant is None:
+        variant = RAY_CAST_VARIANT if general else DEFAULT_SCAN_VARIANT
+    if variant == RAY_CAST_VARIANT:
+        return _ray_cast(pos_w, quat_w, rays, grid, max_distance, base_offset, out, return_hits, attach_yaw_only)
+    if general:
+        raise RuntimeError(f"height_scan: variant {variant} casts vertical yaw-only rays only; this configuration "
+                           f"(attach_yaw_only={bool(attach_yaw_only)}, vertical_down={rays.vertical_down}) needs variant 6")
     if variant == 0:
         grid.ensure_home_grid()
     dev = _lib.require_cuda(pos_w, quat_w, ray_starts_local)
@@ -180,6 +223,32 @@ def height_scan(pos_w: torch.Tensor, quat_w: torch.Tensor, rays, grid: ScanGridH
     return out
 
 
+def _ray_cast(pos_w, quat_w, rays: RayPattern, grid: ScanGridHandle, max_distance, base_offset, out, return_hits,
+              attach_yaw_only):
+    dev = _lib.require_cuda(pos_w, quat_w, rays.starts, rays.dirs)
+    n, r = pos_w.shape[0], rays.n_rays
+    if pos_w.dtype != torch.float32 or quat_w.dtype != torch.float32:
+        raise RuntimeError("height_scan: fp32 tensors required")
+    if pos_w.shape != (n, 3) or quat_w.shape != (n, 4):
+        raise RuntimeError("height_scan: bad shapes")
+    if grid.device != dev:
+        raise RuntimeError("height_scan: grid lives on another device")
+    if grid.cells_struct is None:
+        raise RuntimeError("height_scan: variant 6 needs a ScanGridHandle built with plane_cells=True")
+    args = (pos_w, quat_w, rays.starts, rays.box_t, grid.desc, grid.cells_desc, float(max_distance), float(base_offset),
+            RAY_CAST_VARIANT, rays.dirs, bool(attach_yaw_only))
+    if return_hits:
+        if out is not None:
+            raise RuntimeError("height_scan: return_hits allocates its outputs (out= is not supported with it)")
+        return torch.ops.rover_b200.ray_cast_hits(*args)
+    if out is None:
+        return torch.ops.rover_b200.ray_cast(*args)
+    if out.dtype != torch.float32 or out.shape != (n, r) or out.stride(1) != 1 or out.device != dev:
+        raise RuntimeError("height_scan: out must be fp32 [N,R] with unit inner stride")
+    torch.ops.rover_b200.ray_cast_out(*args, out)
+    return out
+
+
 class HostScanWork:
     """Device work area of ``height_scan_host`` for up to ``n_envs`` environments (poses in, heights out)."""
 
@@ -200,6 +269,7 @@ def height_scan_host(pos_host: torch.Tensor, quat_host: torch.Tensor, rays: "Ray
     (``rover_height_scan_host``; on a PCIe-attached B200 the device-to-host copy is 90 % of the step and slicing does not
     pay, hence the default of one slice).  Asynchronous: ``out_host`` is valid once the current stream of ``work.device`` is
     synchronised."""
+    require_vertical("height_scan_host", rays)
     variant = DEFAULT_SCAN_VARIANT if variant is None else variant
     if variant == 0:
         grid.ensure_home_grid()
@@ -249,6 +319,7 @@ def height_scan_obs(pos_w: torch.Tensor, quat_w: torch.Tensor, rays, grid: ScanG
     The policy rounds fp32 observations to exactly these bf16 values, so actions and trajectory do not change."""
     if not isinstance(rays, RayPattern):
         rays = RayPattern(rays, pos_w.device)
+    require_vertical("height_scan_obs", rays)
     _lib.require_cuda(pos_w, quat_w)  # obs / obs_bf16 are row-strided views: checked below
     n = pos_w.shape[0]
     if (not obs.is_cuda or obs.dtype != torch.float32 or obs.shape[0] != n or obs.stride(1) != 1 or obs.shape[1] < head_cols + rays.n_rays
@@ -265,6 +336,7 @@ def height_scan_encoder(pos_w: torch.Tensor, quat_w: torch.Tensor, rays, grid: S
     ``[N, 64]`` bf16 = ``[e(60), obs[:, 0:4]]``, the input of the MLP.  See ``height_scan_policy``."""
     if not isinstance(rays, RayPattern):
         rays = RayPattern(rays, pos_w.device)
+    require_vertical("height_scan_encoder", rays)
     dev = _lib.require_cuda(pos_w, quat_w)
     if grid.device != dev or grid.cells_struct is None:
         raise RuntimeError("height_scan_encoder: needs a ScanGridHandle with plane cells on the tensors' device")
@@ -517,6 +589,7 @@ def step_fused(buf: MdpBuffers, params: _lib.MdpParams, tables: "TerrainTablesHa
     Per-env results are bit-identical to ``mdp_step(..., rng=)`` followed by ``height_scan``."""
     if not isinstance(rays, RayPattern):
         rays = RayPattern(rays, root_pos_w.device)
+    require_vertical("step_fused", rays)
     dev = _lib.require_cuda(root_pos_w, root_quat_w, new_actions, force_matrix_w)
     if dev != buf.device or tables.device != dev or grid.device != dev or grid.cells_struct is None:
         raise RuntimeError("step_fused: tensors / tables / grid (with plane cells) must live on one CUDA device")

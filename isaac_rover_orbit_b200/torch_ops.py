@@ -32,6 +32,15 @@ _SCHEMAS = {
                        "float max_distance, float base_offset, int variant, Tensor(a!) out) -> ()",
     "height_scan_hits": "(Tensor pos_w, Tensor quat_w, Tensor ray_starts, Tensor pattern_box, Tensor grid, Tensor? cells, "
                         "float max_distance, float base_offset, int variant) -> (Tensor, Tensor)",
+    # ---- the same with rays in any direction (RayCasterCfg.attach_yaw_only, GridPatternCfg.direction)
+    "ray_cast": "(Tensor pos_w, Tensor quat_w, Tensor ray_starts, Tensor pattern_box, Tensor grid, Tensor? cells, "
+                "float max_distance, float base_offset, int variant, Tensor ray_dirs, bool attach_yaw_only) -> Tensor",
+    "ray_cast_out": "(Tensor pos_w, Tensor quat_w, Tensor ray_starts, Tensor pattern_box, Tensor grid, Tensor? cells, "
+                    "float max_distance, float base_offset, int variant, Tensor ray_dirs, bool attach_yaw_only, "
+                    "Tensor(a!) out) -> ()",
+    "ray_cast_hits": "(Tensor pos_w, Tensor quat_w, Tensor ray_starts, Tensor pattern_box, Tensor grid, Tensor? cells, "
+                     "float max_distance, float base_offset, int variant, Tensor ray_dirs, bool attach_yaw_only) "
+                     "-> (Tensor, Tensor)",
     "height_scan_obs": "(Tensor pos_w, Tensor quat_w, Tensor ray_starts, Tensor pattern_box, Tensor grid, Tensor? cells, "
                        "float max_distance, float base_offset, Tensor(a!) obs, int head_cols, Tensor(b!) obs_bf16, "
                        "bool bf16_only=False) -> ()",
@@ -145,6 +154,51 @@ def _height_scan_hits(pos_w, quat_w, ray_starts, pattern_box, grid, cells, max_d
     out = torch.empty(n, r, dtype=torch.float32, device=pos_w.device)
     hits = torch.empty(n, r, 3, dtype=torch.float32, device=pos_w.device)
     _scan_call(pos_w, quat_w, ray_starts, pattern_box, grid, cells, max_distance, base_offset, variant, out, hits)
+    return out, hits
+
+
+def _ray_cast_call(pos_w, quat_w, ray_starts, grid, cells, max_distance, base_offset, variant, ray_dirs, attach_yaw_only,
+                   out, hits):
+    """``variant`` is 6, the only kernel of rays in any direction; ``pattern_box`` is not read."""
+    _f32("ray_cast", pos_w, quat_w, ray_starts, ray_dirs)
+    n, r = pos_w.shape[0], ray_starts.shape[0]
+    if pos_w.shape != (n, 3) or quat_w.shape != (n, 4) or ray_starts.shape != (r, 3) or ray_dirs.shape != (r, 3):
+        raise RuntimeError("rover_b200::ray_cast: pos_w [N,3], quat_w [N,4], ray_starts [R,3], ray_dirs [R,3] expected")
+    if not (pos_w.device == quat_w.device == ray_starts.device == ray_dirs.device):
+        raise RuntimeError("rover_b200::ray_cast: tensors on different devices")
+    if out.dtype != torch.float32 or out.shape != (n, r) or (n > 0 and out.stride(1) != 1) or out.device != pos_w.device:
+        raise RuntimeError("rover_b200::ray_cast: out must be fp32 [N,R] with unit inner stride")
+    if int(variant) != 6:
+        raise RuntimeError(f"rover_b200::ray_cast: variant {variant}: rays in any direction run as variant 6")
+    if cells is None:
+        raise RuntimeError("rover_b200::ray_cast: the plane-cell table is required")
+    _lib.check(_lib.load().rover_ray_cast(
+        _p(pos_w), _p(quat_w), n, _p(ray_starts), _p(ray_dirs), r, int(bool(attach_yaw_only)),
+        _desc(grid, _lib.ScanGrid, "grid"), _desc(cells, _lib.PlaneCells, "cells"), float(max_distance),
+        float(base_offset), _p(out), int(out.stride(0)) if n > 0 else r, _p(hits), _stream(pos_w)))
+
+
+def _ray_cast(pos_w, quat_w, ray_starts, pattern_box, grid, cells, max_distance, base_offset, variant, ray_dirs,
+              attach_yaw_only):
+    out = torch.empty(pos_w.shape[0], ray_starts.shape[0], dtype=torch.float32, device=pos_w.device)
+    _ray_cast_call(pos_w, quat_w, ray_starts, grid, cells, max_distance, base_offset, variant, ray_dirs, attach_yaw_only,
+                   out, None)
+    return out
+
+
+def _ray_cast_out(pos_w, quat_w, ray_starts, pattern_box, grid, cells, max_distance, base_offset, variant, ray_dirs,
+                  attach_yaw_only, out):
+    _ray_cast_call(pos_w, quat_w, ray_starts, grid, cells, max_distance, base_offset, variant, ray_dirs, attach_yaw_only,
+                   out, None)
+
+
+def _ray_cast_hits(pos_w, quat_w, ray_starts, pattern_box, grid, cells, max_distance, base_offset, variant, ray_dirs,
+                   attach_yaw_only):
+    n, r = pos_w.shape[0], ray_starts.shape[0]
+    out = torch.empty(n, r, dtype=torch.float32, device=pos_w.device)
+    hits = torch.empty(n, r, 3, dtype=torch.float32, device=pos_w.device)
+    _ray_cast_call(pos_w, quat_w, ray_starts, grid, cells, max_distance, base_offset, variant, ray_dirs, attach_yaw_only,
+                   out, hits)
     return out, hits
 
 
@@ -469,6 +523,7 @@ def _fill_holes(mask):
 
 _IMPLS = {
     "height_scan": _height_scan, "height_scan_out": _height_scan_out, "height_scan_hits": _height_scan_hits,
+    "ray_cast": _ray_cast, "ray_cast_out": _ray_cast_out, "ray_cast_hits": _ray_cast_hits,
     "height_scan_obs": _height_scan_obs, "height_scan_host": _height_scan_host, "ackermann": _ackermann, "mdp_pre_step": _mdp_pre_step,
     "mdp_post_step": _mdp_post_step, "mdp_step": _mdp_step, "step_fused": _step_fused, "stats_read": _stats_read, "policy_pack": _policy_pack,
     "policy_forward": _policy_forward, "policy_value_forward": _policy_value_forward, "gaussian_act": _gaussian_act,
@@ -492,6 +547,17 @@ def _(pos_w, quat_w, ray_starts, pattern_box, grid, cells, max_distance, base_of
 
 @_fake("height_scan_hits")
 def _(pos_w, quat_w, ray_starts, pattern_box, grid, cells, max_distance, base_offset, variant):
+    n, r = pos_w.shape[0], ray_starts.shape[0]
+    return pos_w.new_empty(n, r), pos_w.new_empty(n, r, 3)
+
+
+@_fake("ray_cast")
+def _(pos_w, quat_w, ray_starts, pattern_box, grid, cells, max_distance, base_offset, variant, ray_dirs, attach_yaw_only):
+    return pos_w.new_empty(pos_w.shape[0], ray_starts.shape[0])
+
+
+@_fake("ray_cast_hits")
+def _(pos_w, quat_w, ray_starts, pattern_box, grid, cells, max_distance, base_offset, variant, ray_dirs, attach_yaw_only):
     n, r = pos_w.shape[0], ray_starts.shape[0]
     return pos_w.new_empty(n, r), pos_w.new_empty(n, r, 3)
 
@@ -546,7 +612,7 @@ def _fake_none(*args, **kwargs):
     return None
 
 
-for _name in ("height_scan_out", "height_scan_obs", "height_scan_host", "gaussian_act_out", "mdp_pre_step", "mdp_post_step", "mdp_step", "step_fused", "stats_read", "policy_pack",
+for _name in ("height_scan_out", "ray_cast_out", "height_scan_obs", "height_scan_host", "gaussian_act_out", "mdp_pre_step", "mdp_post_step", "mdp_step", "step_fused", "stats_read", "policy_pack",
               "policy_pack_fused", "mesh_to_heightmap"):
     torch.library.register_fake(f"{NS}::{_name}", _fake_none, lib=_DEF)
 
