@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define ROVER_B200_ABI_VERSION 4
+#define ROVER_B200_ABI_VERSION 5
 #define ROVER_MAX_LEVELS 12
 #define ROVER_NUM_REWARD_TERMS 7
 #define ROVER_NUM_TERMINATION_TERMS 4
@@ -143,6 +143,31 @@ int rover_height_scan_obs_bf16(const float* pos_w, const float* quat_w, int32_t 
                                int32_t n_rays, const float* pattern_box /* host */, const RoverScanGrid* grid,
                                const RoverPlaneCells* cells, float max_distance, float base_offset, const float* obs_head,
                                int32_t obs_stride, int32_t head_cols, uint16_t* obs_bf16, int32_t bf16_stride, void* stream);
+
+/* The observation and host-buffer forms of rover_ray_cast (rays in any direction; B200-native additions like the two
+ * entries above).  rover_ray_cast_obs / rover_ray_cast_obs_bf16 replace the same reference lines as rover_ray_cast
+ * (rover_env_cfg.py:78-86 + observations.py:35-45) and take the arguments of rover_height_scan_obs /
+ * rover_height_scan_obs_bf16 without pattern_box, plus ray_dirs_local and attach_yaw_only as in rover_ray_cast.  One
+ * launch: the fp32 heights (not in the _bf16 form) are rover_ray_cast's bit for bit, obs_bf16 receives the bf16 (round
+ * to nearest even) mirror of columns [0, head_cols + n_rays); any head_cols >= 0; n_rays == 0 mirrors the head only.
+ * The head columns are read after the kernel in front of this one (the post-step that writes them) has completed.
+ * cells is required, as for rover_ray_cast. */
+int rover_ray_cast_obs(const float* pos_w, const float* quat_w, int32_t n_envs, const float* ray_starts_local,
+                       const float* ray_dirs_local, int32_t n_rays, int32_t attach_yaw_only, const RoverScanGrid* grid /* host */,
+                       const RoverPlaneCells* cells /* host */, float max_distance, float base_offset, float* obs,
+                       int32_t obs_stride, int32_t head_cols, uint16_t* obs_bf16, int32_t bf16_stride, void* stream);
+int rover_ray_cast_obs_bf16(const float* pos_w, const float* quat_w, int32_t n_envs, const float* ray_starts_local,
+                            const float* ray_dirs_local, int32_t n_rays, int32_t attach_yaw_only,
+                            const RoverScanGrid* grid /* host */, const RoverPlaneCells* cells /* host */, float max_distance,
+                            float base_offset, const float* obs_head, int32_t obs_stride, int32_t head_cols,
+                            uint16_t* obs_bf16, int32_t bf16_stride, void* stream);
+/* rover_height_scan_host with rover_ray_cast as the scan: replaces the same reference lines as rover_ray_cast plus the
+ * .cpu() / .to(device) round trip around them.  Arguments of rover_height_scan_host without pattern_box and variant, plus
+ * ray_dirs_local and attach_yaw_only; the same work area (rover_height_scan_host_work_bytes) and n_slices semantics. */
+int rover_ray_cast_host(const float* pos_host, const float* quat_host, int32_t n_envs, const float* ray_starts_local,
+                        const float* ray_dirs_local, int32_t n_rays, int32_t attach_yaw_only, const RoverScanGrid* grid,
+                        const RoverPlaneCells* cells, float max_distance, float base_offset, float* out_host,
+                        int32_t out_stride, void* work, int64_t work_bytes, int32_t n_slices, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------
  * Fused MDP step.  Replaces, in one launch (SURVEY.md 8a rows a-1..a-23):

@@ -19,7 +19,7 @@ NUM_REWARD_TERMS = 7
 NUM_TERMINATION_TERMS = 4
 STATS_LEN = 16
 MDP_BLOCK = 64
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 SYMBOLS = ("rover_abi_version", "rover_last_error", "rover_height_scan", "rover_height_scan_obs", "rover_mdp_pre_step",
            "rover_mdp_post_step", "rover_mdp_post_step_x", "rover_mdp_post_step_v3", "rover_mdp_step", "rover_mdp_step_v3",
@@ -29,7 +29,8 @@ SYMBOLS = ("rover_abi_version", "rover_last_error", "rover_height_scan", "rover_
            "rover_height_scan_host", "rover_height_scan_host_work_bytes", "rover_stats_publish", "rover_height_scan_obs_bf16", "rover_policy_pack", "rover_policy_forward", "rover_value_forward", "rover_policy_value_forward", "rover_policy_forward_bf16",
            "rover_value_forward_bf16", "rover_gaussian_act", "rover_mesh_to_heightmap", "rover_steep_mask",
            "rover_policy_pack_fused", "rover_scan_encoder_fused", "rover_policy_mlp_forward", "rover_morph_box",
-           "rover_fill_holes", "rover_step_fused", "rover_ray_cast")
+           "rover_fill_holes", "rover_step_fused", "rover_ray_cast", "rover_ray_cast_obs", "rover_ray_cast_obs_bf16",
+           "rover_ray_cast_host")
 
 
 class ScanLevel(C.Structure):
@@ -131,6 +132,13 @@ def load() -> C.CDLL:
     lib.rover_ray_cast.restype = C.c_int
     lib.rover_ray_cast.argtypes = [vp, vp, i32, vp, vp, i32, i32, C.POINTER(ScanGrid), C.POINTER(PlaneCells), f32, f32, vp,
                                    i32, vp, vp]
+    for fn in (lib.rover_ray_cast_obs, lib.rover_ray_cast_obs_bf16):
+        fn.restype = C.c_int
+        fn.argtypes = [vp, vp, i32, vp, vp, i32, i32, C.POINTER(ScanGrid), C.POINTER(PlaneCells), f32, f32, vp, i32, i32, vp,
+                       i32, vp]
+    lib.rover_ray_cast_host.restype = C.c_int
+    lib.rover_ray_cast_host.argtypes = [vp, vp, i32, vp, vp, i32, i32, C.POINTER(ScanGrid), C.POINTER(PlaneCells), f32, f32,
+                                        vp, i32, vp, C.c_int64, i32, vp]
     lib.rover_mdp_pre_step.restype = C.c_int
     lib.rover_mdp_pre_step.argtypes = [vp, vp, i32, C.POINTER(MdpParams), C.POINTER(MdpState), C.POINTER(MdpOut), i32,
                                        vp]

@@ -65,6 +65,8 @@ class RayCasterCfg:
     """ORBIT ``RayCasterCfg`` as wired at rover_env_cfg.py:78-86."""
 
     offset_pos: tuple = (0.0, 0.0, 10.0)
+    # RayCasterCfg.offset.rot (w, x, y, z): rotates the pattern's directions, not its starts (RayPattern.grid)
+    offset_rot: tuple = (1.0, 0.0, 0.0, 0.0)
     attach_yaw_only: bool = True
     pattern_cfg: GridPatternCfg = field(default_factory=GridPatternCfg)
     max_distance: float = 100.0

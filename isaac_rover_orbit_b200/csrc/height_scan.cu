@@ -266,24 +266,20 @@ static int host_scan_streams(HostScanStreams*& out) {
 }
 }  // namespace rover
 
-extern "C" int rover_height_scan_host(const float* pos_host, const float* quat_host, int32_t n_envs,
-                                      const float* ray_starts_local, int32_t n_rays, const float* pattern_box,
-                                      const RoverScanGrid* grid, const RoverPlaneCells* cells, float max_distance,
-                                      float base_offset, float* out_host, int32_t out_stride, void* work, int64_t work_bytes,
-                                      int32_t n_slices, int32_t variant, void* stream) {
-    using namespace rover;
-    ROVER_CHECK(n_envs >= 0 && n_rays >= 0, "rover_height_scan_host: negative sizes");
+int rover::host_scan_sliced(const char* what, const float* pos_host, const float* quat_host, int n_envs, int n_rays,
+                            float* out_host, int out_stride, void* work, int64_t work_bytes, int n_slices, cudaStream_t s,
+                            const HostSliceScan& scan) {
+    ROVER_CHECK(n_envs >= 0 && n_rays >= 0, "%s: negative sizes", what);
     const int64_t need = rover_height_scan_host_work_bytes(n_envs, out_stride);
     if (n_envs == 0 || n_rays == 0) return 0;
-    ROVER_CHECK(pos_host && quat_host && out_host && work, "rover_height_scan_host: NULL buffer");
-    ROVER_CHECK(out_stride >= n_rays, "rover_height_scan_host: out_stride %d < n_rays %d", out_stride, n_rays);
+    ROVER_CHECK(pos_host && quat_host && out_host && work, "%s: NULL buffer", what);
+    ROVER_CHECK(out_stride >= n_rays, "%s: out_stride %d < n_rays %d", what, out_stride, n_rays);
     ROVER_CHECK(work_bytes >= need && (reinterpret_cast<uintptr_t>(work) & 255) == 0,
-                "rover_height_scan_host: work area of %lld bytes (256-byte aligned) needed, got %lld", (long long)need,
+                "%s: work area of %lld bytes (256-byte aligned) needed, got %lld", what, (long long)need,
                 (long long)work_bytes);
-    ROVER_CHECK(n_slices >= 1 && n_slices <= 64, "rover_height_scan_host: n_slices %d not in [1, 64]", n_slices);
+    ROVER_CHECK(n_slices >= 1 && n_slices <= 64, "%s: n_slices %d not in [1, 64]", what, n_slices);
     HostScanStreams* hs = nullptr;
     if (int rc = host_scan_streams(hs)) return rc;
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
     float* d_pos = static_cast<float*>(work);
     float* d_quat = d_pos + 3 * (size_t)n_envs;
     float* d_out = reinterpret_cast<float*>(static_cast<unsigned char*>(work) + host_scan_pose_bytes(n_envs));
@@ -291,18 +287,14 @@ extern "C" int rover_height_scan_host(const float* pos_host, const float* quat_h
     ROVER_CUDA(cudaMemcpyAsync(d_quat, quat_host, 16 * (size_t)n_envs, cudaMemcpyHostToDevice, s));
     const int slices = n_slices < n_envs ? n_slices : n_envs;
     if (slices == 1) {  // one launch, everything in order on the caller's stream (no second stream to join)
-        if (int rc = rover_height_scan(d_pos, d_quat, n_envs, ray_starts_local, n_rays, pattern_box, grid, cells, max_distance,
-                                       base_offset, d_out, out_stride, nullptr, variant, stream))
-            return rc;
+        if (int rc = scan(d_pos, d_quat, n_envs, d_out, s)) return rc;
         ROVER_CUDA(cudaMemcpyAsync(out_host, d_out, (size_t)n_envs * out_stride * 4, cudaMemcpyDeviceToHost, s));
         return 0;
     }
     for (int k = 0; k < slices; ++k) {
         // slice k's heights travel to the host on the copy stream while slice k + 1 is scanned on the caller's stream
         const int e0 = (int)((int64_t)n_envs * k / slices), e1 = (int)((int64_t)n_envs * (k + 1) / slices);
-        if (int rc = rover_height_scan(d_pos + 3 * (size_t)e0, d_quat + 4 * (size_t)e0, e1 - e0, ray_starts_local, n_rays,
-                                       pattern_box, grid, cells, max_distance, base_offset, d_out + (size_t)e0 * out_stride,
-                                       out_stride, nullptr, variant, stream))
+        if (int rc = scan(d_pos + 3 * (size_t)e0, d_quat + 4 * (size_t)e0, e1 - e0, d_out + (size_t)e0 * out_stride, s))
             return rc;
         ROVER_CUDA(cudaEventRecord(hs->scanned[k], s));
         ROVER_CUDA(cudaStreamWaitEvent(hs->copy, hs->scanned[k], 0));
@@ -313,6 +305,20 @@ extern "C" int rover_height_scan_host(const float* pos_host, const float* quat_h
     ROVER_CUDA(cudaEventRecord(hs->done, hs->copy));
     ROVER_CUDA(cudaStreamWaitEvent(s, hs->done, 0));
     return 0;
+}
+
+extern "C" int rover_height_scan_host(const float* pos_host, const float* quat_host, int32_t n_envs,
+                                      const float* ray_starts_local, int32_t n_rays, const float* pattern_box,
+                                      const RoverScanGrid* grid, const RoverPlaneCells* cells, float max_distance,
+                                      float base_offset, float* out_host, int32_t out_stride, void* work, int64_t work_bytes,
+                                      int32_t n_slices, int32_t variant, void* stream) {
+    using namespace rover;
+    return host_scan_sliced("rover_height_scan_host", pos_host, quat_host, n_envs, n_rays, out_host, out_stride, work,
+                            work_bytes, n_slices, static_cast<cudaStream_t>(stream),
+                            [&](const float* pos, const float* quat, int n, float* out, cudaStream_t s) {
+                                return rover_height_scan(pos, quat, n, ray_starts_local, n_rays, pattern_box, grid, cells,
+                                                         max_distance, base_offset, out, out_stride, nullptr, variant, s);
+                            });
 }
 
 extern "C" int64_t rover_height_scan_host_work_bytes(int32_t n_envs, int32_t out_stride) {

@@ -14,12 +14,20 @@
 //     cell is solved on its segment from the entry point relative to the cell corner: g(t) = P_z - z(P_x, P_y) is
 //     linear on either side of the crease E = 0, and the first zero / sign change is the hit (double-sided).  A general
 //     cell tests the home-grid records that can cover it: plane intersection, then the three edge functions.
+// The observation form (rover_ray_cast_obs / _bf16) is the same kernel with the stores of rover_height_scan_obs: heights
+// into columns [head_cols, head_cols + n_rays) of the fp32 observation and their bf16 mirror, plus the mirror of the
+// head columns [0, head_cols) that the post-step wrote.
+#include <cuda_bf16.h>
+
 #include "scan_common.cuh"
 
 namespace rover {
 namespace {
 
 constexpr int kRayThreads = 256;
+
+// what the kernel stores: heights (+ hits), fp32 observation + bf16 mirror, or the bf16 mirror only
+enum RayStore { kStoreHeights = 0, kStoreObs = 1, kStoreBf16Only = 2 };
 
 struct RayFrame {
     SensorFrame yaw;       // yaw-only frame (attach_yaw_only)
@@ -222,11 +230,16 @@ __device__ __forceinline__ float cast_tilted(const ScanGridDev& g, const PlaneCe
     }
 }
 
+// kStoreHeights: heights to out[env, r] (head_cols == 0), hits optional.  The observation modes: `out` is the fp32
+// observation, heights go to out[env, head_cols + r] (kStoreObs only) and their bf16 to obs_bf16[env, head_cols + r];
+// the CTAs of chunk 0 mirror out[env, 0:head_cols] into obs_bf16.
+template <int kStore>
 __global__ void __launch_bounds__(kRayThreads, 2)
 ray_cast_kernel(const float* __restrict__ pos_w, const float* __restrict__ quat_w, int n_chunks,
                 const float* __restrict__ ray_local, const float* __restrict__ ray_dirs, int n_rays, int yaw_only,
                 const __grid_constant__ ScanGridDev g, const __grid_constant__ PlaneCellsDev pc, float max_d,
-                float base_offset, float* __restrict__ out, int out_stride, float* __restrict__ hits) {
+                float base_offset, float* __restrict__ out, int out_stride, int head_cols, float* __restrict__ hits,
+                __nv_bfloat16* __restrict__ obs_bf16, int bf16_stride) {
     const int env = blockIdx.x / n_chunks;
     const int r = (blockIdx.x - env * n_chunks) * kRayThreads + threadIdx.x;
     // the ray pattern is launch-invariant: read it before waiting for the kernel in front of this one
@@ -244,6 +257,12 @@ ray_cast_kernel(const float* __restrict__ pos_w, const float* __restrict__ quat_
         frame_s.qx = q[1];
         frame_s.qy = q[2];
         frame_s.qz = q[3];
+    }
+    if (kStore != kStoreHeights && blockIdx.x == env * n_chunks) {
+        // the head columns are written by the kernel in front of this one (the post-step): read only after the wait
+        const float* head = out + (size_t)env * out_stride;
+        __nv_bfloat16* dst = obs_bf16 + (size_t)env * bf16_stride;
+        for (int c = threadIdx.x; c < head_cols; c += kRayThreads) dst[c] = __float2bfloat16_rn(head[c]);
     }
     __syncthreads();
     if (r >= n_rays) return;
@@ -291,8 +310,9 @@ ray_cast_kernel(const float* __restrict__ pos_w, const float* __restrict__ quat_
         hz = fmaf(t, Dz, Z);
         h = __fsub_rn(__fsub_rn(f.yaw.pz, hz), base_offset);
     }
-    out[(size_t)env * out_stride + r] = h;
-    if (hits) {
+    if (kStore != kStoreBf16Only) out[(size_t)env * out_stride + head_cols + r] = h;
+    if (kStore != kStoreHeights) obs_bf16[(size_t)env * bf16_stride + head_cols + r] = __float2bfloat16_rn(h);
+    if (kStore == kStoreHeights && hits) {
         float* p3 = hits + ((size_t)env * n_rays + r) * 3;
         p3[0] = hx;
         p3[1] = hy;
@@ -304,6 +324,50 @@ ray_cast_kernel(const float* __restrict__ pos_w, const float* __restrict__ quat_
 
 int make_dev_grid(const RoverScanGrid* grid, ScanGridDev& g);  // height_scan.cu
 
+// the checks and the launch shared by the entry points (`what` names the entry point in messages); n_envs > 0, and
+// n_rays > 0 in the heights mode.  In the observation modes n_rays may be 0: one CTA per environment mirrors the head.
+template <int kStore>
+static int launch_ray_cast(const char* what, const float* pos_w, const float* quat_w, int32_t n_envs,
+                           const float* ray_starts_local, const float* ray_dirs_local, int32_t n_rays, int32_t attach_yaw_only,
+                           const RoverScanGrid* grid, const RoverPlaneCells* cells, float max_distance, float base_offset,
+                           float* out, int32_t out_stride, int32_t head_cols, float* out_hits_w, uint16_t* obs_bf16,
+                           int32_t bf16_stride, void* stream) {
+    ROVER_CHECK(pos_w && quat_w && (n_rays == 0 || (ray_starts_local && ray_dirs_local)), "%s: NULL tensor", what);
+    ROVER_CHECK(cells != nullptr, "%s: the plane-cell table is required", what);
+    ROVER_CHECK(cells->xs && cells->ys && cells->entries && cells->nx > 0 && cells->ny > 0, "%s: bad plane-cell table", what);
+    ROVER_CHECK((reinterpret_cast<uintptr_t>(cells->entries) & 15) == 0, "%s: plane-cell entries not 16B aligned", what);
+    ScanGridDev g;
+    if (int rc = make_dev_grid(grid, g)) return rc;
+    const int n_chunks = n_rays > 0 ? (n_rays + kRayThreads - 1) / kRayThreads : 1;
+    ROVER_CHECK((int64_t)n_envs * n_chunks <= 0x7fffffff, "%s: %d environments x %d chunks is too many", what, n_envs,
+                n_chunks);
+    const PlaneCellsDev pc{cells->xs, cells->ys, reinterpret_cast<const float4*>(cells->entries), cells->nx, cells->ny,
+                           cells->inv_dx, cells->inv_dy};
+    ROVER_CUDA(launch_overlapped(ray_cast_kernel<kStore>, dim3(n_envs * n_chunks), dim3(kRayThreads), 0,
+                                 static_cast<cudaStream_t>(stream), pos_w, quat_w, n_chunks, ray_starts_local, ray_dirs_local,
+                                 n_rays, (int)(attach_yaw_only != 0), g, pc, max_distance, base_offset, out, out_stride,
+                                 head_cols, out_hits_w, reinterpret_cast<__nv_bfloat16*>(obs_bf16), bf16_stride));
+    return check_launch("ray_cast_kernel");
+}
+
+// the observation entry points: fp32 + bf16 (kStoreObs) or bf16 only (kStoreBf16Only)
+template <int kStore>
+static int ray_cast_obs_impl(const char* what, const float* pos_w, const float* quat_w, int32_t n_envs,
+                             const float* ray_starts_local, const float* ray_dirs_local, int32_t n_rays, int32_t attach_yaw_only,
+                             const RoverScanGrid* grid, const RoverPlaneCells* cells, float max_distance, float base_offset,
+                             float* obs, int32_t obs_stride, int32_t head_cols, uint16_t* obs_bf16, int32_t bf16_stride,
+                             void* stream) {
+    ROVER_CHECK(n_envs >= 0 && n_rays >= 0 && head_cols >= 0, "%s: negative sizes", what);
+    if (n_envs == 0 || n_rays + head_cols == 0) return 0;
+    ROVER_CHECK(obs && obs_bf16, "%s: NULL observation buffer", what);
+    ROVER_CHECK((int64_t)head_cols + n_rays <= obs_stride && (int64_t)head_cols + n_rays <= bf16_stride,
+                "%s: row strides %d / %d < head_cols + n_rays = %lld", what, obs_stride, bf16_stride,
+                (long long)head_cols + n_rays);
+    return launch_ray_cast<kStore>(what, pos_w, quat_w, n_envs, ray_starts_local, ray_dirs_local, n_rays, attach_yaw_only,
+                                   grid, cells, max_distance, base_offset, obs, obs_stride, head_cols, nullptr, obs_bf16,
+                                   bf16_stride, stream);
+}
+
 }  // namespace rover
 
 extern "C" int rover_ray_cast(const float* pos_w, const float* quat_w, int32_t n_envs, const float* ray_starts_local,
@@ -313,23 +377,45 @@ extern "C" int rover_ray_cast(const float* pos_w, const float* quat_w, int32_t n
     using namespace rover;
     ROVER_CHECK(n_envs >= 0 && n_rays >= 0, "rover_ray_cast: negative sizes");
     if (n_envs == 0 || n_rays == 0) return 0;
-    ROVER_CHECK(pos_w && quat_w && ray_starts_local && ray_dirs_local && out_heights, "rover_ray_cast: NULL tensor");
+    ROVER_CHECK(out_heights, "rover_ray_cast: NULL tensor");
     ROVER_CHECK(out_stride >= n_rays, "rover_ray_cast: out_stride %d < n_rays %d", out_stride, n_rays);
-    ROVER_CHECK(cells != nullptr, "rover_ray_cast: the plane-cell table is required");
-    ROVER_CHECK(cells->xs && cells->ys && cells->entries && cells->nx > 0 && cells->ny > 0,
-                "rover_ray_cast: bad plane-cell table");
-    ROVER_CHECK((reinterpret_cast<uintptr_t>(cells->entries) & 15) == 0,
-                "rover_ray_cast: plane-cell entries not 16B aligned");
-    ScanGridDev g;
-    if (int rc = make_dev_grid(grid, g)) return rc;
-    const int n_chunks = (n_rays + kRayThreads - 1) / kRayThreads;
-    ROVER_CHECK((int64_t)n_envs * n_chunks <= 0x7fffffff, "rover_ray_cast: %d environments x %d chunks is too many", n_envs,
-                n_chunks);
-    const PlaneCellsDev pc{cells->xs, cells->ys, reinterpret_cast<const float4*>(cells->entries), cells->nx, cells->ny,
-                           cells->inv_dx, cells->inv_dy};
-    ROVER_CUDA(launch_overlapped(ray_cast_kernel, dim3(n_envs * n_chunks), dim3(kRayThreads), 0,
-                                 static_cast<cudaStream_t>(stream), pos_w, quat_w, n_chunks, ray_starts_local, ray_dirs_local,
-                                 n_rays, (int)(attach_yaw_only != 0), g, pc, max_distance, base_offset, out_heights,
-                                 out_stride, out_hits_w));
-    return check_launch("ray_cast_kernel");
+    return launch_ray_cast<kStoreHeights>("rover_ray_cast", pos_w, quat_w, n_envs, ray_starts_local, ray_dirs_local, n_rays,
+                                          attach_yaw_only, grid, cells, max_distance, base_offset, out_heights, out_stride,
+                                          0, out_hits_w, nullptr, 0, stream);
+}
+
+extern "C" int rover_ray_cast_obs(const float* pos_w, const float* quat_w, int32_t n_envs, const float* ray_starts_local,
+                                  const float* ray_dirs_local, int32_t n_rays, int32_t attach_yaw_only,
+                                  const RoverScanGrid* grid, const RoverPlaneCells* cells, float max_distance,
+                                  float base_offset, float* obs, int32_t obs_stride, int32_t head_cols, uint16_t* obs_bf16,
+                                  int32_t bf16_stride, void* stream) {
+    return rover::ray_cast_obs_impl<rover::kStoreObs>("rover_ray_cast_obs", pos_w, quat_w, n_envs, ray_starts_local,
+                                                      ray_dirs_local, n_rays, attach_yaw_only, grid, cells, max_distance,
+                                                      base_offset, obs, obs_stride, head_cols, obs_bf16, bf16_stride, stream);
+}
+
+extern "C" int rover_ray_cast_obs_bf16(const float* pos_w, const float* quat_w, int32_t n_envs,
+                                       const float* ray_starts_local, const float* ray_dirs_local, int32_t n_rays,
+                                       int32_t attach_yaw_only, const RoverScanGrid* grid, const RoverPlaneCells* cells,
+                                       float max_distance, float base_offset, const float* obs_head, int32_t obs_stride,
+                                       int32_t head_cols, uint16_t* obs_bf16, int32_t bf16_stride, void* stream) {
+    // the kernel does not store to obs_head in this mode
+    return rover::ray_cast_obs_impl<rover::kStoreBf16Only>(
+        "rover_ray_cast_obs_bf16", pos_w, quat_w, n_envs, ray_starts_local, ray_dirs_local, n_rays, attach_yaw_only, grid,
+        cells, max_distance, base_offset, const_cast<float*>(obs_head), obs_stride, head_cols, obs_bf16, bf16_stride, stream);
+}
+
+extern "C" int rover_ray_cast_host(const float* pos_host, const float* quat_host, int32_t n_envs,
+                                   const float* ray_starts_local, const float* ray_dirs_local, int32_t n_rays,
+                                   int32_t attach_yaw_only, const RoverScanGrid* grid, const RoverPlaneCells* cells,
+                                   float max_distance, float base_offset, float* out_host, int32_t out_stride, void* work,
+                                   int64_t work_bytes, int32_t n_slices, void* stream) {
+    using namespace rover;
+    return host_scan_sliced("rover_ray_cast_host", pos_host, quat_host, n_envs, n_rays, out_host, out_stride, work,
+                            work_bytes, n_slices, static_cast<cudaStream_t>(stream),
+                            [&](const float* pos, const float* quat, int n, float* out, cudaStream_t s) {
+                                return rover_ray_cast(pos, quat, n, ray_starts_local, ray_dirs_local, n_rays,
+                                                      attach_yaw_only, grid, cells, max_distance, base_offset, out,
+                                                      out_stride, nullptr, s);
+                            });
 }

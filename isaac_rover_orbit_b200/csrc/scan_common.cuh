@@ -1,5 +1,7 @@
 // Device structs and helpers shared by the height-scan kernels.
 #pragma once
+#include <functional>
+
 #include "common.cuh"
 
 namespace rover {
@@ -74,5 +76,13 @@ __device__ __forceinline__ void test_record(const float4 r0, const float4 r1, co
     const float t = Z - z;
     if (fminf(e0, fminf(e1, e2)) >= 0.f && t >= 0.f && t < max_d) best = fmaxf(best, z);
 }
+
+// The body of the host-buffer entry points (height_scan.cu): copy the poses into the work area, run `scan` on each of
+// `n_slices` slices of environments and copy each slice's heights to out_host, slice k's copy overlapping the scan of
+// slice k + 1.  `what` names the entry point in error messages.
+using HostSliceScan = std::function<int(const float* pos, const float* quat, int n_envs, float* out, cudaStream_t s)>;
+int host_scan_sliced(const char* what, const float* pos_host, const float* quat_host, int n_envs, int n_rays,
+                     float* out_host, int out_stride, void* work, int64_t work_bytes, int n_slices, cudaStream_t s,
+                     const HostSliceScan& scan);
 
 }  // namespace rover

@@ -68,7 +68,7 @@ class RayCaster:
         self.cfg = cfg
         self._env = env
         self.ray_pattern = ops.RayPattern.grid(env.device, cfg.pattern_cfg.resolution, cfg.pattern_cfg.size, cfg.offset_pos,
-                                               direction=cfg.pattern_cfg.direction)
+                                               direction=cfg.pattern_cfg.direction, offset_rot=cfg.offset_rot)
         self.ray_starts = self.ray_pattern.starts
         outer = self
 

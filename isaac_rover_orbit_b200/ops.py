@@ -160,17 +160,35 @@ class RayPattern:
 
     @classmethod
     def grid(cls, device, resolution: float = 0.1, size=(3.0, 3.0), offset_pos=(0.0, 0.0, 10.0),
-             direction=(0.0, 0.0, -1.0)) -> "RayPattern":
-        """ORBIT ``grid_pattern``: every ray of the grid casts along ``direction`` (``GridPatternCfg.direction``)."""
-        return cls(grid_pattern(resolution, size, offset_pos), device, directions=direction)
+             direction=(0.0, 0.0, -1.0), offset_rot=(1.0, 0.0, 0.0, 0.0)) -> "RayPattern":
+        """ORBIT ``grid_pattern``: every ray of the grid casts along ``direction`` (``GridPatternCfg.direction``), rotated
+        by the sensor's ``offset_rot`` (``RayCasterCfg.offset.rot``, (w, x, y, z)) as ORBIT's ``_initialize_rays_impl``
+        does (SURVEY.md A.3): the directions are rotated with ``quat_apply`` in fp32, the starts are only translated by
+        ``offset_pos``.  These are the semantics of the ORBIT the reference was written against (early 2024); later
+        releases fold the offset into the sensor's frame instead.  The identity leaves the directions bit for bit."""
+        starts = grid_pattern(resolution, size, offset_pos)
+        n = starts.shape[0]
+        dirs = torch.tensor(direction, dtype=torch.float32).expand(n, 3)
+        dirs = quat_apply(torch.tensor(offset_rot, dtype=torch.float32).expand(n, 4), dirs)
+        return cls(starts, device, directions=dirs)
 
 
-def require_vertical(what: str, rays: "RayPattern", attach_yaw_only: bool = True) -> None:
-    """The fused / bf16 / encoder / host / single-launch step paths cast vertical yaw-only rays only."""
+def quat_apply(quat: torch.Tensor, vec: torch.Tensor) -> torch.Tensor:
+    """ORBIT ``quat_apply`` (SURVEY.md A.1), in its operation order: ``v + w * t + xyz x t`` with ``t = 2 * (xyz x v)``;
+    ``quat [..., 4]`` (w, x, y, z), ``vec [..., 3]``."""
+    xyz = quat[..., 1:]
+    t = xyz.cross(vec, dim=-1) * 2
+    return vec + quat[..., 0:1] * t + xyz.cross(t, dim=-1)
+
+
+def require_vertical(what: str, rays: "RayPattern", attach_yaw_only: bool = True, takes_variant: bool = False) -> None:
+    """The fused / bf16 / encoder / host / single-launch step paths cast vertical yaw-only rays only, unless the entry
+    point takes ``variant`` and is given ``variant=6`` (``takes_variant`` adds that hint to the message)."""
     if not attach_yaw_only or not rays.vertical_down:
+        hint = " or pass variant=6" if takes_variant else ""
         raise RuntimeError(f"{what}: only vertical rays (direction (0, 0, -1), attach_yaw_only=True) are supported; this "
                            f"pattern has attach_yaw_only={bool(attach_yaw_only)}, vertical_down={rays.vertical_down}: use "
-                           f"height_scan(..., attach_yaw_only=...)")
+                           f"height_scan(..., attach_yaw_only=...){hint}")
 
 
 DEFAULT_SCAN_VARIANT = 5
@@ -250,12 +268,16 @@ def _ray_cast(pos_w, quat_w, rays: RayPattern, grid: ScanGridHandle, max_distanc
 
 
 class HostScanWork:
-    """Device work area of ``height_scan_host`` for up to ``n_envs`` environments (poses in, heights out)."""
+    """Device work area of ``height_scan_host`` for up to ``n_envs`` environments (poses in, heights out) and host
+    height rows of up to ``out_stride`` floats (default ``n_rays``: a dense ``[N, R]`` ``out_host``)."""
 
-    def __init__(self, n_envs: int, n_rays: int, device):
+    def __init__(self, n_envs: int, n_rays: int, device, out_stride: int | None = None):
         self.device = torch.device(device)
         self.n_envs, self.n_rays = int(n_envs), int(n_rays)
-        n_bytes = int(_lib.load().rover_height_scan_host_work_bytes(self.n_envs, self.n_rays))
+        self.out_stride = self.n_rays if out_stride is None else int(out_stride)
+        if self.out_stride < self.n_rays:
+            raise RuntimeError(f"HostScanWork: out_stride {self.out_stride} < n_rays {self.n_rays}")
+        n_bytes = int(_lib.load().rover_height_scan_host_work_bytes(self.n_envs, self.out_stride))
         raw = torch.empty(n_bytes + 65536, dtype=torch.uint8, device=self.device)
         off = (-raw.data_ptr()) % 65536
         self.buffer = raw[off: off + n_bytes]
@@ -263,14 +285,16 @@ class HostScanWork:
 
 def height_scan_host(pos_host: torch.Tensor, quat_host: torch.Tensor, rays: "RayPattern", grid: ScanGridHandle,
                      out_host: torch.Tensor, work: HostScanWork, n_slices: int = 1, max_distance: float = 100.0,
-                     base_offset: float = 0.26878, variant: int | None = None) -> torch.Tensor:
+                     base_offset: float = 0.26878, variant: int | None = None, attach_yaw_only: bool = True) -> torch.Tensor:
     """``height_scan`` for a caller whose poses and heights live in HOST memory (page-locked tensors): copies the poses
     in, scans the environments in ``n_slices`` slices and sends slice k's heights to the host while slice k+1 is scanned
     (``rover_height_scan_host``; on a PCIe-attached B200 the device-to-host copy is 90 % of the step and slicing does not
     pay, hence the default of one slice).  Asynchronous: ``out_host`` is valid once the current stream of ``work.device`` is
-    synchronised."""
-    require_vertical("height_scan_host", rays)
-    variant = DEFAULT_SCAN_VARIANT if variant is None else variant
+    synchronised.  ``variant=6`` scans with the kernel of rays in any direction (``rover_ray_cast_host``) for any pattern
+    and either ``attach_yaw_only``; the other variants cast vertical yaw-only rays only."""
+    if variant != RAY_CAST_VARIANT:
+        require_vertical("height_scan_host", rays, attach_yaw_only, takes_variant=True)
+        variant = DEFAULT_SCAN_VARIANT if variant is None else variant
     if variant == 0:
         grid.ensure_home_grid()
     n = pos_host.shape[0]
@@ -278,23 +302,37 @@ def height_scan_host(pos_host: torch.Tensor, quat_host: torch.Tensor, rays: "Ray
         raise RuntimeError("height_scan_host: work area was sized for fewer environments / another ray pattern")
     if grid.device != work.device or rays.starts.device != work.device:
         raise RuntimeError("height_scan_host: grid / rays / work area live on different devices")
-    if variant in (2, 4, 5) and grid.cells_struct is None:
-        raise RuntimeError("height_scan_host: variants 2, 4, 5 need a ScanGridHandle built with plane_cells=True")
+    if variant in (2, 4, 5, RAY_CAST_VARIANT) and grid.cells_struct is None:
+        raise RuntimeError("height_scan_host: variants 2, 4, 5, 6 need a ScanGridHandle built with plane_cells=True")
     # A synchronous host loop pays every microsecond in front of the first copy: the validated call (the same one
-    # torch.ops.rover_b200.height_scan_host makes) is prepared once per set of buffers and replayed as one ctypes call.
+    # torch.ops.rover_b200.height_scan_host / ray_cast_host makes) is prepared once per set of buffers and replayed as one
+    # ctypes call.  The key holds everything the prepared arguments depend on, the route and the frame included.
     key = (pos_host.data_ptr(), quat_host.data_ptr(), out_host.data_ptr(), n, out_host.stride(0), id(rays), id(grid), id(work),
-           int(n_slices), int(variant), float(max_distance), float(base_offset))
+           int(n_slices), int(variant), bool(attach_yaw_only), float(max_distance), float(base_offset))
     call = _HOST_SCAN_CALLS.get(key)
     if call is None:
-        torch.ops.rover_b200.height_scan_host(pos_host, quat_host, rays.starts, rays.box_t, grid.desc, grid.cells_desc,
-                                              float(max_distance), float(base_offset), int(variant), int(n_slices),
-                                              work.buffer, out_host)  # first use: the operator, with all its checks
-        fn = _lib.load().rover_height_scan_host
-        cargs = (C.c_void_p(pos_host.data_ptr()), C.c_void_p(quat_host.data_ptr()), n, C.c_void_p(rays.starts.data_ptr()),
-                 rays.starts.shape[0], C.cast(C.c_void_p(rays.box_t.data_ptr()), C.POINTER(C.c_float * 4)),
-                 C.byref(grid.struct), C.byref(grid.cells_struct) if grid.cells_struct is not None else None,
-                 float(max_distance), float(base_offset), C.c_void_p(out_host.data_ptr()), int(out_host.stride(0)),
-                 C.c_void_p(work.buffer.data_ptr()), int(work.buffer.numel()), int(n_slices), int(variant))
+        if n > 0 and out_host.stride(0) > work.out_stride:  # (the key holds the stride and the work area)
+            raise RuntimeError(f"height_scan_host: work area was sized for out_host rows of {work.out_stride} floats, "
+                               f"not {out_host.stride(0)} (HostScanWork(..., out_stride=))")
+        head = (C.c_void_p(pos_host.data_ptr()), C.c_void_p(quat_host.data_ptr()), n, C.c_void_p(rays.starts.data_ptr()))
+        tail = (float(max_distance), float(base_offset), C.c_void_p(out_host.data_ptr()), int(out_host.stride(0)),
+                C.c_void_p(work.buffer.data_ptr()), int(work.buffer.numel()), int(n_slices))
+        # first use: the operator, with all its checks
+        if variant == RAY_CAST_VARIANT:
+            torch.ops.rover_b200.ray_cast_host(pos_host, quat_host, rays.starts, rays.dirs, bool(attach_yaw_only), grid.desc,
+                                               grid.cells_desc, float(max_distance), float(base_offset), int(n_slices),
+                                               work.buffer, out_host)
+            fn = _lib.load().rover_ray_cast_host
+            cargs = head + (C.c_void_p(rays.dirs.data_ptr()), rays.n_rays, int(bool(attach_yaw_only)), C.byref(grid.struct),
+                            C.byref(grid.cells_struct)) + tail
+        else:
+            torch.ops.rover_b200.height_scan_host(pos_host, quat_host, rays.starts, rays.box_t, grid.desc, grid.cells_desc,
+                                                  float(max_distance), float(base_offset), int(variant), int(n_slices),
+                                                  work.buffer, out_host)
+            fn = _lib.load().rover_height_scan_host
+            cargs = head + (rays.starts.shape[0], C.cast(C.c_void_p(rays.box_t.data_ptr()), C.POINTER(C.c_float * 4)),
+                            C.byref(grid.struct),
+                            C.byref(grid.cells_struct) if grid.cells_struct is not None else None) + tail + (int(variant),)
         keep = (pos_host, quat_host, out_host, rays, grid, work)  # the pointers above stay valid while the entry lives
         if len(_HOST_SCAN_CALLS) >= 64:
             _HOST_SCAN_CALLS.clear()
@@ -310,22 +348,37 @@ _HOST_SCAN_CALLS: dict = {}
 
 def height_scan_obs(pos_w: torch.Tensor, quat_w: torch.Tensor, rays, grid: ScanGridHandle, obs: torch.Tensor,
                     obs_bf16: torch.Tensor, head_cols: int = 4, max_distance: float = 100.0,
-                    base_offset: float = 0.26878, bf16_only: bool = False) -> None:
+                    base_offset: float = 0.26878, bf16_only: bool = False, variant: int | None = None,
+                    attach_yaw_only: bool = True) -> None:
     """Height scan into the observation buffers of the closed loop: heights -> ``obs[:, head_cols:head_cols + R]``
     (fp32) and the bf16 mirror of ``obs[:, :head_cols + R]`` -> ``obs_bf16`` (``policy.alloc_obs_bf16``), the operand
     of ``GaussianNeuralNetwork.compute_bf16``.  One launch (variant 5 with the extra stores).
     ``bf16_only``: only the mirror is written (``rover_height_scan_obs_bf16``) -- ``obs`` is read for its head columns and
     its height columns keep what they held; for loops in which the bf16 policy forward is the heights' only consumer.
-    The policy rounds fp32 observations to exactly these bf16 values, so actions and trajectory do not change."""
+    The policy rounds fp32 observations to exactly these bf16 values, so actions and trajectory do not change.
+    ``variant=6``: the same stores from the kernel of rays in any direction (``rover_ray_cast_obs``), one launch for any
+    pattern and either ``attach_yaw_only``; its heights equal ``height_scan(..., variant=6)`` bit for bit.  Otherwise
+    (``variant=None``) the rays must be vertical and yaw-only."""
     if not isinstance(rays, RayPattern):
         rays = RayPattern(rays, pos_w.device)
-    require_vertical("height_scan_obs", rays)
-    _lib.require_cuda(pos_w, quat_w)  # obs / obs_bf16 are row-strided views: checked below
+    if variant != RAY_CAST_VARIANT:
+        require_vertical("height_scan_obs", rays, attach_yaw_only, takes_variant=True)
+        if variant is not None:
+            raise RuntimeError(f"height_scan_obs: variant {variant}: pass variant=None (the vertical kernels) or 6")
+    dev = _lib.require_cuda(pos_w, quat_w)  # obs / obs_bf16 are row-strided views: checked below
     n = pos_w.shape[0]
     if (not obs.is_cuda or obs.dtype != torch.float32 or obs.shape[0] != n or obs.stride(1) != 1 or obs.shape[1] < head_cols + rays.n_rays
             or obs_bf16.dtype != torch.bfloat16 or obs_bf16.shape[0] != n or obs_bf16.stride(1) != 1
             or obs_bf16.shape[1] < head_cols + rays.n_rays or not obs_bf16.is_cuda):
         raise RuntimeError("height_scan_obs: obs must be fp32 and obs_bf16 bf16, both [N, >= head_cols + R] with unit inner stride")
+    if variant == RAY_CAST_VARIANT:
+        if grid.device != dev or grid.cells_struct is None:
+            raise RuntimeError("height_scan_obs: variant 6 needs a ScanGridHandle built with plane_cells=True on the "
+                               "tensors' device")
+        torch.ops.rover_b200.ray_cast_obs(pos_w, quat_w, rays.starts, rays.dirs, bool(attach_yaw_only), grid.desc,
+                                          grid.cells_desc, float(max_distance), float(base_offset), obs, int(head_cols),
+                                          obs_bf16, bool(bf16_only))
+        return
     torch.ops.rover_b200.height_scan_obs(pos_w, quat_w, rays.starts, rays.box_t, grid.desc, grid.cells_desc,
                                          float(max_distance), float(base_offset), obs, int(head_cols), obs_bf16, bool(bf16_only))
 

@@ -47,6 +47,12 @@ _SCHEMAS = {
     "height_scan_host": "(Tensor pos_host, Tensor quat_host, Tensor ray_starts, Tensor pattern_box, Tensor grid, "
                         "Tensor? cells, float max_distance, float base_offset, int variant, int n_slices, Tensor(a!) work, "
                         "Tensor(b!) out_host) -> ()",
+    "ray_cast_obs": "(Tensor pos_w, Tensor quat_w, Tensor ray_starts, Tensor ray_dirs, bool attach_yaw_only, Tensor grid, "
+                    "Tensor cells, float max_distance, float base_offset, Tensor(a!) obs, int head_cols, Tensor(b!) obs_bf16, "
+                    "bool bf16_only=False) -> ()",
+    "ray_cast_host": "(Tensor pos_host, Tensor quat_host, Tensor ray_starts, Tensor ray_dirs, bool attach_yaw_only, "
+                     "Tensor grid, Tensor cells, float max_distance, float base_offset, int n_slices, Tensor(a!) work, "
+                     "Tensor(b!) out_host) -> ()",
     # ---- fused MDP step (ackermann_actions.py:226-322, rewards.py:14-137, terminations.py:14-64, ...)
     "ackermann": "(Tensor actions, Tensor params) -> (Tensor, Tensor, Tensor)",
     "mdp_pre_step": "(Tensor? new_actions, Tensor? force_matrix_w, Tensor params, Tensor(a!)[] state, Tensor(b!)[] out, "
@@ -205,27 +211,33 @@ def _ray_cast_hits(pos_w, quat_w, ray_starts, pattern_box, grid, cells, max_dist
 _PINNED_SEEN: set = set()
 
 
-def _height_scan_host(pos_host, quat_host, ray_starts, pattern_box, grid, cells, max_distance, base_offset, variant, n_slices,
-                      work, out_host):
-    """Poses and heights in HOST memory (page-locked tensors), ray pattern / tables / work area on the device."""
+def _host_buffers(what, pos_host, quat_host, ray_starts, work, out_host):
+    """The checks of the host-buffer operators: page-locked fp32 poses / heights, the work area on the rays' device."""
     n, r = pos_host.shape[0], ray_starts.shape[0]
-    for t, shape, what in ((pos_host, (n, 3), "pos_host"), (quat_host, (n, 4), "quat_host")):
+    for t, shape, name in ((pos_host, (n, 3), "pos_host"), (quat_host, (n, 4), "quat_host")):
         if t.device.type != "cpu" or t.dtype != torch.float32 or t.shape != shape or not t.is_contiguous():
-            raise RuntimeError(f"rover_b200::height_scan_host: {what} must be a contiguous CPU fp32 {list(shape)} tensor")
+            raise RuntimeError(f"rover_b200::{what}: {name} must be a contiguous CPU fp32 {list(shape)} tensor")
     if (out_host.device.type != "cpu" or out_host.dtype != torch.float32 or out_host.dim() != 2 or out_host.shape[0] != n
             or out_host.shape[1] != r or out_host.stride(1) != 1):
-        raise RuntimeError("rover_b200::height_scan_host: out_host must be a CPU fp32 [N,R] tensor with unit inner stride")
+        raise RuntimeError(f"rover_b200::{what}: out_host must be a CPU fp32 [N,R] tensor with unit inner stride")
     for t in (pos_host, quat_host, out_host):  # is_pinned() asks the driver (~2 us): once per buffer, not once per step
         key = (t.data_ptr(), t.numel())
         if key not in _PINNED_SEEN:
             if not t.is_pinned():
-                raise RuntimeError("rover_b200::height_scan_host: host tensors must be page-locked (tensor.pin_memory())")
+                raise RuntimeError(f"rover_b200::{what}: host tensors must be page-locked (tensor.pin_memory())")
             if len(_PINNED_SEEN) > 4096:
                 _PINNED_SEEN.clear()
             _PINNED_SEEN.add(key)
-    _f32("height_scan_host", ray_starts)
+    _f32(what, ray_starts)
     if not work.is_cuda or work.dtype != torch.uint8 or not work.is_contiguous() or ray_starts.device != work.device:
-        raise RuntimeError("rover_b200::height_scan_host: work must be a contiguous CUDA uint8 tensor on the rays' device")
+        raise RuntimeError(f"rover_b200::{what}: work must be a contiguous CUDA uint8 tensor on the rays' device")
+    return n, r
+
+
+def _height_scan_host(pos_host, quat_host, ray_starts, pattern_box, grid, cells, max_distance, base_offset, variant, n_slices,
+                      work, out_host):
+    """Poses and heights in HOST memory (page-locked tensors), ray pattern / tables / work area on the device."""
+    n, r = _host_buffers("height_scan_host", pos_host, quat_host, ray_starts, work, out_host)
     if pattern_box.device.type != "cpu" or pattern_box.dtype != torch.float32 or pattern_box.numel() != 4:
         raise RuntimeError("rover_b200::height_scan_host: pattern_box must be a CPU fp32 tensor of 4 values")
     _lib.check(_lib.load().rover_height_scan_host(
@@ -250,6 +262,43 @@ def _height_scan_obs(pos_w, quat_w, ray_starts, pattern_box, grid, cells, max_di
         _desc(grid, _lib.ScanGrid, "grid"), _desc(cells, _lib.PlaneCells, "cells") if cells is not None else None,
         float(max_distance), float(base_offset), _p(obs), int(obs.stride(0)), int(head_cols), _p(obs_bf16),
         int(obs_bf16.stride(0)), _stream(pos_w)))
+
+
+def _ray_cast_host(pos_host, quat_host, ray_starts, ray_dirs, attach_yaw_only, grid, cells, max_distance, base_offset,
+                   n_slices, work, out_host):
+    """``height_scan_host`` with the kernel of rays in any direction (variant 6)."""
+    n, r = _host_buffers("ray_cast_host", pos_host, quat_host, ray_starts, work, out_host)
+    _f32("ray_cast_host", ray_dirs)
+    if ray_starts.shape != (r, 3) or ray_dirs.shape != (r, 3) or ray_dirs.device != work.device:
+        raise RuntimeError("rover_b200::ray_cast_host: ray_starts [R,3] and ray_dirs [R,3] on the work area's device expected")
+    _lib.check(_lib.load().rover_ray_cast_host(
+        _p(pos_host), _p(quat_host), n, _p(ray_starts), _p(ray_dirs), r, int(bool(attach_yaw_only)),
+        _desc(grid, _lib.ScanGrid, "grid"), _desc(cells, _lib.PlaneCells, "cells"), float(max_distance), float(base_offset),
+        _p(out_host), int(out_host.stride(0)) if n > 0 else r, _p(work), int(work.numel()), int(n_slices), _stream(work)))
+
+
+def _ray_cast_obs(pos_w, quat_w, ray_starts, ray_dirs, attach_yaw_only, grid, cells, max_distance, base_offset, obs,
+                  head_cols, obs_bf16, bf16_only=False):
+    """``height_scan_obs`` with the kernel of rays in any direction (variant 6): one launch, any ``head_cols >= 0``."""
+    _f32("ray_cast_obs", pos_w, quat_w, ray_starts, ray_dirs)
+    n, r = pos_w.shape[0], ray_starts.shape[0]
+    if pos_w.shape != (n, 3) or quat_w.shape != (n, 4) or ray_starts.shape != (r, 3) or ray_dirs.shape != (r, 3):
+        raise RuntimeError("rover_b200::ray_cast_obs: pos_w [N,3], quat_w [N,4], ray_starts [R,3], ray_dirs [R,3] expected")
+    if head_cols < 0:
+        raise RuntimeError("rover_b200::ray_cast_obs: head_cols must be >= 0")
+    if (obs.dtype != torch.float32 or obs.dim() != 2 or obs.shape[0] != n or obs.stride(1) != 1
+            or obs.shape[1] < head_cols + r or obs_bf16.dtype != torch.bfloat16 or obs_bf16.dim() != 2
+            or obs_bf16.shape[0] != n or obs_bf16.stride(1) != 1 or obs_bf16.shape[1] < head_cols + r):
+        raise RuntimeError("rover_b200::ray_cast_obs: obs must be fp32 and obs_bf16 bf16, both [N, >= head_cols + R] "
+                           "with unit inner stride")
+    if not all(t.is_cuda and t.device == pos_w.device for t in (pos_w, quat_w, ray_starts, ray_dirs, obs, obs_bf16)):
+        raise RuntimeError("rover_b200::ray_cast_obs: tensors must be CUDA tensors on one device")
+    entry = _lib.load().rover_ray_cast_obs_bf16 if bf16_only else _lib.load().rover_ray_cast_obs
+    _lib.check(entry(
+        _p(pos_w), _p(quat_w), n, _p(ray_starts), _p(ray_dirs), r, int(bool(attach_yaw_only)),
+        _desc(grid, _lib.ScanGrid, "grid"), _desc(cells, _lib.PlaneCells, "cells"), float(max_distance), float(base_offset),
+        _p(obs), int(obs.stride(0)) if n > 0 else head_cols + r, int(head_cols), _p(obs_bf16),
+        int(obs_bf16.stride(0)) if n > 0 else head_cols + r, _stream(pos_w)))
 
 
 # ----------------------------------------------------------------------------------------------------- MDP step
@@ -524,7 +573,8 @@ def _fill_holes(mask):
 _IMPLS = {
     "height_scan": _height_scan, "height_scan_out": _height_scan_out, "height_scan_hits": _height_scan_hits,
     "ray_cast": _ray_cast, "ray_cast_out": _ray_cast_out, "ray_cast_hits": _ray_cast_hits,
-    "height_scan_obs": _height_scan_obs, "height_scan_host": _height_scan_host, "ackermann": _ackermann, "mdp_pre_step": _mdp_pre_step,
+    "height_scan_obs": _height_scan_obs, "height_scan_host": _height_scan_host, "ray_cast_obs": _ray_cast_obs,
+    "ray_cast_host": _ray_cast_host, "ackermann": _ackermann, "mdp_pre_step": _mdp_pre_step,
     "mdp_post_step": _mdp_post_step, "mdp_step": _mdp_step, "step_fused": _step_fused, "stats_read": _stats_read, "policy_pack": _policy_pack,
     "policy_forward": _policy_forward, "policy_value_forward": _policy_value_forward, "gaussian_act": _gaussian_act,
     "gaussian_act_out": _gaussian_act_out, "policy_pack_fused": _policy_pack_fused,
@@ -612,7 +662,8 @@ def _fake_none(*args, **kwargs):
     return None
 
 
-for _name in ("height_scan_out", "ray_cast_out", "height_scan_obs", "height_scan_host", "gaussian_act_out", "mdp_pre_step", "mdp_post_step", "mdp_step", "step_fused", "stats_read", "policy_pack",
+for _name in ("height_scan_out", "ray_cast_out", "height_scan_obs", "height_scan_host", "ray_cast_obs", "ray_cast_host",
+              "gaussian_act_out", "mdp_pre_step", "mdp_post_step", "mdp_step", "step_fused", "stats_read", "policy_pack",
               "policy_pack_fused", "mesh_to_heightmap"):
     torch.library.register_fake(f"{NS}::{_name}", _fake_none, lib=_DEF)
 
