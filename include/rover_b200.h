@@ -498,6 +498,24 @@ int rover_gaussian_act(const float* mean, const float* log_std, const float* eps
                        float* log_prob, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------
+ * PPO returns and advantages.  Replaces skrl 1.1.0 PPO._update's compute_gae (agents/torch/ppo/ppo.py; third-party,
+ * restated in DESIGN.md section 2): the backward loop over the memory_size rows of the rollout memory, returns =
+ * advantages + values, then advantages normalised over all T * N entries.
+ *   rewards, values [T, n_envs] fp32 and dones [T, n_envs] uint8 (0 = not done), row-major (the memory's [T, N, 1]
+ *   tensors); last_values [n_envs]: the value network on the last next_states.  Per environment, i = T-1 .. 0:
+ *     adv = (rewards[i] - values[i]) + ((discount_factor * not_done[i]) * (nv + lambda_coefficient * adv)),
+ *   nv = values[i+1] (last_values for i = T-1), adv = 0 before the first step, every operation one fp32 rounding (no
+ *   contraction; a done step multiplies by 0, it does not branch).  returns = adv + values.  advantages receives
+ *   fl32(fl32(adv - mean_f) / fl32(std_f + 1e-8f)) with mean_f = fl32(sum / n), std_f = fl32(sqrt(M2 / (n - 1))) (NaN
+ *   for n = 1), sum and M2 = sum (adv - sum / n)^2 accumulated in fp64 in a fixed order: deterministic, graph-capturable.
+ *   `work`: device scratch of rover_ppo_gae_work_bytes(T, n_envs) bytes, 8-byte aligned.  Outputs must not overlap the
+ *   inputs or each other. */
+int64_t rover_ppo_gae_work_bytes(int32_t T, int32_t n_envs);
+int rover_ppo_gae(const float* rewards, const uint8_t* dones, const float* values, const float* last_values, int32_t T,
+                  int32_t n_envs, float discount_factor, float lambda_coefficient, float* returns, float* advantages,
+                  void* work, int64_t work_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------------------
  * Init-time terrain tables (SURVEY.md 8 f-3).  Not on the step path; built once per terrain.
  * rover_mesh_to_heightmap replaces mesh_to_heightmap (rover_envs/utils/terrains/terrain_utils.py:23-57): per face, the
  * cells covered by its XY bounding box take max(cell, max z of the face).  heightmap [rows, cols] fp32 must be

@@ -30,7 +30,7 @@ SYMBOLS = ("rover_abi_version", "rover_last_error", "rover_height_scan", "rover_
            "rover_value_forward_bf16", "rover_gaussian_act", "rover_mesh_to_heightmap", "rover_steep_mask",
            "rover_policy_pack_fused", "rover_scan_encoder_fused", "rover_policy_mlp_forward", "rover_morph_box",
            "rover_fill_holes", "rover_step_fused", "rover_ray_cast", "rover_ray_cast_obs", "rover_ray_cast_obs_bf16",
-           "rover_ray_cast_host")
+           "rover_ray_cast_host", "rover_ppo_gae", "rover_ppo_gae_work_bytes")
 
 
 class ScanLevel(C.Structure):
@@ -222,6 +222,10 @@ def load() -> C.CDLL:
     lib.rover_policy_mlp_forward.argtypes = [vp, i32, vp, vp, i32, vp]
     lib.rover_gaussian_act.restype = C.c_int
     lib.rover_gaussian_act.argtypes = [vp, vp, vp, i32, vp, vp, vp]
+    lib.rover_ppo_gae_work_bytes.restype = C.c_int64
+    lib.rover_ppo_gae_work_bytes.argtypes = [i32, i32]
+    lib.rover_ppo_gae.restype = C.c_int
+    lib.rover_ppo_gae.argtypes = [vp, vp, vp, vp, i32, i32, f32, f32, vp, vp, vp, C.c_int64, vp]
     _lib = lib
     return lib
 

@@ -83,6 +83,9 @@ _SCHEMAS = {
     "policy_value_forward": "(Tensor obs, Tensor packed_policy, Tensor packed_value) -> (Tensor, Tensor)",
     "gaussian_act": "(Tensor mean, Tensor log_std, Tensor eps) -> (Tensor, Tensor)",
     "gaussian_act_out": "(Tensor mean, Tensor log_std, Tensor eps, Tensor(a!) actions, Tensor(b!) log_prob) -> ()",
+    # ---- PPO returns and advantages over the rollout memory (skrl PPO._update -> compute_gae)
+    "ppo_gae": "(Tensor rewards, Tensor dones, Tensor values, Tensor last_values, float discount_factor, "
+               "float lambda_coefficient, Tensor(a!) returns, Tensor(b!) advantages) -> ()",
     # ---- init-time tables (terrain_utils.py:23-57, 265-279)
     "mesh_to_heightmap": "(Tensor vertices, Tensor faces, float min_x, float min_y, float cell_x, float cell_y, "
                          "Tensor(a!) heightmap, Tensor(b!) out_of_range) -> ()",
@@ -530,6 +533,44 @@ def _gaussian_act(mean, log_std, eps):
     return actions, log_prob
 
 
+# ----------------------------------------------------------------------------------------------------- PPO
+def _overlaps(a: torch.Tensor, b: torch.Tensor) -> bool:
+    if a.numel() == 0 or b.numel() == 0 or a.device != b.device:
+        return False
+    a0, b0 = a.data_ptr(), b.data_ptr()
+    return a0 < b0 + b.numel() * b.element_size() and b0 < a0 + a.numel() * a.element_size()
+
+
+def _ppo_gae(rewards, dones, values, last_values, discount_factor, lambda_coefficient, returns, advantages):
+    """The memory's ``[T, N]`` / ``[T, N, 1]`` tensors; ``last_values`` ``[N]`` / ``[N, 1]``."""
+    what = "rover_b200::ppo_gae"
+    ts = (rewards, dones, values, last_values, returns, advantages)
+    if not all(t.is_cuda and t.device == rewards.device for t in ts):
+        raise RuntimeError(f"{what}: every tensor must be a CUDA tensor on one device")
+    if not all(t.is_contiguous() for t in ts):
+        raise RuntimeError(f"{what}: contiguous tensors required")
+    if rewards.dim() not in (2, 3) or (rewards.dim() == 3 and rewards.shape[2] != 1):
+        raise RuntimeError(f"{what}: rewards must be [T, N] or [T, N, 1]")
+    t_, n = rewards.shape[0], rewards.shape[1]
+    for t, name in ((rewards, "rewards"), (values, "values"), (returns, "returns"), (advantages, "advantages")):
+        if t.dtype != torch.float32 or t.shape != rewards.shape:
+            raise RuntimeError(f"{what}: {name} must be fp32 of the rewards' shape {list(rewards.shape)}")
+    if dones.dtype not in (torch.bool, torch.uint8) or dones.shape != rewards.shape:
+        raise RuntimeError(f"{what}: dones must be bool or uint8 of the rewards' shape {list(rewards.shape)}")
+    if last_values.dtype != torch.float32 or last_values.shape not in ((n,), (n, 1)):
+        raise RuntimeError(f"{what}: last_values must be fp32 [N] or [N, 1] with N = {n}")
+    for out, name in ((returns, "returns"), (advantages, "advantages")):
+        if any(_overlaps(out, t) for t in (rewards, dones, values, last_values)):
+            raise RuntimeError(f"{what}: {name} overlaps an input")
+    if _overlaps(returns, advantages):
+        raise RuntimeError(f"{what}: returns and advantages overlap")
+    lib = _lib.load()
+    work = torch.empty(max(int(lib.rover_ppo_gae_work_bytes(t_, n)), 8), dtype=torch.uint8, device=rewards.device)
+    _lib.check(lib.rover_ppo_gae(_p(rewards), _p(dones), _p(values), _p(last_values), t_, n, float(discount_factor),
+                                 float(lambda_coefficient), _p(returns), _p(advantages), _p(work), int(work.numel()),
+                                 _stream(rewards)))
+
+
 # ----------------------------------------------------------------------------------------------------- init-time tables
 def _mesh_to_heightmap(vertices, faces, min_x, min_y, cell_x, cell_y, heightmap, out_of_range):
     _f32("mesh_to_heightmap", vertices, heightmap)
@@ -579,7 +620,7 @@ _IMPLS = {
     "policy_forward": _policy_forward, "policy_value_forward": _policy_value_forward, "gaussian_act": _gaussian_act,
     "gaussian_act_out": _gaussian_act_out, "policy_pack_fused": _policy_pack_fused,
     "scan_encoder_fused": _scan_encoder_fused, "policy_mlp_forward": _policy_mlp_forward, "mesh_to_heightmap": _mesh_to_heightmap,
-    "steep_mask": _steep_mask, "morph_box": _morph_box, "fill_holes": _fill_holes,
+    "steep_mask": _steep_mask, "morph_box": _morph_box, "fill_holes": _fill_holes, "ppo_gae": _ppo_gae,
 }
 for _name, _fn in _IMPLS.items():
     _IMPL.impl(_name, _fn)
@@ -664,7 +705,7 @@ def _fake_none(*args, **kwargs):
 
 for _name in ("height_scan_out", "ray_cast_out", "height_scan_obs", "height_scan_host", "ray_cast_obs", "ray_cast_host",
               "gaussian_act_out", "mdp_pre_step", "mdp_post_step", "mdp_step", "step_fused", "stats_read", "policy_pack",
-              "policy_pack_fused", "mesh_to_heightmap"):
+              "policy_pack_fused", "mesh_to_heightmap", "ppo_gae"):
     torch.library.register_fake(f"{NS}::{_name}", _fake_none, lib=_DEF)
 
 OPS = tuple(_SCHEMAS)

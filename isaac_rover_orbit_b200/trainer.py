@@ -1,12 +1,13 @@
 """The caller of the hot path: ``SkrlSequentialLogTrainer`` (reference rover_envs/utils/skrl_utils.py:42-206), the
 rollout storage it writes through the agent (skrl 1.1.0 ``Memory.add_samples``) and a small agent that samples
-actions with the tcgen05 policy -- SURVEY.md 8 (f-2).
+actions with the tcgen05 policy -- SURVEY.md 8 (f-2) -- and, for PPO, the returns and advantages skrl computes at the
+end of every rollout (``compute_gae``, ``PPORolloutAgent``; one CUDA pass over the memory, DESIGN.md 3.8).
 
 The trainer mirrors the reference call for call (same order, same keyword arguments, the double ``agents.init`` of
 ``__init__`` + ``train`` included), so that a maintainer can swap the import.  It is host-side glue: every tensor
 stays on the GPU, nothing here synchronises except the ``.item()`` calls the reference itself makes when it logs
 episode information (``log_episode_info=False`` skips them; ``RoverEnv`` keeps those statistics on the device anyway).
-PPO's optimisation step is outside the hot path and is not provided.
+PPO's optimisation step (minibatches, clipped surrogate, backward pass) is outside the hot path and is not provided.
 
 ``capture_steps`` records a step function into CUDA graphs (one per input variant) -- how ``bench.py`` runs
 act -> step -> record without per-launch host overhead.
@@ -16,6 +17,8 @@ from __future__ import annotations
 import copy
 
 import torch
+
+from . import torch_ops  # noqa: F401  (registers torch.ops.rover_b200.*, which the agents and compute_gae call)
 
 # skrl 1.1.0, skrl/trainers/torch/sequential.py (third-party, pinned by the reference's environment; restated)
 SEQUENTIAL_TRAINER_DEFAULT_CONFIG = {
@@ -182,6 +185,60 @@ class RolloutAgent(BaseAgent):
         if self.memory is not None:
             self.memory.add_samples(states=states, actions=actions, rewards=rewards, terminated=terminated,
                                     log_prob=self._log_prob, **({"values": self._values} if self.value is not None else {}))
+
+
+def compute_gae(rewards: torch.Tensor, dones: torch.Tensor, values: torch.Tensor, next_values: torch.Tensor,
+                discount_factor: float = 0.99, lambda_coefficient: float = 0.95):
+    """skrl 1.1.0 ``PPO._update.compute_gae`` (restated in DESIGN.md 2): ``(returns, advantages)`` of the memory's
+    ``[T, N, 1]`` (or ``[T, N]``) rewards / dones / values and the last values ``[N, 1]``, advantages normalised over all
+    ``T * N`` entries.  One ``rover_b200::ppo_gae`` call (three launches, no host synchronisation); returns bit-identical
+    to skrl's loop, the normalisation as DESIGN.md 2 states it."""
+    returns = torch.empty_like(rewards, memory_format=torch.contiguous_format)
+    advantages = torch.empty_like(rewards, memory_format=torch.contiguous_format)
+    torch.ops.rover_b200.ppo_gae(rewards.contiguous(), dones.contiguous(), values.contiguous(), next_values.contiguous(),
+                                 float(discount_factor), float(lambda_coefficient), returns, advantages)
+    return returns, advantages
+
+
+class PPORolloutAgent(RolloutAgent):
+    """``RolloutAgent`` plus what skrl 1.1.0's PPO does with the rollout before its optimisation epochs: it creates the
+    memory's ``returns`` / ``advantages`` (``PPO.init``), keeps the last ``next_states`` (``record_transition``) and, on
+    every ``memory_size``-th ``post_interaction`` (``_rollout % _rollouts``), evaluates the value network on them and
+    writes ``compute_gae`` of the memory into those tensors (``PPO._update``).  ``dones`` is the memory's ``terminated``,
+    as in skrl 1.1.0: a truncated step bootstraps from the next row's value.  The optimisation epochs are not provided."""
+
+    def __init__(self, policy, value, memory: RolloutMemory, discount_factor: float = 0.99, lambda_: float = 0.95,
+                 action_out: torch.Tensor | None = None):
+        if value is None or memory is None:
+            raise ValueError("PPORolloutAgent needs a value network and a memory")
+        super().__init__(policy, memory, value=value, action_out=action_out)
+        self.discount_factor = float(discount_factor)
+        self.lambda_ = float(lambda_)
+        self._rollout = 0
+        self._current_next_states = None
+        memory.create_tensor("returns", 1)
+        memory.create_tensor("advantages", 1)
+
+    def record_transition(self, states, actions, rewards, next_states, terminated, truncated, infos, timestep,
+                          timesteps) -> None:
+        super().record_transition(states, actions, rewards, next_states, terminated, truncated, infos, timestep, timesteps)
+        self._current_next_states = next_states
+
+    def post_interaction(self, timestep: int, timesteps: int) -> None:
+        self._rollout += 1
+        if self._rollout % self.memory.memory_size == 0:
+            self._update_returns()
+        super().post_interaction(timestep, timesteps)
+
+    def _update_returns(self) -> None:
+        mem = self.memory
+        with torch.no_grad():
+            # skrl passes next_states.float(); the value network gives the same values on bf16 and fp32 states
+            last_values = self.value.act({"states": self._current_next_states}, role="value")[0]
+            torch.ops.rover_b200.ppo_gae(mem.get_tensor_by_name("rewards"), mem.get_tensor_by_name("terminated"),
+                                         mem.get_tensor_by_name("values"), last_values.contiguous(), self.discount_factor,
+                                         self.lambda_, mem.get_tensor_by_name("returns"),
+                                         mem.get_tensor_by_name("advantages"))
 
 
 class SkrlSequentialLogTrainer:
