@@ -342,6 +342,14 @@ int rover_rng_variates(uint64_t seed, uint64_t step, int32_t n_envs, int32_t n_r
                        int64_t* spawn_by_env, float* yaw_u, float* heading_u, float* theta_u);
 /* HOST: one Philox4x32-10 block (Random123 known-answer vectors pin it: tests/test_rng_cpu.py) */
 int rover_philox4x32_10(const uint32_t counter[4], const uint32_t key[2], uint32_t out[4]);
+/* The MDP step's functions that are not correctly rounded, evaluated elementwise by the same device code the step kernels
+ * run (test support: an fp32 model of the step takes them from here, tests/mdp_exact.py).  DEVICE f32 arrays of n:
+ * ROVER_MDP_MATH_ATAN2: out = atan2f(a, b); ROVER_MDP_MATH_SIN: out = sinf(a); ROVER_MDP_MATH_COS: out = cosf(a)
+ * (b unused, may be NULL).  Asynchronous on `stream`. */
+#define ROVER_MDP_MATH_ATAN2 0
+#define ROVER_MDP_MATH_SIN 1
+#define ROVER_MDP_MATH_COS 2
+int rover_mdp_math(int32_t op, const float* a, const float* b, float* out, int32_t n, void* stream);
 
 /* rover_mdp_pre_step + rover_mdp_post_step_x in ONE launch, for callers whose physics does not sit between the two (the
  * synthetic-physics loop of bench.py; a simulator that hands over root state and contacts before the step): the reset

@@ -30,7 +30,7 @@ SYMBOLS = ("rover_abi_version", "rover_last_error", "rover_height_scan", "rover_
            "rover_value_forward_bf16", "rover_gaussian_act", "rover_mesh_to_heightmap", "rover_steep_mask",
            "rover_policy_pack_fused", "rover_scan_encoder_fused", "rover_policy_mlp_forward", "rover_morph_box",
            "rover_fill_holes", "rover_step_fused", "rover_ray_cast", "rover_ray_cast_obs", "rover_ray_cast_obs_bf16",
-           "rover_ray_cast_host", "rover_ppo_gae", "rover_ppo_gae_work_bytes")
+           "rover_ray_cast_host", "rover_ppo_gae", "rover_ppo_gae_work_bytes", "rover_mdp_math")
 
 
 class ScanLevel(C.Structure):
@@ -226,6 +226,8 @@ def load() -> C.CDLL:
     lib.rover_ppo_gae_work_bytes.argtypes = [i32, i32]
     lib.rover_ppo_gae.restype = C.c_int
     lib.rover_ppo_gae.argtypes = [vp, vp, vp, vp, i32, i32, f32, f32, vp, vp, vp, C.c_int64, vp]
+    lib.rover_mdp_math.restype = C.c_int
+    lib.rover_mdp_math.argtypes = [i32, vp, vp, vp, i32, vp]
     _lib = lib
     return lib
 
@@ -274,3 +276,17 @@ def rng_variates(seed: int, step: int, n_envs: int, n_rounds: int, n_spawns: int
     check(load().rover_rng_variates(C.c_uint64(seed), C.c_uint64(step), n_envs, n_rounds, n_spawns, sp.ctypes.data,
                                     yaw.ctypes.data, head.ctypes.data, theta.ctypes.data))
     return sp, yaw, head, theta
+
+
+MDP_MATH_ATAN2, MDP_MATH_SIN, MDP_MATH_COS = 0, 1, 2
+
+
+def mdp_math(op: int, a: torch.Tensor, b: torch.Tensor | None = None) -> torch.Tensor:
+    """``atan2f(a, b)``, ``sinf(a)`` or ``cosf(a)`` elementwise, by the device code of the MDP step kernels
+    (``rover_mdp_math``; test support).  ``a`` / ``b``: contiguous fp32 CUDA tensors of one shape."""
+    dev = require_cuda(a, b)
+    if a.dtype != torch.float32 or (b is not None and (b.dtype != torch.float32 or b.shape != a.shape)):
+        raise RuntimeError("mdp_math: fp32 tensors of one shape expected")
+    out = torch.empty_like(a)
+    check(load().rover_mdp_math(int(op), ptr(a), ptr(b), ptr(out), a.numel(), current_stream(dev)))
+    return out

@@ -686,15 +686,20 @@ __device__ __forceinline__ void post_env_work(int i, bool valid, bool reset, int
         if (phases & ROVER_PHASE_COMMAND) {
         // _update_command (terrain_importer.py:97-101): quat_rotate_inverse(yaw_quat(q), target - root)
         const float vx = __fsub_rn(cwx, px), vy = __fsub_rn(cwy, py), vz = __fsub_rn(cwz, pz);
+        // a - b + c with q_vec = (0, 0, sz): the products with the yaw quaternion's zero x / y components are kept -- they
+        // decide the sign of a zero result (pos_cmd_b.z of a level target with |yaw| > pi / 2 is -0 in ORBIT's formula)
         const YawQuat yq = yaw_quat(q.x, q.y, q.z, q.w);
         const float k = __fsub_rn(__fmul_rn(2.f, __fmul_rn(yq.cw, yq.cw)), 1.f);
-        const float b_x = __fmul_rn(__fmul_rn(-__fmul_rn(yq.sz, vy), yq.cw), 2.f);
-        const float b_y = __fmul_rn(__fmul_rn(__fmul_rn(yq.sz, vx), yq.cw), 2.f);
-        const float dot = __fmul_rn(yq.sz, vz);
+        const float zx = __fmul_rn(0.f, vx), zy = __fmul_rn(0.f, vy), zz = __fmul_rn(0.f, vz);
+        const float b_x = __fmul_rn(__fmul_rn(__fsub_rn(zz, __fmul_rn(yq.sz, vy)), yq.cw), 2.f);
+        const float b_y = __fmul_rn(__fmul_rn(__fsub_rn(__fmul_rn(yq.sz, vx), zz), yq.cw), 2.f);
+        const float b_z = __fmul_rn(__fmul_rn(__fsub_rn(zy, zx), yq.cw), 2.f);
+        const float dot = __fadd_rn(__fadd_rn(zx, zy), __fmul_rn(yq.sz, vz));
+        const float c_xy = __fmul_rn(__fmul_rn(0.f, dot), 2.f);
         const float c_z = __fmul_rn(__fmul_rn(yq.sz, dot), 2.f);
-        pbx = __fsub_rn(__fmul_rn(vx, k), b_x);
-        pby = __fsub_rn(__fmul_rn(vy, k), b_y);
-        const float pbz = __fadd_rn(__fmul_rn(vz, k), c_z);
+        pbx = __fadd_rn(__fsub_rn(__fmul_rn(vx, k), b_x), c_xy);
+        pby = __fadd_rn(__fsub_rn(__fmul_rn(vy, k), b_y), c_xy);
+        const float pbz = __fadd_rn(__fsub_rn(__fmul_rn(vz, k), b_z), c_z);
         S.pos_cmd_b[3 * (size_t)i] = pbx;
         S.pos_cmd_b[3 * (size_t)i + 1] = pby;
         S.pos_cmd_b[3 * (size_t)i + 2] = pbz;

@@ -819,6 +819,27 @@ extern "C" int rover_philox4x32_10(const uint32_t counter[4], const uint32_t key
     return 0;
 }
 
+// The step's three functions that are not correctly rounded (atan2f, sinf, cosf), evaluated elementwise by the device code
+// the step kernels run (this translation unit's flags and libdevice): an fp32 model of the step takes them from here.
+__global__ void mdp_math_kernel(int op, const float* __restrict__ a, const float* __restrict__ b, float* __restrict__ out,
+                                int n) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float x = a[i];
+    out[i] = op == ROVER_MDP_MATH_ATAN2 ? atan2f(x, b[i]) : (op == ROVER_MDP_MATH_SIN ? sinf(x) : cosf(x));
+}
+
+extern "C" int rover_mdp_math(int32_t op, const float* a, const float* b, float* out, int32_t n, void* stream) {
+    using namespace rover;
+    ROVER_CHECK(op == ROVER_MDP_MATH_ATAN2 || op == ROVER_MDP_MATH_SIN || op == ROVER_MDP_MATH_COS,
+                "rover_mdp_math: op must be ROVER_MDP_MATH_ATAN2, _SIN or _COS");
+    ROVER_CHECK(n >= 0, "rover_mdp_math: negative n");
+    if (n == 0) return 0;
+    ROVER_CHECK(a && out && (b || op != ROVER_MDP_MATH_ATAN2), "rover_mdp_math: NULL argument");
+    mdp_math_kernel<<<(n + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream)>>>(op, a, b, out, n);
+    return check_launch("mdp_math_kernel");
+}
+
 __global__ void __launch_bounds__(ROVER_MDP_BLOCK) stats_publish_kernel(const __grid_constant__ rover::StatsExchangeDev X) {
     __shared__ rover::MdpShared sh;
     const int tid = (int)threadIdx.x;
