@@ -504,6 +504,31 @@ int rover_policy_mlp_forward(const uint16_t* enc_bf16, int32_t n_envs, const voi
 /* actions = clamp(mean + exp(clamp(log_std,-20,2)) * eps, -1, 1); log_prob [N] = sum_j log N(a_j) */
 int rover_gaussian_act(const float* mean, const float* log_std, const float* eps, int32_t n_envs, float* actions,
                        float* log_prob, void* stream);
+/* The forward pass with skrl 1.1.0 GaussianMixin.act in its last epilogue (models.py:39-102; SURVEY.md A.4): ONE launch
+ * writes mean [N,2] (outputs["mean_actions"]), actions [N,2] and log_prob [N] (NULL: not written), where
+ *   eps[i] = normal2({seed, step}, env_offset + i)   (Philox4x32-10 + Box-Muller, csrc/rng.cuh; two N(0,1) per env)
+ * and actions / log_prob are what rover_gaussian_act gives for (mean, log_std, eps) -- the same device function, the
+ * same bits.  The noise of env i depends on (seed, step, env_offset + i) only: not on n_envs, not on torch's generator.
+ *   rng_state: device int64[2] {seed, step}, 8-byte aligned.  The launch reads it after the kernel in front of it has
+ *     finished and leaves step + 1 (graph-capturable; step must stay below 2^40 - 1: while the launch runs, bits 40..63
+ *     of the step word count its blocks).  Same distribution as torch.randn, not the same numbers (by design).
+ *   env_offset >= 0, env_offset + n_envs <= 2^32: the first env's index in the noise stream (a shard of a larger batch).
+ *   log_std [2] fp32 (the raw parameter; clamped to [-20, 2] as rover_gaussian_act does).  mean, actions 8-byte aligned.
+ * rover_policy_value_act also writes value [N] of the value network, as rover_policy_value_forward does. */
+int rover_policy_act(const float* obs, int32_t obs_stride, int32_t n_envs, const void* packed, const float* log_std,
+                     int64_t* rng_state, int32_t env_offset, float* mean, float* actions, float* log_prob, void* stream);
+int rover_policy_act_bf16(const uint16_t* obs_bf16, int32_t stride, int32_t n_envs, const void* packed,
+                          const float* log_std, int64_t* rng_state, int32_t env_offset, float* mean, float* actions,
+                          float* log_prob, void* stream);
+int rover_policy_value_act(const float* obs, int32_t obs_stride, int32_t n_envs, const void* packed_policy,
+                           const void* packed_value, const float* log_std, int64_t* rng_state, int32_t env_offset,
+                           float* mean, float* value, float* actions, float* log_prob, void* stream);
+/* The eps [N,2] (8-byte aligned) that the next rover_policy_*act launch with rng_state and env_offset draws, computed on
+ * the device with the same code (host libm's log / sin / cos round differently).  advance != 0: the step advances by one
+ * as an act launch would; advance == 0 leaves rng_state unchanged.  Feed it to rover_gaussian_act to reproduce an act
+ * launch (GaussianMixin.act with explicit noise). */
+int rover_action_noise(int64_t* rng_state, int32_t env_offset, int32_t n_envs, float* eps_out, int32_t advance,
+                       void* stream);
 
 /* ---------------------------------------------------------------------------------------------------
  * PPO returns and advantages.  Replaces skrl 1.1.0 PPO._update's compute_gae (agents/torch/ppo/ppo.py; third-party,

@@ -30,7 +30,8 @@ SYMBOLS = ("rover_abi_version", "rover_last_error", "rover_height_scan", "rover_
            "rover_value_forward_bf16", "rover_gaussian_act", "rover_mesh_to_heightmap", "rover_steep_mask",
            "rover_policy_pack_fused", "rover_scan_encoder_fused", "rover_policy_mlp_forward", "rover_morph_box",
            "rover_fill_holes", "rover_step_fused", "rover_ray_cast", "rover_ray_cast_obs", "rover_ray_cast_obs_bf16",
-           "rover_ray_cast_host", "rover_ppo_gae", "rover_ppo_gae_work_bytes", "rover_mdp_math")
+           "rover_ray_cast_host", "rover_ppo_gae", "rover_ppo_gae_work_bytes", "rover_mdp_math", "rover_policy_act",
+           "rover_policy_act_bf16", "rover_policy_value_act", "rover_action_noise")
 
 
 class ScanLevel(C.Structure):
@@ -228,6 +229,13 @@ def load() -> C.CDLL:
     lib.rover_ppo_gae.argtypes = [vp, vp, vp, vp, i32, i32, f32, f32, vp, vp, vp, C.c_int64, vp]
     lib.rover_mdp_math.restype = C.c_int
     lib.rover_mdp_math.argtypes = [i32, vp, vp, vp, i32, vp]
+    for fn in (lib.rover_policy_act, lib.rover_policy_act_bf16):
+        fn.restype = C.c_int
+        fn.argtypes = [vp, i32, i32, vp, vp, vp, i32, vp, vp, vp, vp]
+    lib.rover_policy_value_act.restype = C.c_int
+    lib.rover_policy_value_act.argtypes = [vp, i32, i32, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp]
+    lib.rover_action_noise.restype = C.c_int
+    lib.rover_action_noise.argtypes = [vp, i32, i32, vp, i32, vp]
     _lib = lib
     return lib
 

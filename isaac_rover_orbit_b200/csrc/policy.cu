@@ -320,18 +320,25 @@ __global__ void gaussian_act_kernel(const float* __restrict__ mean, const float*
     grid_dependency_wait();  // launched as a programmatic dependent of the forward pass (common.cuh)
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    float lp = 0.f;
-#pragma unroll
-    for (int j = 0; j < 2; ++j) {
-        const float ls = fminf(fmaxf(__ldg(log_std + j), -20.f), 2.f);
-        const float sd = expf(ls);
-        const float m = mean[2 * i + j];
-        const float a = fminf(fmaxf(fmaf(sd, eps[2 * i + j], m), -1.f), 1.f);
-        actions[2 * i + j] = a;
-        const float d = a - m;
-        lp += -(d * d) / (2.f * sd * sd) - ls - 0.91893853320467274178f;
-    }
+    const float m[2] = {mean[2 * i], mean[2 * i + 1]};
+    const float ls[2] = {__ldg(log_std), __ldg(log_std + 1)};
+    const float e[2] = {eps[2 * i], eps[2 * i + 1]};
+    float a[2];
+    const float lp = gaussian_sample(m, ls, e, a);
+    actions[2 * i] = a[0];
+    actions[2 * i + 1] = a[1];
     if (log_prob) log_prob[i] = lp;
+}
+
+// eps [N, 2] that the next sampling launch with this {seed, step} draws (rover_action_noise); advance: take the step
+__global__ void action_noise_kernel(unsigned long long* __restrict__ rng, uint32_t env_offset, int n, float* __restrict__ eps,
+                                    int advance) {
+    __shared__ RngKey key;
+    grid_dependency_wait();
+    if (threadIdx.x == 0) key = take_step(rng, gridDim.x, advance != 0);
+    __syncthreads();
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+        *reinterpret_cast<float2*>(eps + 2 * (size_t)i) = normal2(key, env_offset + (uint32_t)i);
 }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
@@ -340,7 +347,7 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
 
 int launch_policy_forward_ws(const void* obs, int obs_stride, int n_envs, const void* packed, float* out,
                              bool value_head, bool bf16_in, cudaStream_t stream, const void* packed2 = nullptr,
-                             float* value2 = nullptr);  // policy_ws.cu
+                             float* value2 = nullptr, const SampleArgs* sample = nullptr);  // policy_ws.cu
 
 }  // namespace rover
 
@@ -472,4 +479,88 @@ extern "C" int rover_gaussian_act(const float* mean, const float* log_std, const
     ROVER_CUDA(launch_overlapped(gaussian_act_kernel, dim3((n_envs + 255) / 256), dim3(256), 0, static_cast<cudaStream_t>(stream),
                                  mean, log_std, eps, (int)n_envs, actions, log_prob));
     return check_launch("gaussian_act_kernel");
+}
+
+// ---------------------------------------------------------------------------------------------------- sampling in the pass
+static int check_act_args(const char* who, int32_t n_envs, const void* packed, const float* log_std, const int64_t* rng_state,
+                          int32_t env_offset, const float* mean, const float* actions) {
+    using namespace rover;
+    ROVER_CHECK(packed && log_std && rng_state && mean && actions, "%s: NULL argument", who);
+    ROVER_CHECK(env_offset >= 0, "%s: env_offset must be >= 0 (got %d)", who, env_offset);
+    ROVER_CHECK((uint64_t)env_offset + (uint64_t)n_envs <= (1ull << 32), "%s: env_offset + n_envs exceeds 2^32", who);
+    ROVER_CHECK((reinterpret_cast<uintptr_t>(packed) & 127) == 0, "%s: packed blob not 128B aligned", who);
+    ROVER_CHECK((reinterpret_cast<uintptr_t>(rng_state) & 7) == 0 && (reinterpret_cast<uintptr_t>(log_std) & 3) == 0,
+                "%s: rng_state must be 8-byte and log_std 4-byte aligned", who);
+    ROVER_CHECK((reinterpret_cast<uintptr_t>(mean) & 7) == 0 && (reinterpret_cast<uintptr_t>(actions) & 7) == 0,
+                "%s: mean and actions must be 8-byte aligned [N, 2] arrays", who);
+    return 0;
+}
+
+extern "C" int rover_policy_act(const float* obs, int32_t obs_stride, int32_t n_envs, const void* packed, const float* log_std,
+                                int64_t* rng_state, int32_t env_offset, float* mean, float* actions, float* log_prob,
+                                void* stream) {
+    using namespace rover;
+    ROVER_CHECK(n_envs >= 0, "rover_policy_act: negative n_envs");
+    if (n_envs == 0) return 0;
+    ROVER_CHECK(obs != nullptr, "rover_policy_act: NULL argument");
+    if (int rc = check_act_args("rover_policy_act", n_envs, packed, log_std, rng_state, env_offset, mean, actions)) return rc;
+    ROVER_CHECK(obs_stride >= kObsCols && obs_stride % 4 == 0 && (reinterpret_cast<uintptr_t>(obs) & 15) == 0,
+                "rover_policy_act: obs rows must be 16-byte aligned (obs_stride %% 4 == 0, got %d); allocate the "
+                "observation buffer with ops.alloc_obs()", obs_stride);
+    const SampleArgs s{log_std, reinterpret_cast<unsigned long long*>(rng_state), (uint32_t)env_offset, actions, log_prob};
+    return launch_policy_forward_ws(obs, obs_stride, n_envs, packed, mean, false, false, static_cast<cudaStream_t>(stream),
+                                    nullptr, nullptr, &s);
+}
+
+extern "C" int rover_policy_act_bf16(const uint16_t* obs_bf16, int32_t stride, int32_t n_envs, const void* packed,
+                                     const float* log_std, int64_t* rng_state, int32_t env_offset, float* mean, float* actions,
+                                     float* log_prob, void* stream) {
+    using namespace rover;
+    ROVER_CHECK(n_envs >= 0, "rover_policy_act_bf16: negative n_envs");
+    if (n_envs == 0) return 0;
+    ROVER_CHECK(obs_bf16 != nullptr, "rover_policy_act_bf16: NULL argument");
+    if (int rc = check_act_args("rover_policy_act_bf16", n_envs, packed, log_std, rng_state, env_offset, mean, actions)) return rc;
+    ROVER_CHECK(stride >= kObsCols && stride % 8 == 0 && (reinterpret_cast<uintptr_t>(obs_bf16) & 15) == 0,
+                "rover_policy_act_bf16: bf16 observation rows must be 16-byte aligned (stride %% 8 == 0, got %d)", stride);
+    const SampleArgs s{log_std, reinterpret_cast<unsigned long long*>(rng_state), (uint32_t)env_offset, actions, log_prob};
+    return launch_policy_forward_ws(obs_bf16, stride, n_envs, packed, mean, false, true, static_cast<cudaStream_t>(stream),
+                                    nullptr, nullptr, &s);
+}
+
+extern "C" int rover_policy_value_act(const float* obs, int32_t obs_stride, int32_t n_envs, const void* packed_policy,
+                                      const void* packed_value, const float* log_std, int64_t* rng_state, int32_t env_offset,
+                                      float* mean, float* value, float* actions, float* log_prob, void* stream) {
+    using namespace rover;
+    ROVER_CHECK(n_envs >= 0, "rover_policy_value_act: negative n_envs");
+    if (n_envs == 0) return 0;
+    ROVER_CHECK(obs && packed_value && value, "rover_policy_value_act: NULL argument");
+    if (int rc = check_act_args("rover_policy_value_act", n_envs, packed_policy, log_std, rng_state, env_offset, mean, actions))
+        return rc;
+    ROVER_CHECK(obs_stride >= kObsCols && obs_stride % 4 == 0 && (reinterpret_cast<uintptr_t>(obs) & 15) == 0,
+                "rover_policy_value_act: obs rows must be 16-byte aligned (obs_stride %% 4 == 0, got %d); allocate the "
+                "observation buffer with ops.alloc_obs()", obs_stride);
+    ROVER_CHECK((reinterpret_cast<uintptr_t>(packed_value) & 127) == 0, "rover_policy_value_act: packed blob not 128B aligned");
+    const SampleArgs s{log_std, reinterpret_cast<unsigned long long*>(rng_state), (uint32_t)env_offset, actions, log_prob};
+    return launch_policy_forward_ws(obs, obs_stride, n_envs, packed_policy, mean, false, false, static_cast<cudaStream_t>(stream),
+                                    packed_value, value, &s);
+}
+
+extern "C" int rover_action_noise(int64_t* rng_state, int32_t env_offset, int32_t n_envs, float* eps_out, int32_t advance,
+                                  void* stream) {
+    using namespace rover;
+    ROVER_CHECK(n_envs >= 0, "rover_action_noise: negative n_envs");
+    ROVER_CHECK(env_offset >= 0, "rover_action_noise: env_offset must be >= 0 (got %d)", env_offset);
+    ROVER_CHECK(rng_state && (eps_out || n_envs == 0), "rover_action_noise: NULL argument");
+    ROVER_CHECK((reinterpret_cast<uintptr_t>(rng_state) & 7) == 0 && (reinterpret_cast<uintptr_t>(eps_out) & 7) == 0,
+                "rover_action_noise: rng_state and eps_out must be 8-byte aligned");
+    int blocks = (n_envs + 255) / 256;
+    if (blocks > 1024) blocks = 1024;
+    if (blocks == 0) {
+        if (!advance) return 0;
+        blocks = 1;  // nothing to draw, but the step still advances
+    }
+    ROVER_CUDA(launch_overlapped(action_noise_kernel, dim3(blocks), dim3(256), 0, static_cast<cudaStream_t>(stream),
+                                 reinterpret_cast<unsigned long long*>(rng_state), (uint32_t)env_offset, (int)n_envs, eps_out,
+                                 (int)(advance != 0)));
+    return check_launch("action_noise_kernel");
 }

@@ -7,6 +7,7 @@
 #include <cstdlib>
 
 #include "common.cuh"
+#include "rng.cuh"
 
 namespace rover {
 
@@ -122,6 +123,35 @@ __device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
     return *reinterpret_cast<uint32_t*>(&h);
 }
 __device__ __forceinline__ float leaky(float x) { return x > 0.f ? x : 0.01f * x; }
+
+// skrl 1.1.0 GaussianMixin.act for one environment (models.py:65-67: clip_log_std, min -20, max 2): log_std clamped to
+// [-20, 2], the reparameterised sample mean + std * eps clipped to the action box [-1, 1], log-prob of the clipped action
+// under Normal(mean, std) summed over the two action dimensions.  Shared by gaussian_act_kernel and the sampling
+// epilogue of the forward pass, so both give the same bits.
+__device__ __forceinline__ float gaussian_sample(const float (&mean)[2], const float (&log_std)[2], const float (&eps)[2],
+                                                 float (&actions)[2]) {
+    float lp = 0.f;
+#pragma unroll
+    for (int j = 0; j < 2; ++j) {
+        const float ls = fminf(fmaxf(log_std[j], -20.f), 2.f);
+        const float sd = expf(ls);
+        const float m = mean[j];
+        const float a = fminf(fmaxf(fmaf(sd, eps[j], m), -1.f), 1.f);
+        actions[j] = a;
+        const float d = a - m;
+        lp += -(d * d) / (2.f * sd * sd) - ls - 0.91893853320467274178f;
+    }
+    return lp;
+}
+
+// What the forward pass needs to sample in its last epilogue (rover_policy_act): eps = normal2({seed, step}, env_offset + env)
+struct SampleArgs {
+    const float* log_std;      // [2]
+    unsigned long long* rng;   // {seed, step}, advanced once per launch
+    uint32_t env_offset;
+    float* actions;            // [N, 2]
+    float* log_prob;           // [N] or nullptr
+};
 
 constexpr int kWsPlane = kTileM * 16;  // bytes between K-adjacent core matrices of a 128-row A operand (SWIZZLE_NONE)
 

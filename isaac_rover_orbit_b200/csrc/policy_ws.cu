@@ -97,11 +97,16 @@ static_assert(kTileM * kBfChunkK * 2 == kTileM * kWsChunkK * 4, "both modes use 
 
 // kDual: `packed` = policy, `packed2` = value network, outputs `mean` [N, 2] and `value2` [N]; else one network
 // (value_head: linear [N] output instead of tanh [N, 2]).
-template <bool kBf16In, bool kDual = false>
+// kSample (policy head): the last epilogue also samples skrl's GaussianMixin.act -- eps = normal2({seed, step},
+// env_offset + env) in registers, then gaussian_sample(), the function gaussian_act_kernel runs -- and stores `actions`
+// and `log_prob` beside `mean`.  {seed, step} is taken once per CTA after griddepcontrol.wait; the launch advances the
+// step once (rng.cuh, take_step).
+template <bool kBf16In, bool kDual = false, bool kSample = false>
 __global__ void __launch_bounds__(kBf16In ? kWsThreads : kWsThreadsF32, 1)
 policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const float* __restrict__ obs, int obs_stride,
                          int n_envs, int tile_rows, const unsigned char* __restrict__ packed, float* __restrict__ mean,
-                         int value_head, const unsigned char* __restrict__ packed2, float* __restrict__ value2) {
+                         int value_head, const unsigned char* __restrict__ packed2, float* __restrict__ value2,
+                         const __grid_constant__ SampleArgs sample) {
     static_assert(!(kDual && kBf16In), "the two-network pass reads fp32 observations");
     using Smem = WsSmemT<kDual>;
     constexpr int kNets = Smem::kNets, kStagesFK = Smem::kStagesFT;
@@ -174,6 +179,7 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem = sm.tmem_base;
+    __shared__ RngKey s_key;    // kSample: {seed, step} of this launch (unused otherwise)
     grid_dependency_wait();     // every thread, before anything of the predecessor's is read or `mean` is written
     grid_dependency_trigger();  // (the sampling kernel behind this one only saves its launch latency)
 
@@ -371,6 +377,7 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
 #pragma unroll
                 for (int k = 0; k < kPer; ++k)
                     if (tid + 128 * k < kWsBiasFloats) sm.bias[net][tid + 128 * k] = b[net][k];
+            if (kSample && tid == 0) s_key = take_step(sample.rng, gridDim.x, true);  // (after griddepcontrol.wait above)
             layer_group_sync();
         }
         // layer 2's input operand: planes 0.. (one network), planes 24..31 in the two-network pass, where layer 2 runs
@@ -498,6 +505,15 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
                         m.x = tanhf(v[0] + b5[0]);
                         m.y = tanhf(v[1] + b5[1]);
                         *reinterpret_cast<float2*>(dst + 2 * (size_t)grow) = m;
+                        if (kSample) {  // GaussianMixin.act on the mean just computed (the policy is network 0)
+                            const float2 e2 = normal2(s_key, sample.env_offset + (uint32_t)grow);
+                            const float mm[2] = {m.x, m.y}, e[2] = {e2.x, e2.y};
+                            const float ls[2] = {__ldg(sample.log_std), __ldg(sample.log_std + 1)};
+                            float a[2];
+                            const float lp = gaussian_sample(mm, ls, e, a);
+                            *reinterpret_cast<float2*>(sample.actions + 2 * (size_t)grow) = make_float2(a[0], a[1]);
+                            if (sample.log_prob != nullptr) sample.log_prob[grow] = lp;
+                        }
                     }
                 }
                 LDBG(13);
@@ -528,13 +544,16 @@ typedef CUresult (*WsEncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_
 // obs: fp32 [N, obs_stride] (bf16_in == false) or bf16 [N, obs_stride] (bf16_in == true; strides in elements).
 // packed2 != nullptr (fp32 observations only): policy (`packed` -> mean [N, 2]) and value network (`packed2` -> value2 [N])
 // in one pass over the observation.
+// sample != nullptr (policy head): the pass also samples the actions (kSample).
 int launch_policy_forward_ws(const void* obs, int obs_stride, int n_envs, const void* packed, float* mean,
-                             bool value_head, bool bf16_in, cudaStream_t stream, const void* packed2, float* value2) {
+                             bool value_head, bool bf16_in, cudaStream_t stream, const void* packed2, float* value2,
+                             const SampleArgs* sample) {
     static WsEncodeTiledFn encode = nullptr;
     static int n_sms = 0;
     constexpr int kSmemBytes = (int)sizeof(WsSmem) + 1024, kSmemBytesDual = (int)sizeof(WsSmemT<true>) + 1024;
     const bool dual = packed2 != nullptr;
     ROVER_CHECK(!(dual && (bf16_in || value2 == nullptr || value_head)), "policy + value pass: fp32 observations, two outputs");
+    ROVER_CHECK(!(sample && value_head), "sampling needs the policy head");
     if (!encode) {
         int dev = 0;
         ROVER_CUDA(cudaGetDevice(&dev));
@@ -542,6 +561,12 @@ int launch_policy_forward_ws(const void* obs, int obs_stride, int n_envs, const 
         ROVER_CUDA(cudaFuncSetAttribute(policy_forward_ws_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
         ROVER_CUDA(cudaFuncSetAttribute(policy_forward_ws_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
         ROVER_CUDA(cudaFuncSetAttribute(policy_forward_ws_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        kSmemBytesDual));
+        ROVER_CUDA(cudaFuncSetAttribute(policy_forward_ws_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        kSmemBytes));
+        ROVER_CUDA(cudaFuncSetAttribute(policy_forward_ws_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        kSmemBytes));
+        ROVER_CUDA(cudaFuncSetAttribute(policy_forward_ws_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                         kSmemBytesDual));
         void* fn = nullptr;
         cudaDriverEntryPointQueryResult q;
@@ -571,20 +596,21 @@ int launch_policy_forward_ws(const void* obs, int obs_stride, int n_envs, const 
     const int grid = n_tiles < n_sms ? n_tiles : n_sms;
     const unsigned char* no_net = nullptr;
     float* no_out = nullptr;
-    if (dual)
-        ROVER_CUDA(launch_overlapped(policy_forward_ws_kernel<false, true>, dim3(grid), dim3(kWsThreadsF32), (size_t)kSmemBytesDual,
-                                     stream, map, static_cast<const float*>(obs), obs_stride, n_envs, tile_rows,
-                                     static_cast<const unsigned char*>(packed), mean, 0,
-                                     static_cast<const unsigned char*>(packed2), value2));
-    else if (bf16_in)
-        ROVER_CUDA(launch_overlapped(policy_forward_ws_kernel<true>, dim3(grid), dim3(kWsThreads), (size_t)kSmemBytes, stream, map,
-                                     static_cast<const float*>(obs), obs_stride, n_envs, tile_rows,
-                                     static_cast<const unsigned char*>(packed), mean, value_head ? 1 : 0, no_net, no_out));
-    else
-        ROVER_CUDA(launch_overlapped(policy_forward_ws_kernel<false>, dim3(grid), dim3(kWsThreadsF32), (size_t)kSmemBytes, stream, map,
-                                     static_cast<const float*>(obs), obs_stride, n_envs, tile_rows,
-                                     static_cast<const unsigned char*>(packed), mean, value_head ? 1 : 0, no_net, no_out));
-    return check_launch("policy_forward_ws_kernel");
+    const SampleArgs sa = sample ? *sample : SampleArgs{nullptr, nullptr, 0u, nullptr, nullptr};
+    // kernel<kBf16In, kDual, kSample>: one launch of the instantiation the arguments select
+    auto launch = [&](auto kernel, int threads, int smem) {
+        return launch_overlapped(kernel, dim3(grid), dim3(threads), (size_t)smem, stream, map, static_cast<const float*>(obs),
+                                 obs_stride, n_envs, tile_rows, static_cast<const unsigned char*>(packed), mean,
+                                 value_head ? 1 : 0, dual ? static_cast<const unsigned char*>(packed2) : no_net,
+                                 dual ? value2 : no_out, sa);
+    };
+    if (dual && sample) ROVER_CUDA(launch(policy_forward_ws_kernel<false, true, true>, kWsThreadsF32, kSmemBytesDual));
+    else if (dual) ROVER_CUDA(launch(policy_forward_ws_kernel<false, true>, kWsThreadsF32, kSmemBytesDual));
+    else if (bf16_in && sample) ROVER_CUDA(launch(policy_forward_ws_kernel<true, false, true>, kWsThreads, kSmemBytes));
+    else if (bf16_in) ROVER_CUDA(launch(policy_forward_ws_kernel<true>, kWsThreads, kSmemBytes));
+    else if (sample) ROVER_CUDA(launch(policy_forward_ws_kernel<false, false, true>, kWsThreadsF32, kSmemBytes));
+    else ROVER_CUDA(launch(policy_forward_ws_kernel<false>, kWsThreadsF32, kSmemBytes));
+    return check_launch(sample ? "policy_forward_ws_kernel (sampling)" : "policy_forward_ws_kernel");
 }
 
 }  // namespace rover

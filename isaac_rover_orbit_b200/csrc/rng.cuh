@@ -17,6 +17,13 @@
 // evaluated at K distinct env ids has the same distribution (K distinct, uniformly drawn rows) and needs no reset rank --
 // no cross-block prefix sum in front of the reset chain.
 // The same functions are compiled for the host (rover_rng_variates) so that the oracle consumes identical numbers.
+//
+// The policy's action noise (skrl GaussianMixin.act: torch.randn(N, 2) -> Normal.rsample) comes from the same
+// generator with its own {seed, step} state and its own stream:
+//   counter = (env, step_lo, step_hi, kActionStream)    -> normal2(): two N(0, 1) draws by Box-Muller
+// kActionStream lies outside the reset path's streams (0 and 1 + q, q < 1024) and the spawn key's 0xffffffff.  Same
+// distribution as torch's draw, not the same numbers: the same documented deviation, by design, as the spawn permutation.
+// normal2 is device code only (logf / sinf / cosf of the host's libm round differently; rover_action_noise exports it).
 #pragma once
 #include <stdint.h>
 
@@ -103,5 +110,41 @@ ROVER_HD uint32_t spawn_perm_at(const SpawnPermKey& p, uint32_t j) {
     } while (x >= p.n);
     return x;
 }
+
+constexpr uint32_t kActionStream = 0x80000000u;
+
+#if defined(__CUDACC__)
+// Two standard-normal fp32 values of env `env`: Box-Muller on the first two words of one Philox4x32-10 call.
+//   u1 = (24 bits + 1) * 2^-24 in (0, 1]   (log never sees 0)      u2 = 24 bits * 2^-24 in [0, 1)
+//   r = sqrt(-2 ln u1),  z0 = r cos(2 pi u2),  z1 = r sin(2 pi u2)
+// Every operation is written out with its rounding (no contraction left to the compiler).  The angle goes to
+// sincospif(2 u2) = (sin, cos)(pi * 2 u2): 2 u2 is exact, so no rounded 2 pi enters, and the argument is known to be
+// small -- sinf / cosf of 2 pi u2 would carry the large-argument reduction (a local-memory frame) into the forward pass.
+__device__ __forceinline__ float2 normal2(const RngKey& k, uint32_t env) {
+    uint32_t w[4];
+    rng_env_stream(k, env, kActionStream, w);
+    const float u1 = __fmul_rn((float)((w[0] >> 8) + 1u), 5.9604644775390625e-8f);
+    const float u2 = __fmul_rn((float)(w[1] >> 8), 5.9604644775390625e-8f);
+    const float r = __fsqrt_rn(__fmul_rn(-2.f, logf(u1)));
+    float s, c;
+    sincospif(__fmul_rn(2.f, u2), &s, &c);
+    return make_float2(__fmul_rn(r, c), __fmul_rn(r, s));
+}
+
+// {seed, step} (device int64[2]) of a launch that draws with it.  advance: the launch takes the step once and leaves
+// step + 1 behind, by the last-block pattern -- each of the n_blocks blocks takes a ticket with one atomic on the step
+// word (bits 40..63 count the tickets, bits 0..39 hold the step, so step < 2^40 - 1), and the block that takes the last
+// ticket writes step + 1.  One call per block, after griddepcontrol.wait (the launch in front may be the one advancing it).
+constexpr int kStepTicketShift = 40;
+constexpr unsigned long long kStepMask = (1ull << kStepTicketShift) - 1ull;
+__device__ __forceinline__ RngKey take_step(unsigned long long* state, unsigned n_blocks, bool advance) {
+    const unsigned long long seed = *reinterpret_cast<volatile unsigned long long*>(state);
+    if (!advance) return make_rng_key(seed, *reinterpret_cast<volatile unsigned long long*>(state + 1) & kStepMask);
+    const unsigned long long old = atomicAdd(state + 1, 1ull << kStepTicketShift);
+    const unsigned long long step = old & kStepMask;
+    if ((old >> kStepTicketShift) == (unsigned long long)n_blocks - 1ull) atomicExch(state + 1, step + 1ull);
+    return make_rng_key(seed, step);
+}
+#endif
 
 }  // namespace rover

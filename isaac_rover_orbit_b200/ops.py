@@ -615,6 +615,33 @@ class ResetRng:
         return out
 
 
+class ActionRng:
+    """``{seed, step}`` of the policy's action noise (``rover_policy_act``): a CUDA int64[2] tensor that every sampling
+    launch reads and advances by one, apart from ``ResetRng`` so that seeding the environment never shifts the policy's
+    noise, nor the other way round.  Env ``i`` draws ``normal2(seed, step, env_offset + i)`` (``csrc/rng.cuh``), whatever
+    ``N`` is and whatever else uses torch's generator.  ``noise(n, env_offset)`` is the ``eps [n, 2]`` the NEXT launch will
+    draw, computed on the device by the same code, without advancing the state (tests feed it to ``gaussian_act``)."""
+
+    STEP_LIMIT = (1 << 40) - 1  # the launches count their blocks in bits 40..63 of the step word
+
+    def __init__(self, seed: int, device, step: int = 0):
+        self.device = torch.device(device)
+        if self.device.type != "cuda":
+            raise RuntimeError("ActionRng needs a CUDA device; there is no CPU fallback")
+        if not 0 <= int(step) < self.STEP_LIMIT:
+            raise ValueError(f"ActionRng: step must be in [0, 2^40 - 1), got {step}")
+        seed = int(seed) & 0xFFFFFFFFFFFFFFFF
+        self.state = torch.tensor([seed - (1 << 64) if seed >= 1 << 63 else seed, int(step)], dtype=torch.int64,
+                                  device=self.device)
+
+    def peek(self) -> tuple:
+        seed, step = (int(v) for v in self.state.cpu())
+        return seed & 0xFFFFFFFFFFFFFFFF, step
+
+    def noise(self, n: int, env_offset: int = 0) -> torch.Tensor:
+        return torch.ops.rover_b200.action_noise(self.state, int(env_offset), int(n), False)
+
+
 def mdp_pre_step(buf: MdpBuffers, params: _lib.MdpParams, actions: torch.Tensor | None,
                  force_matrix_w: torch.Tensor | None, phases: int = _lib.PRE_ALL):
     """Action shift + Ackermann (``PRE_ACTIONS``) and counters + terminations + rewards (``PRE_TERMS``);

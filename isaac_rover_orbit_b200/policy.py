@@ -149,10 +149,14 @@ class GaussianNeuralNetwork(_RoverNetwork):
         return self._forward_bf16(inputs["states"], False), self.log_std_parameter, {}
 
     def act(self, inputs: dict, role: str = "actor", eps: torch.Tensor | None = None,
-            out_actions: torch.Tensor | None = None):
+            out_actions: torch.Tensor | None = None, rng=None):
         """skrl 1.1.0 ``GaussianMixin.act`` (SURVEY.md A.4): returns ``(actions [N,2], log_prob [N,1], outputs)``.
         ``eps`` (standard-normal draws) may be supplied for reproducible parity checks; ``out_actions`` (fp32 ``[N,2]``,
-        e.g. the env's action input buffer) receives the actions in place of a new tensor (no copy on the way to the env)."""
+        e.g. the env's action input buffer) receives the actions in place of a new tensor (no copy on the way to the env).
+        ``rng`` (an ``ops.ActionRng``) and no ``eps``: the forward pass samples in its last epilogue -- ONE launch, noise
+        keyed on (seed, step, env) instead of ``torch.randn`` (``rover_policy_act``); fp32 or bf16 states."""
+        if rng is not None and eps is None:
+            return self._act_sampled(inputs["states"], out_actions, rng)
         mean, log_std, outputs = self.compute(inputs, role)
         n = mean.shape[0]
         if eps is None:
@@ -165,6 +169,48 @@ class GaussianNeuralNetwork(_RoverNetwork):
             actions, log_prob = torch.ops.rover_b200.gaussian_act(mean, log_std, eps.contiguous())
         outputs["mean_actions"] = mean
         return actions, log_prob.unsqueeze(-1), outputs
+
+    def _act_sampled(self, states: torch.Tensor, out_actions: torch.Tensor | None, rng):
+        if states.dtype != torch.bfloat16:
+            states = _aligned_states(states, "act")
+        if self._dirty:
+            self._pack()
+        n = states.shape[0]
+        mean = torch.empty(n, 2, dtype=torch.float32, device=states.device)
+        actions = out_actions if out_actions is not None else torch.empty_like(mean)
+        log_prob = torch.empty(n, 1, dtype=torch.float32, device=states.device)
+        torch.ops.rover_b200.policy_act(states, self._packed, self.log_std_parameter, rng.state, 0, mean, actions, log_prob)
+        return actions, log_prob, {"mean_actions": mean}
+
+
+def _aligned_states(states: torch.Tensor, what: str) -> torch.Tensor:
+    """fp32 ``[N,965]`` CUDA states with 16-byte aligned rows: the tensor itself, or one copy into ``alloc_obs``."""
+    if not states.is_cuda or states.dtype != torch.float32 or states.dim() != 2 or states.shape[1] != OBS_COLS:
+        raise RuntimeError(f"{what}: states must be a CUDA fp32 [N,965] tensor")
+    if states.stride(1) != 1 or states.stride(0) % 4 != 0 or states.data_ptr() % 16 != 0:
+        buf = alloc_obs(states.shape[0], states.device)
+        buf.copy_(states)
+        states = buf
+    return states
+
+
+def policy_value_act(policy: "GaussianNeuralNetwork", value: "DeterministicNeuralNetwork", states: torch.Tensor, rng,
+                     out_actions: torch.Tensor | None = None):
+    """``policy.act`` (sampled with ``rng``, an ``ops.ActionRng``) and the value network on fp32 ``states [N,965]`` in ONE
+    launch (``rover_policy_value_act``): ``(actions [N,2], log_prob [N,1], value [N,1], mean [N,2])``, each bit-identical
+    to ``policy_value_forward`` followed by ``gaussian_act`` with ``rng.noise(N)``."""
+    states = _aligned_states(states, "policy_value_act")
+    for net in (policy, value):
+        if net._dirty:
+            net._pack()
+    n = states.shape[0]
+    mean = torch.empty(n, 2, dtype=torch.float32, device=states.device)
+    val = torch.empty(n, 1, dtype=torch.float32, device=states.device)
+    actions = out_actions if out_actions is not None else torch.empty_like(mean)
+    log_prob = torch.empty(n, 1, dtype=torch.float32, device=states.device)
+    torch.ops.rover_b200.policy_value_act(states, policy._packed, value._packed, policy.log_std_parameter, rng.state, 0, mean,
+                                          val, actions, log_prob)
+    return actions, log_prob, val, mean
 
 
 def policy_value_forward(policy: "GaussianNeuralNetwork", value: "DeterministicNeuralNetwork", states: torch.Tensor):

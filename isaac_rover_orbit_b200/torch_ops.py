@@ -83,6 +83,12 @@ _SCHEMAS = {
     "policy_value_forward": "(Tensor obs, Tensor packed_policy, Tensor packed_value) -> (Tensor, Tensor)",
     "gaussian_act": "(Tensor mean, Tensor log_std, Tensor eps) -> (Tensor, Tensor)",
     "gaussian_act_out": "(Tensor mean, Tensor log_std, Tensor eps, Tensor(a!) actions, Tensor(b!) log_prob) -> ()",
+    # ---- the forward pass with GaussianMixin.act in its last epilogue: noise keyed on (seed, step, env_offset + env)
+    "policy_act": "(Tensor obs, Tensor packed, Tensor log_std, Tensor(a!) rng_state, int env_offset, Tensor(b!) mean, "
+                  "Tensor(c!) actions, Tensor(d!) log_prob) -> ()",
+    "policy_value_act": "(Tensor obs, Tensor packed_policy, Tensor packed_value, Tensor log_std, Tensor(a!) rng_state, "
+                        "int env_offset, Tensor(b!) mean, Tensor(c!) value, Tensor(d!) actions, Tensor(e!) log_prob) -> ()",
+    "action_noise": "(Tensor(a!) rng_state, int env_offset, int n_envs, bool advance) -> Tensor",
     # ---- PPO returns and advantages over the rollout memory (skrl PPO._update -> compute_gae)
     "ppo_gae": "(Tensor rewards, Tensor dones, Tensor values, Tensor last_values, float discount_factor, "
                "float lambda_coefficient, Tensor(a!) returns, Tensor(b!) advantages) -> ()",
@@ -533,6 +539,58 @@ def _gaussian_act(mean, log_std, eps):
     return actions, log_prob
 
 
+def _act_checks(what, obs, log_std, rng_state, env_offset, mean, actions, log_prob, value=None):
+    """The checks of the sampling operators: what the forward operators check on ``obs``, plus the sampling tensors."""
+    n = obs.shape[0] if obs.dim() == 2 else -1
+    if obs.dtype == torch.bfloat16 and what == "policy_act":
+        if obs.dim() != 2 or obs.shape[1] != 965 or obs.stride(1) != 1 or obs.stride(0) % 8 != 0 or obs.data_ptr() % 16 != 0:
+            raise RuntimeError(f"rover_b200::{what}: bf16 states must be a [N,965] view from alloc_obs_bf16()")
+    elif (obs.dtype != torch.float32 or obs.dim() != 2 or obs.shape[1] != 965 or obs.stride(1) != 1
+            or obs.stride(0) % 4 != 0 or obs.data_ptr() % 16 != 0):
+        raise RuntimeError(f"rover_b200::{what}: states must be fp32 [N,965] with 16-byte aligned rows")
+    ts = [obs, log_std, rng_state, mean, actions, log_prob] + ([value] if value is not None else [])
+    if not all(t.is_cuda and t.device == obs.device for t in ts):
+        raise RuntimeError(f"rover_b200::{what}: every tensor must be a CUDA tensor on the states' device")
+    if rng_state.dtype != torch.int64 or rng_state.numel() != 2 or not rng_state.is_contiguous():
+        raise RuntimeError(f"rover_b200::{what}: rng_state must be a CUDA int64 tensor {{seed, step}}")
+    _f32(what, log_std, mean, actions, log_prob, value)
+    if log_std.numel() != 2:
+        raise RuntimeError(f"rover_b200::{what}: log_std must hold 2 values")
+    if mean.shape != (n, 2) or actions.shape != (n, 2) or log_prob.numel() != n or (value is not None and value.numel() != n):
+        raise RuntimeError(f"rover_b200::{what}: mean / actions [N,2], log_prob [N]" + (", value [N]" if value is not None else "")
+                           + " expected")
+    if mean.data_ptr() % 8 or actions.data_ptr() % 8:
+        raise RuntimeError(f"rover_b200::{what}: mean and actions must be 8-byte aligned")
+    if not 0 <= int(env_offset) < 2 ** 31:  # (then env_offset + N < 2^32 for any int32 N)
+        raise RuntimeError(f"rover_b200::{what}: env_offset must be a non-negative int32 with env_offset + N <= 2^32")
+    return n
+
+
+def _policy_act(obs, packed, log_std, rng_state, env_offset, mean, actions, log_prob):
+    n = _act_checks("policy_act", obs, log_std, rng_state, env_offset, mean, actions, log_prob)
+    entry = _lib.load().rover_policy_act_bf16 if obs.dtype == torch.bfloat16 else _lib.load().rover_policy_act
+    _lib.check(entry(_p(obs), int(obs.stride(0)), n, _p(packed), _p(log_std), _p(rng_state), int(env_offset), _p(mean),
+                     _p(actions), _p(log_prob), _stream(obs)))
+
+
+def _policy_value_act(obs, packed_policy, packed_value, log_std, rng_state, env_offset, mean, value, actions, log_prob):
+    n = _act_checks("policy_value_act", obs, log_std, rng_state, env_offset, mean, actions, log_prob, value)
+    _lib.check(_lib.load().rover_policy_value_act(_p(obs), int(obs.stride(0)), n, _p(packed_policy), _p(packed_value),
+                                                  _p(log_std), _p(rng_state), int(env_offset), _p(mean), _p(value),
+                                                  _p(actions), _p(log_prob), _stream(obs)))
+
+
+def _action_noise(rng_state, env_offset, n_envs, advance):
+    if not rng_state.is_cuda or rng_state.dtype != torch.int64 or rng_state.numel() != 2 or not rng_state.is_contiguous():
+        raise RuntimeError("rover_b200::action_noise: rng_state must be a CUDA int64 tensor {seed, step}")
+    if not (0 <= int(env_offset) < 2 ** 31 and 0 <= int(n_envs) < 2 ** 31):
+        raise RuntimeError("rover_b200::action_noise: env_offset and n_envs must be non-negative int32")
+    eps = torch.empty(int(n_envs), 2, dtype=torch.float32, device=rng_state.device)
+    _lib.check(_lib.load().rover_action_noise(_p(rng_state), int(env_offset), int(n_envs), _p(eps), int(bool(advance)),
+                                              _stream(rng_state)))
+    return eps
+
+
 # ----------------------------------------------------------------------------------------------------- PPO
 def _overlaps(a: torch.Tensor, b: torch.Tensor) -> bool:
     if a.numel() == 0 or b.numel() == 0 or a.device != b.device:
@@ -621,6 +679,7 @@ _IMPLS = {
     "gaussian_act_out": _gaussian_act_out, "policy_pack_fused": _policy_pack_fused,
     "scan_encoder_fused": _scan_encoder_fused, "policy_mlp_forward": _policy_mlp_forward, "mesh_to_heightmap": _mesh_to_heightmap,
     "steep_mask": _steep_mask, "morph_box": _morph_box, "fill_holes": _fill_holes, "ppo_gae": _ppo_gae,
+    "policy_act": _policy_act, "policy_value_act": _policy_value_act, "action_noise": _action_noise,
 }
 for _name, _fn in _IMPLS.items():
     _IMPL.impl(_name, _fn)
@@ -684,6 +743,11 @@ def _(mean, log_std, eps):
     return torch.empty_like(mean), mean.new_empty(mean.shape[0])
 
 
+@_fake("action_noise")
+def _(rng_state, env_offset, n_envs, advance):
+    return rng_state.new_empty(int(n_envs), 2, dtype=torch.float32)
+
+
 @_fake("steep_mask")
 def _(heightmap, threshold):
     return heightmap.new_empty(heightmap.shape, dtype=torch.uint8)
@@ -705,7 +769,7 @@ def _fake_none(*args, **kwargs):
 
 for _name in ("height_scan_out", "ray_cast_out", "height_scan_obs", "height_scan_host", "ray_cast_obs", "ray_cast_host",
               "gaussian_act_out", "mdp_pre_step", "mdp_post_step", "mdp_step", "step_fused", "stats_read", "policy_pack",
-              "policy_pack_fused", "mesh_to_heightmap", "ppo_gae"):
+              "policy_pack_fused", "mesh_to_heightmap", "ppo_gae", "policy_act", "policy_value_act"):
     torch.library.register_fake(f"{NS}::{_name}", _fake_none, lib=_DEF)
 
 OPS = tuple(_SCHEMAS)

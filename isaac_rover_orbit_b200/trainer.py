@@ -138,13 +138,17 @@ class RolloutAgent(BaseAgent):
     hooks the trainer calls around them exist and do what skrl's base ``Agent`` does (tracking), nothing more."""
 
     def __init__(self, policy, memory: RolloutMemory | None = None, observation_size: int = 965, action_size: int = 2,
-                 value=None, action_out: torch.Tensor | None = None):
+                 value=None, action_out: torch.Tensor | None = None, action_rng=None):
         """``value``: the PPO value network (``DeterministicNeuralNetwork``).  skrl's PPO evaluates it in
         ``record_transition`` on the states ``act`` just saw; here both networks run in ONE pass over the observation
-        (``policy.policy_value_forward``) and the values are written to the memory's ``values`` tensor."""
+        (``policy.policy_value_forward``) and the values are written to the memory's ``values`` tensor.
+        ``action_rng`` (an ``ops.ActionRng``): the policy samples inside its forward pass with noise keyed on
+        (seed, step, env) instead of ``torch.randn`` -- one launch per ``act``, policy and value together on fp32 states
+        (``policy.policy_value_act``); without it ``act`` draws ``torch.randn`` as before."""
         super().__init__()
         self.policy = policy
         self.value = value
+        self.action_rng = action_rng
         self.action_out = action_out  # e.g. ``env.action_input``: the sampled actions land where the env's step reads them
         self.memory = memory
         self._log_prob = None
@@ -159,8 +163,17 @@ class RolloutAgent(BaseAgent):
             memory.create_tensor("log_prob", 1)
 
     def act(self, states: torch.Tensor, timestep: int, timesteps: int):
+        if self.action_rng is not None and self.value is not None and states.dtype == torch.float32:
+            from .policy import policy_value_act
+
+            actions, log_prob, self._values, mean = policy_value_act(self.policy, self.value, states, self.action_rng,
+                                                                     out_actions=self.action_out)
+            self._log_prob = log_prob
+            return actions, log_prob, {"mean_actions": mean}
         if self.value is None or states.dtype != torch.float32:
             extra = {"out_actions": self.action_out} if self.action_out is not None else {}  # (any skrl-style policy works)
+            if self.action_rng is not None:
+                extra["rng"] = self.action_rng
             actions, log_prob, outputs = self.policy.act({"states": states}, role="policy", **extra)
             if self.value is not None:
                 self._values = self.value.act({"states": states}, role="value")[0]
@@ -208,10 +221,10 @@ class PPORolloutAgent(RolloutAgent):
     as in skrl 1.1.0: a truncated step bootstraps from the next row's value.  The optimisation epochs are not provided."""
 
     def __init__(self, policy, value, memory: RolloutMemory, discount_factor: float = 0.99, lambda_: float = 0.95,
-                 action_out: torch.Tensor | None = None):
+                 action_out: torch.Tensor | None = None, action_rng=None):
         if value is None or memory is None:
             raise ValueError("PPORolloutAgent needs a value network and a memory")
-        super().__init__(policy, memory, value=value, action_out=action_out)
+        super().__init__(policy, memory, value=value, action_out=action_out, action_rng=action_rng)
         self.discount_factor = float(discount_factor)
         self.lambda_ = float(lambda_)
         self._rollout = 0
