@@ -529,6 +529,14 @@ int rover_policy_value_act(const float* obs, int32_t obs_stride, int32_t n_envs,
  * launch (GaussianMixin.act with explicit noise). */
 int rover_action_noise(int64_t* rng_state, int32_t env_offset, int32_t n_envs, float* eps_out, int32_t advance,
                        void* stream);
+/* The sampling's functions that are not correctly rounded, evaluated elementwise by the same device code the policy
+ * kernels run (test support: an fp32 model of the sampling takes them from here, tests/act_exact.py).  DEVICE f32 arrays
+ * of n: ROVER_POLICY_MATH_LOG: out0 = logf(a); ROVER_POLICY_MATH_EXP: out0 = expf(a) (out1 unused, may be NULL);
+ * ROVER_POLICY_MATH_SINCOSPI: sincospif(a, out0, out1), out0 = sin(pi a), out1 = cos(pi a).  Asynchronous on `stream`. */
+#define ROVER_POLICY_MATH_LOG 0
+#define ROVER_POLICY_MATH_EXP 1
+#define ROVER_POLICY_MATH_SINCOSPI 2
+int rover_policy_math(int32_t op, const float* a, float* out0, float* out1, int32_t n, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------
  * PPO returns and advantages.  Replaces skrl 1.1.0 PPO._update's compute_gae (agents/torch/ppo/ppo.py; third-party,

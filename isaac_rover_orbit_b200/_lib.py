@@ -31,7 +31,7 @@ SYMBOLS = ("rover_abi_version", "rover_last_error", "rover_height_scan", "rover_
            "rover_policy_pack_fused", "rover_scan_encoder_fused", "rover_policy_mlp_forward", "rover_morph_box",
            "rover_fill_holes", "rover_step_fused", "rover_ray_cast", "rover_ray_cast_obs", "rover_ray_cast_obs_bf16",
            "rover_ray_cast_host", "rover_ppo_gae", "rover_ppo_gae_work_bytes", "rover_mdp_math", "rover_policy_act",
-           "rover_policy_act_bf16", "rover_policy_value_act", "rover_action_noise")
+           "rover_policy_act_bf16", "rover_policy_value_act", "rover_action_noise", "rover_policy_math")
 
 
 class ScanLevel(C.Structure):
@@ -236,6 +236,8 @@ def load() -> C.CDLL:
     lib.rover_policy_value_act.argtypes = [vp, i32, i32, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp]
     lib.rover_action_noise.restype = C.c_int
     lib.rover_action_noise.argtypes = [vp, i32, i32, vp, i32, vp]
+    lib.rover_policy_math.restype = C.c_int
+    lib.rover_policy_math.argtypes = [i32, vp, vp, vp, i32, vp]
     _lib = lib
     return lib
 
@@ -298,3 +300,18 @@ def mdp_math(op: int, a: torch.Tensor, b: torch.Tensor | None = None) -> torch.T
     out = torch.empty_like(a)
     check(load().rover_mdp_math(int(op), ptr(a), ptr(b), ptr(out), a.numel(), current_stream(dev)))
     return out
+
+
+POLICY_MATH_LOG, POLICY_MATH_EXP, POLICY_MATH_SINCOSPI = 0, 1, 2
+
+
+def policy_math(op: int, a: torch.Tensor):
+    """``logf(a)`` or ``expf(a)`` (one tensor), or ``sincospif(a)`` (``(sin(pi a), cos(pi a))``) elementwise, by the
+    device code of the policy kernels (``rover_policy_math``; test support).  ``a``: a contiguous fp32 CUDA tensor."""
+    dev = require_cuda(a)
+    if a.dtype != torch.float32:
+        raise RuntimeError("policy_math: an fp32 tensor expected")
+    out0 = torch.empty_like(a)
+    out1 = torch.empty_like(a) if op == POLICY_MATH_SINCOSPI else None
+    check(load().rover_policy_math(int(op), ptr(a), ptr(out0), ptr(out1), a.numel(), current_stream(dev)))
+    return out0 if out1 is None else (out0, out1)

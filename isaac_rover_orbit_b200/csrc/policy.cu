@@ -341,6 +341,25 @@ __global__ void action_noise_kernel(unsigned long long* __restrict__ rng, uint32
         *reinterpret_cast<float2*>(eps + 2 * (size_t)i) = normal2(key, env_offset + (uint32_t)i);
 }
 
+// The sampling's functions that are not correctly rounded (logf, expf, sincospif), evaluated elementwise by the device
+// code the policy kernels run (this library's flags and libdevice): an fp32 model of the sampling takes them from here.
+__global__ void policy_math_kernel(int op, const float* __restrict__ a, float* __restrict__ out0, float* __restrict__ out1,
+                                   int n) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float x = a[i];
+    if (op == ROVER_POLICY_MATH_LOG) {
+        out0[i] = logf(x);
+    } else if (op == ROVER_POLICY_MATH_EXP) {
+        out0[i] = expf(x);
+    } else {
+        float s, c;
+        sincospif(x, &s, &c);
+        out0[i] = s;
+        out1[i] = c;
+    }
+}
+
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -563,4 +582,15 @@ extern "C" int rover_action_noise(int64_t* rng_state, int32_t env_offset, int32_
                                  reinterpret_cast<unsigned long long*>(rng_state), (uint32_t)env_offset, (int)n_envs, eps_out,
                                  (int)(advance != 0)));
     return check_launch("action_noise_kernel");
+}
+
+extern "C" int rover_policy_math(int32_t op, const float* a, float* out0, float* out1, int32_t n, void* stream) {
+    using namespace rover;
+    ROVER_CHECK(op == ROVER_POLICY_MATH_LOG || op == ROVER_POLICY_MATH_EXP || op == ROVER_POLICY_MATH_SINCOSPI,
+                "rover_policy_math: op must be ROVER_POLICY_MATH_LOG, _EXP or _SINCOSPI");
+    ROVER_CHECK(n >= 0, "rover_policy_math: negative n");
+    if (n == 0) return 0;
+    ROVER_CHECK(a && out0 && (out1 || op != ROVER_POLICY_MATH_SINCOSPI), "rover_policy_math: NULL argument");
+    policy_math_kernel<<<(n + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream)>>>(op, a, out0, out1, n);
+    return check_launch("policy_math_kernel");
 }

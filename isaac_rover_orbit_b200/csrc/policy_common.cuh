@@ -124,19 +124,29 @@ __device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
 }
 __device__ __forceinline__ float leaky(float x) { return x > 0.f ? x : 0.01f * x; }
 
+// clamp(x, lo, hi) that keeps a NaN NaN, as torch.clamp does: PTX max.NaN / min.NaN (one FMNMX each, like fmaxf /
+// fminf, which return the other operand and would turn a NaN into a bound)
+__device__ __forceinline__ float clamp_keep_nan(float x, float lo, float hi) {
+    float y;
+    asm("max.NaN.f32 %0, %1, %2;" : "=f"(y) : "f"(x), "f"(lo));
+    asm("min.NaN.f32 %0, %0, %1;" : "+f"(y) : "f"(hi));
+    return y;
+}
+
 // skrl 1.1.0 GaussianMixin.act for one environment (models.py:65-67: clip_log_std, min -20, max 2): log_std clamped to
 // [-20, 2], the reparameterised sample mean + std * eps clipped to the action box [-1, 1], log-prob of the clipped action
-// under Normal(mean, std) summed over the two action dimensions.  Shared by gaussian_act_kernel and the sampling
-// epilogue of the forward pass, so both give the same bits.
+// under Normal(mean, std) summed over the two action dimensions.  Both clamps keep NaN (torch.clamp): a NaN mean -- a
+// missed ray's -inf height through the network -- gives a NaN action and log-prob, not the action -1.  Shared by
+// gaussian_act_kernel and the sampling epilogue of the forward pass, so both give the same bits.
 __device__ __forceinline__ float gaussian_sample(const float (&mean)[2], const float (&log_std)[2], const float (&eps)[2],
                                                  float (&actions)[2]) {
     float lp = 0.f;
 #pragma unroll
     for (int j = 0; j < 2; ++j) {
-        const float ls = fminf(fmaxf(log_std[j], -20.f), 2.f);
+        const float ls = clamp_keep_nan(log_std[j], -20.f, 2.f);
         const float sd = expf(ls);
         const float m = mean[j];
-        const float a = fminf(fmaxf(fmaf(sd, eps[j], m), -1.f), 1.f);
+        const float a = clamp_keep_nan(fmaf(sd, eps[j], m), -1.f, 1.f);
         actions[j] = a;
         const float d = a - m;
         lp += -(d * d) / (2.f * sd * sd) - ls - 0.91893853320467274178f;
