@@ -474,6 +474,13 @@ int rover_policy_forward_bf16(const uint16_t* obs_bf16, int32_t stride, int32_t 
                               void* stream);
 int rover_value_forward_bf16(const uint16_t* obs_bf16, int32_t stride, int32_t n_envs, const void* packed, float* value,
                              void* stream);
+/* Policy AND value network in ONE pass over the bf16 observation (models.py:89-102 + :151-162, as
+ * rover_policy_value_forward): each 64-column tile of obs_bf16 (layout of rover_policy_forward_bf16) meets both
+ * heightmap encoders.  mean [N,2] and value [N] are bit-identical to rover_policy_forward_bf16 /
+ * rover_value_forward_bf16 on the same blobs, and to rover_policy_value_forward on an fp32 observation that rounds to
+ * the same bf16 values. */
+int rover_policy_value_forward_bf16(const uint16_t* obs_bf16, int32_t stride, int32_t n_envs, const void* packed_policy,
+                                    const void* packed_value, float* mean, float* value, void* stream);
 /* Height scan FUSED with the heightmap encoder of the policy (or value) network -- BASELINE.json configs[3], "policy
  * forward fused with the observation kernel".  rover_scan_encoder_fused replaces height_scan_rover
  * (mdp/observations.py:35-45, over ORBIT RayCaster / warp raycast) and HeightmapEncoder (learning/skrl/models.py:24-36,
@@ -523,6 +530,13 @@ int rover_policy_act_bf16(const uint16_t* obs_bf16, int32_t stride, int32_t n_en
 int rover_policy_value_act(const float* obs, int32_t obs_stride, int32_t n_envs, const void* packed_policy,
                            const void* packed_value, const float* log_std, int64_t* rng_state, int32_t env_offset,
                            float* mean, float* value, float* actions, float* log_prob, void* stream);
+/* rover_policy_value_act on the bf16 observation of rover_policy_value_forward_bf16 (skrl GaussianMixin.act,
+ * models.py:39-102, + DeterministicNeuralNetwork.compute, :151-162): one launch, the same noise stream and step
+ * advance; mean, value, actions and log_prob equal rover_policy_value_forward_bf16 + rover_gaussian_act fed the eps of
+ * rover_action_noise bit for bit. */
+int rover_policy_value_act_bf16(const uint16_t* obs_bf16, int32_t stride, int32_t n_envs, const void* packed_policy,
+                                const void* packed_value, const float* log_std, int64_t* rng_state, int32_t env_offset,
+                                float* mean, float* value, float* actions, float* log_prob, void* stream);
 /* The eps [N,2] (8-byte aligned) that the next rover_policy_*act launch with rng_state and env_offset draws, computed on
  * the device with the same code (host libm's log / sin / cos round differently).  advance != 0: the step advances by one
  * as an act launch would; advance == 0 leaves rng_state unchanged.  Feed it to rover_gaussian_act to reproduce an act

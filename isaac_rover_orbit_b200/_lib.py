@@ -31,7 +31,8 @@ SYMBOLS = ("rover_abi_version", "rover_last_error", "rover_height_scan", "rover_
            "rover_policy_pack_fused", "rover_scan_encoder_fused", "rover_policy_mlp_forward", "rover_morph_box",
            "rover_fill_holes", "rover_step_fused", "rover_ray_cast", "rover_ray_cast_obs", "rover_ray_cast_obs_bf16",
            "rover_ray_cast_host", "rover_ppo_gae", "rover_ppo_gae_work_bytes", "rover_mdp_math", "rover_policy_act",
-           "rover_policy_act_bf16", "rover_policy_value_act", "rover_action_noise", "rover_policy_math")
+           "rover_policy_act_bf16", "rover_policy_value_act", "rover_action_noise", "rover_policy_math",
+           "rover_policy_value_forward_bf16", "rover_policy_value_act_bf16")
 
 
 class ScanLevel(C.Structure):
@@ -209,8 +210,9 @@ def load() -> C.CDLL:
     lib.rover_policy_forward.argtypes = [vp, i32, i32, vp, vp, vp]
     lib.rover_value_forward.restype = C.c_int
     lib.rover_value_forward.argtypes = [vp, i32, i32, vp, vp, vp]
-    lib.rover_policy_value_forward.restype = C.c_int
-    lib.rover_policy_value_forward.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp]
+    for fn in (lib.rover_policy_value_forward, lib.rover_policy_value_forward_bf16):
+        fn.restype = C.c_int
+        fn.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp]
     for fn in (lib.rover_policy_forward_bf16, lib.rover_value_forward_bf16):
         fn.restype = C.c_int
         fn.argtypes = [vp, i32, i32, vp, vp, vp]
@@ -232,8 +234,9 @@ def load() -> C.CDLL:
     for fn in (lib.rover_policy_act, lib.rover_policy_act_bf16):
         fn.restype = C.c_int
         fn.argtypes = [vp, i32, i32, vp, vp, vp, i32, vp, vp, vp, vp]
-    lib.rover_policy_value_act.restype = C.c_int
-    lib.rover_policy_value_act.argtypes = [vp, i32, i32, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp]
+    for fn in (lib.rover_policy_value_act, lib.rover_policy_value_act_bf16):
+        fn.restype = C.c_int
+        fn.argtypes = [vp, i32, i32, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp]
     lib.rover_action_noise.restype = C.c_int
     lib.rover_action_noise.argtypes = [vp, i32, i32, vp, i32, vp]
     lib.rover_policy_math.restype = C.c_int

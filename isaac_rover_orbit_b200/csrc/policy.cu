@@ -484,6 +484,22 @@ extern "C" int rover_value_forward_bf16(const uint16_t* obs_bf16, int32_t stride
     return forward_bf16(obs_bf16, stride, n_envs, packed, value, stream, true);
 }
 
+extern "C" int rover_policy_value_forward_bf16(const uint16_t* obs_bf16, int32_t stride, int32_t n_envs,
+                                               const void* packed_policy, const void* packed_value, float* mean, float* value,
+                                               void* stream) {
+    using namespace rover;
+    ROVER_CHECK(n_envs >= 0, "rover_policy_value_forward_bf16: negative n_envs");
+    if (n_envs == 0) return 0;
+    ROVER_CHECK(obs_bf16 && packed_policy && packed_value && mean && value, "rover_policy_value_forward_bf16: NULL argument");
+    ROVER_CHECK(stride >= kObsCols && stride % 8 == 0 && (reinterpret_cast<uintptr_t>(obs_bf16) & 15) == 0,
+                "rover_policy_value_forward_bf16: bf16 observation rows must be 16-byte aligned (stride %% 8 == 0, got %d)",
+                stride);
+    ROVER_CHECK((reinterpret_cast<uintptr_t>(packed_policy) & 127) == 0 && (reinterpret_cast<uintptr_t>(packed_value) & 127) == 0,
+                "rover_policy_value_forward_bf16: packed blob not 128B aligned");
+    return launch_policy_forward_ws(obs_bf16, stride, n_envs, packed_policy, mean, false, true, static_cast<cudaStream_t>(stream),
+                                    packed_value, value);
+}
+
 extern "C" int rover_value_forward(const float* obs, int32_t obs_stride, int32_t n_envs, const void* packed,
                                    float* value, void* stream) {
     return policy_or_value_forward(obs, obs_stride, n_envs, packed, value, stream, true);
@@ -561,6 +577,25 @@ extern "C" int rover_policy_value_act(const float* obs, int32_t obs_stride, int3
     ROVER_CHECK((reinterpret_cast<uintptr_t>(packed_value) & 127) == 0, "rover_policy_value_act: packed blob not 128B aligned");
     const SampleArgs s{log_std, reinterpret_cast<unsigned long long*>(rng_state), (uint32_t)env_offset, actions, log_prob};
     return launch_policy_forward_ws(obs, obs_stride, n_envs, packed_policy, mean, false, false, static_cast<cudaStream_t>(stream),
+                                    packed_value, value, &s);
+}
+
+extern "C" int rover_policy_value_act_bf16(const uint16_t* obs_bf16, int32_t stride, int32_t n_envs, const void* packed_policy,
+                                           const void* packed_value, const float* log_std, int64_t* rng_state,
+                                           int32_t env_offset, float* mean, float* value, float* actions, float* log_prob,
+                                           void* stream) {
+    using namespace rover;
+    ROVER_CHECK(n_envs >= 0, "rover_policy_value_act_bf16: negative n_envs");
+    if (n_envs == 0) return 0;
+    ROVER_CHECK(obs_bf16 && packed_value && value, "rover_policy_value_act_bf16: NULL argument");
+    if (int rc = check_act_args("rover_policy_value_act_bf16", n_envs, packed_policy, log_std, rng_state, env_offset, mean,
+                                actions))
+        return rc;
+    ROVER_CHECK(stride >= kObsCols && stride % 8 == 0 && (reinterpret_cast<uintptr_t>(obs_bf16) & 15) == 0,
+                "rover_policy_value_act_bf16: bf16 observation rows must be 16-byte aligned (stride %% 8 == 0, got %d)", stride);
+    ROVER_CHECK((reinterpret_cast<uintptr_t>(packed_value) & 127) == 0, "rover_policy_value_act_bf16: packed blob not 128B aligned");
+    const SampleArgs s{log_std, reinterpret_cast<unsigned long long*>(rng_state), (uint32_t)env_offset, actions, log_prob};
+    return launch_policy_forward_ws(obs_bf16, stride, n_envs, packed_policy, mean, false, true, static_cast<cudaStream_t>(stream),
                                     packed_value, value, &s);
 }
 

@@ -23,6 +23,11 @@
 // the layer group then runs layers 1-5 once per network.  TMEM: 2 x 160 D0 columns + a 192-column accumulator, so layer 2
 // (N = 256) runs as two N halves and its input operand sits in planes 24-31, which the first half's output (planes
 // 0-15) does not touch.  Same arithmetic per network, so both outputs equal the two single passes bit for bit.
+//
+// kDual && kBf16In: the same two-network pass over the bf16 observation.  Each 64-column TMA stage meets both W0 images
+// (the policy's four K = 16 MMAs into D0[buf] columns 0-79, then the value network's four into columns 80-159); 352
+// threads, no converter warps; the TMEM plan is the fp32 dual plan.  Shared memory: the 4-stage observation ring of the
+// dual layout, and a W0 ring of TWO 20 KB stages (both networks' 10 KB chunks) overlaid on a_bf16[] + w0[] (46 KB).
 #include "policy_common.cuh"
 
 #ifndef ROVER_POLICY_DBG
@@ -68,6 +73,7 @@ static_assert(kW0ChunkBytes == 2 * kWsW0Chunk, "a 32-column chunk is half of a p
 constexpr int kBfChunkK = 64;
 constexpr int kBfChunks = 16;                 // columns [0, 1024); beyond column 963 the tensor map zero-fills
 constexpr int kBfStagesW = 3;                 // 10 KB W0 chunks in the space of a_bf16[] + w0[]
+constexpr int kBfStagesWDual = 2;             // 2 x 10 KB (policy + value) W0 chunks in the same space of the dual layout
 
 template <bool kDual>
 struct WsSmemT {
@@ -94,6 +100,11 @@ static_assert(offsetof(WsSmem, w0) == offsetof(WsSmem, a_bf16) + kWsStagesA * 4 
                   kBfStagesW * kW0ChunkBytes <= kWsStagesA * 4 * kWsPlane + kWsStagesW * kWsW0Chunk,
               "bf16-observation mode: W0 ring overlays a_bf16[] + w0[]");
 static_assert(kTileM * kBfChunkK * 2 == kTileM * kWsChunkK * 4, "both modes use the same 16 KB stages");
+static_assert(offsetof(WsSmemT<true>, w0) == offsetof(WsSmemT<true>, a_bf16) + kWsStagesA * 4 * kWsPlane &&
+                  kBfStagesWDual * 2 * kW0ChunkBytes <= kWsStagesA * 4 * kWsPlane + kWsStagesW * 2 * kWsW0Chunk &&
+                  (kBfStagesWDual + 1) * 2 * kW0ChunkBytes > kWsStagesA * 4 * kWsPlane + kWsStagesW * 2 * kWsW0Chunk,
+              "bf16 two-network mode: two (not three) W0 stages of both networks overlay a_bf16[] + w0[]");
+static_assert(kBfStagesWDual <= kWsStagesW, "w0_full[] / w0_empty[] cover the ring");
 
 // kDual: `packed` = policy, `packed2` = value network, outputs `mean` [N, 2] and `value2` [N]; else one network
 // (value_head: linear [N] output instead of tanh [N, 2]).
@@ -107,7 +118,6 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
                          int n_envs, int tile_rows, const unsigned char* __restrict__ packed, float* __restrict__ mean,
                          int value_head, const unsigned char* __restrict__ packed2, float* __restrict__ value2,
                          const __grid_constant__ SampleArgs sample) {
-    static_assert(!(kDual && kBf16In), "the two-network pass reads fp32 observations");
     using Smem = WsSmemT<kDual>;
     constexpr int kNets = Smem::kNets, kStagesFK = Smem::kStagesFT;
     constexpr uint32_t kColD0Stride = kDual ? kWsColD0StrideDual : kWsColD0Stride, kColAcc = kDual ? kWsColAccDual : kWsColAcc;
@@ -122,7 +132,7 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
     const int n_tiles = (n_envs + tile_rows - 1) / tile_rows;
     constexpr int kChunks = kBf16In ? kBfChunks : kWsChunks;
     constexpr int kChunkK = kBf16In ? kBfChunkK : kWsChunkK;        // observation columns per chunk
-    constexpr int kStagesW = kBf16In ? kBfStagesW : kWsStagesW;
+    constexpr int kStagesW = kBf16In ? (kDual ? kBfStagesWDual : kBfStagesW) : kWsStagesW;
     constexpr int kW0Chunk = kBf16In ? kW0ChunkBytes : kWsW0Chunk;  // bytes of ONE packed W0 image per chunk
     constexpr int kW0Stage = kNets * kW0Chunk;                      // bytes of a W0 ring stage
     const uint32_t chunk_bytes = (uint32_t)tile_rows * 128u;        // 32 fp32 or 64 bf16 columns per row
@@ -239,7 +249,16 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
                     mb_wait(&sm.w0_full[sw], pw & 1u);
                     tc_fence_after();
                     const uint32_t b0 = sptr(w0_ring + sw * kW0Stage);
-                    if (kBf16In) {
+                    if (kBf16In && kDual) {
+                        const uint32_t a0 = sptr(sm.stage_f[sa]);
+#pragma unroll
+                        for (int net = 0; net < 2; ++net)
+#pragma unroll
+                            for (int j = 0; j < kBfChunkK / 16; ++j)
+                                umma(d0 + net * 80, make_desc_sw128(a0 + j * 32),
+                                     make_desc(b0 + net * kW0Chunk + j * 2 * 80 * 16, 80 * 16), idesc0, (c | j) != 0);
+                        umma_commit(&sm.f_empty[sa]);
+                    } else if (kBf16In) {
                         const uint32_t a0 = sptr(sm.stage_f[sa]);
 #pragma unroll
                         for (int j = 0; j < kBfChunkK / 16; ++j)  // 16 bf16 = 32 B further along K inside the 128 B rows
@@ -266,8 +285,10 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
         }
     } else if (warp >= 4 && kBf16In) {
         // bf16-observation mode: no conversion stage; these warps only pull the packed weights into L2
-        for (int off = (tid - 128) * 128; off < kPackedBytes; off += 128 * 128)
+        for (int off = (tid - 128) * 128; off < kPackedBytes; off += 128 * 128) {
             asm volatile("prefetch.global.L2 [%0];" ::"l"(packed + off));
+            if (kDual) asm volatile("prefetch.global.L2 [%0];" ::"l"(packed2 + off));
+        }
     } else if (warp >= 4) {
         // =============================================================== converters: fp32 stage -> bf16 A operand
         // first the packed weights into L2 (326 KB; after an L2 flush every layer's first load was a cold miss that the
@@ -542,8 +563,8 @@ typedef CUresult (*WsEncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_
                                     CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
 // obs: fp32 [N, obs_stride] (bf16_in == false) or bf16 [N, obs_stride] (bf16_in == true; strides in elements).
-// packed2 != nullptr (fp32 observations only): policy (`packed` -> mean [N, 2]) and value network (`packed2` -> value2 [N])
-// in one pass over the observation.
+// packed2 != nullptr: policy (`packed` -> mean [N, 2]) and value network (`packed2` -> value2 [N]) in one pass over the
+// observation (either dtype).
 // sample != nullptr (policy head): the pass also samples the actions (kSample).
 int launch_policy_forward_ws(const void* obs, int obs_stride, int n_envs, const void* packed, float* mean,
                              bool value_head, bool bf16_in, cudaStream_t stream, const void* packed2, float* value2,
@@ -552,7 +573,7 @@ int launch_policy_forward_ws(const void* obs, int obs_stride, int n_envs, const 
     static int n_sms = 0;
     constexpr int kSmemBytes = (int)sizeof(WsSmem) + 1024, kSmemBytesDual = (int)sizeof(WsSmemT<true>) + 1024;
     const bool dual = packed2 != nullptr;
-    ROVER_CHECK(!(dual && (bf16_in || value2 == nullptr || value_head)), "policy + value pass: fp32 observations, two outputs");
+    ROVER_CHECK(!(dual && (value2 == nullptr || value_head)), "policy + value pass: two outputs");
     ROVER_CHECK(!(sample && value_head), "sampling needs the policy head");
     if (!encode) {
         int dev = 0;
@@ -567,6 +588,10 @@ int launch_policy_forward_ws(const void* obs, int obs_stride, int n_envs, const 
         ROVER_CUDA(cudaFuncSetAttribute(policy_forward_ws_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                         kSmemBytes));
         ROVER_CUDA(cudaFuncSetAttribute(policy_forward_ws_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        kSmemBytesDual));
+        ROVER_CUDA(cudaFuncSetAttribute(policy_forward_ws_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        kSmemBytesDual));
+        ROVER_CUDA(cudaFuncSetAttribute(policy_forward_ws_kernel<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                         kSmemBytesDual));
         void* fn = nullptr;
         cudaDriverEntryPointQueryResult q;
@@ -604,7 +629,9 @@ int launch_policy_forward_ws(const void* obs, int obs_stride, int n_envs, const 
                                  value_head ? 1 : 0, dual ? static_cast<const unsigned char*>(packed2) : no_net,
                                  dual ? value2 : no_out, sa);
     };
-    if (dual && sample) ROVER_CUDA(launch(policy_forward_ws_kernel<false, true, true>, kWsThreadsF32, kSmemBytesDual));
+    if (dual && bf16_in && sample) ROVER_CUDA(launch(policy_forward_ws_kernel<true, true, true>, kWsThreads, kSmemBytesDual));
+    else if (dual && bf16_in) ROVER_CUDA(launch(policy_forward_ws_kernel<true, true>, kWsThreads, kSmemBytesDual));
+    else if (dual && sample) ROVER_CUDA(launch(policy_forward_ws_kernel<false, true, true>, kWsThreadsF32, kSmemBytesDual));
     else if (dual) ROVER_CUDA(launch(policy_forward_ws_kernel<false, true>, kWsThreadsF32, kSmemBytesDual));
     else if (bf16_in && sample) ROVER_CUDA(launch(policy_forward_ws_kernel<true, false, true>, kWsThreads, kSmemBytes));
     else if (bf16_in) ROVER_CUDA(launch(policy_forward_ws_kernel<true>, kWsThreads, kSmemBytes));

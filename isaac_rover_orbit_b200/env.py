@@ -189,13 +189,20 @@ class RoverEnv:
     Random variates of the reset path come from the in-kernel counter-based generator keyed on ``seed`` (no torch
     generator call per step); ``set_variates`` feeds explicit arrays instead (parity tests).
     ``enable_cuda_graph()`` captures the whole step once; ``step`` then costs one action copy + one graph launch.
+    ``observation_dtype=torch.bfloat16``: the height scan also writes a bf16 mirror of the observation (same launch,
+    ``ops.height_scan_obs``), and ``reset`` / ``step`` return that mirror (``policy.alloc_obs_bf16`` layout) -- the operand
+    the policy and value networks read in place at half the bytes.  ``obs_buf`` stays fp32 and is written as before.
     """
 
     def __init__(self, cfg: RoverEnvCfg, terrain: TerrainTables, device="cuda:0", physics=None, seed: int = 0,
-                 physics_needs_targets: bool = True, scan_grid: "ops.ScanGridHandle | None" = None):
+                 physics_needs_targets: bool = True, scan_grid: "ops.ScanGridHandle | None" = None,
+                 observation_dtype: torch.dtype = torch.float32):
         from .mdp.actions import AckermannAction2
         from .mdp.commands import TerrainBasedPositionCommand
-        from .policy import alloc_obs
+        from .policy import alloc_obs, alloc_obs_bf16
+
+        if observation_dtype not in (torch.float32, torch.bfloat16):
+            raise ValueError(f"observation_dtype must be torch.float32 or torch.bfloat16, not {observation_dtype}")
 
         self.cfg = cfg
         self.device = torch.device(device)
@@ -225,6 +232,10 @@ class RoverEnv:
         self.command_manager = CommandManager(self, {"target_pose": TerrainBasedPositionCommand(cfg.commands, self)})
         # rows padded to 16 bytes: the policy kernel's TMA tensor map reads the buffer in place (no re-homing copy)
         self.obs_buf = alloc_obs(n, self.device, 4 + self.scene.sensors["height_scanner"].ray_pattern.n_rays)
+        self.observation_dtype = observation_dtype
+        # bf16: the mirror of obs_buf that the scan writes beside it (rows padded to 16 bytes, as the policy reads it)
+        self.obs_buf_bf16 = alloc_obs_bf16(n, self.device, self.obs_buf.shape[1]) if observation_dtype == torch.bfloat16 else None
+        self._obs_out = self.obs_buf if self.obs_buf_bf16 is None else self.obs_buf_bf16
         self.reward_buf = self._buf.reward
         self.reset_buf = self._buf.reset_flags
         # the kernels write 0 / 1 bytes: the bool tensors the reference returns are views, not per-step conversions
@@ -293,8 +304,15 @@ class RoverEnv:
         self._run_post(ids[:0], _lib.PHASE_METRICS | _lib.PHASE_COMMAND | _lib.PHASE_OBS, obs=self.obs_buf)
         self._scan()
         # a private copy: ``step`` refreshes ``obs_buf`` in place, and the reference's trainer keeps the tensor it got
-        # from ``reset`` as its ``states`` buffer (``states.copy_(next_states)``, skrl_utils.py:148)
-        return self.obs_buf.clone(), self.extras
+        # from ``reset`` as its ``states`` buffer (``states.copy_(next_states)``, skrl_utils.py:148).  The bf16 copy keeps
+        # the padded rows of alloc_obs_bf16 (a .clone() of the view comes back dense, a layout the bf16 kernels reject).
+        if self.obs_buf_bf16 is None:
+            return self.obs_buf.clone(), self.extras
+        from .policy import alloc_obs_bf16
+
+        states = alloc_obs_bf16(self.num_envs, self.device, self.obs_buf_bf16.shape[1])
+        states.copy_(self.obs_buf_bf16)
+        return states, self.extras
 
     def _reset_idx(self, idx):
         """rover_env.py:27-39 / ORBIT ``RLTaskEnv._reset_idx`` (A.2) for explicit ids."""
@@ -303,6 +321,14 @@ class RoverEnv:
     def _scan(self):
         robot = self.scene["robot"].data
         sensor = self.scene.sensors["height_scanner"]
+        if self.obs_buf_bf16 is not None:
+            # one launch: the fp32 heights (the term functions read obs_buf) and the bf16 mirror of columns 0..4+R-1
+            general = not sensor.cfg.attach_yaw_only or not sensor.ray_pattern.vertical_down
+            ops.height_scan_obs(robot.root_pos_w, robot.root_quat_w, sensor.ray_pattern, self.scan_grid, obs=self.obs_buf,
+                                obs_bf16=self.obs_buf_bf16, head_cols=4, max_distance=sensor.cfg.max_distance,
+                                base_offset=self.cfg.height_scan_base_offset, variant=ops.RAY_CAST_VARIANT if general else None,
+                                attach_yaw_only=sensor.cfg.attach_yaw_only)
+            return
         ops.height_scan(robot.root_pos_w, robot.root_quat_w, sensor.ray_pattern, self.scan_grid,
                         sensor.cfg.max_distance, self.cfg.height_scan_base_offset, out=self.obs_buf[:, 4:],
                         attach_yaw_only=sensor.cfg.attach_yaw_only)
@@ -393,4 +419,4 @@ class RoverEnv:
             self._step_body(action)
         self.common_step_counter += 1
         self._terms_current = True
-        return self.obs_buf, self.reward_buf, self.reset_terminated, self.reset_time_outs, self.extras
+        return self._obs_out, self.reward_buf, self.reset_terminated, self.reset_time_outs, self.extras

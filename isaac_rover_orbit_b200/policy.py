@@ -125,9 +125,7 @@ class _RoverNetwork:
 
     def _forward_bf16(self, states: torch.Tensor, value_head: bool) -> torch.Tensor:
         """bf16 observations ``[N, 965]`` (``alloc_obs_bf16`` layout): the TMA tile is the MMA operand, no conversion."""
-        if (not states.is_cuda or states.dtype != torch.bfloat16 or states.dim() != 2 or states.shape[1] != OBS_COLS
-                or states.stride(1) != 1 or states.stride(0) % 8 != 0 or states.data_ptr() % 16 != 0):
-            raise RuntimeError("compute_bf16: states must be a CUDA bf16 [N,965] view from alloc_obs_bf16()")
+        _check_bf16_states(states, "compute_bf16")
         if self._dirty:
             self._pack()
         return torch.ops.rover_b200.policy_forward(states, self._packed, value_head)
@@ -183,6 +181,13 @@ class GaussianNeuralNetwork(_RoverNetwork):
         return actions, log_prob, {"mean_actions": mean}
 
 
+def _check_bf16_states(states: torch.Tensor, what: str) -> None:
+    """bf16 states must already be in the ``alloc_obs_bf16`` layout (a copy into it would cost what the mirror saves)."""
+    if (not states.is_cuda or states.dtype != torch.bfloat16 or states.dim() != 2 or states.shape[1] != OBS_COLS
+            or states.stride(1) != 1 or states.stride(0) % 8 != 0 or states.data_ptr() % 16 != 0):
+        raise RuntimeError(f"{what}: states must be a CUDA bf16 [N,965] view from alloc_obs_bf16()")
+
+
 def _aligned_states(states: torch.Tensor, what: str) -> torch.Tensor:
     """fp32 ``[N,965]`` CUDA states with 16-byte aligned rows: the tensor itself, or one copy into ``alloc_obs``."""
     if not states.is_cuda or states.dtype != torch.float32 or states.dim() != 2 or states.shape[1] != OBS_COLS:
@@ -196,10 +201,15 @@ def _aligned_states(states: torch.Tensor, what: str) -> torch.Tensor:
 
 def policy_value_act(policy: "GaussianNeuralNetwork", value: "DeterministicNeuralNetwork", states: torch.Tensor, rng,
                      out_actions: torch.Tensor | None = None):
-    """``policy.act`` (sampled with ``rng``, an ``ops.ActionRng``) and the value network on fp32 ``states [N,965]`` in ONE
+    """``policy.act`` (sampled with ``rng``, an ``ops.ActionRng``) and the value network on ``states [N,965]`` in ONE
     launch (``rover_policy_value_act``): ``(actions [N,2], log_prob [N,1], value [N,1], mean [N,2])``, each bit-identical
-    to ``policy_value_forward`` followed by ``gaussian_act`` with ``rng.noise(N)``."""
-    states = _aligned_states(states, "policy_value_act")
+    to ``policy_value_forward`` followed by ``gaussian_act`` with ``rng.noise(N)``.  bf16 states (``alloc_obs_bf16``
+    layout) take ``rover_policy_value_act_bf16``."""
+    bf16 = states.dtype == torch.bfloat16
+    if bf16:
+        _check_bf16_states(states, "policy_value_act")
+    else:
+        states = _aligned_states(states, "policy_value_act")
     for net in (policy, value):
         if net._dirty:
             net._pack()
@@ -208,8 +218,8 @@ def policy_value_act(policy: "GaussianNeuralNetwork", value: "DeterministicNeura
     val = torch.empty(n, 1, dtype=torch.float32, device=states.device)
     actions = out_actions if out_actions is not None else torch.empty_like(mean)
     log_prob = torch.empty(n, 1, dtype=torch.float32, device=states.device)
-    torch.ops.rover_b200.policy_value_act(states, policy._packed, value._packed, policy.log_std_parameter, rng.state, 0, mean,
-                                          val, actions, log_prob)
+    op = torch.ops.rover_b200.policy_value_act_bf16 if bf16 else torch.ops.rover_b200.policy_value_act
+    op(states, policy._packed, value._packed, policy.log_std_parameter, rng.state, 0, mean, val, actions, log_prob)
     return actions, log_prob, val, mean
 
 
@@ -217,17 +227,23 @@ def policy_value_forward(policy: "GaussianNeuralNetwork", value: "DeterministicN
     """Policy mean ``[N,2]`` and value ``[N,1]`` of ``states [N,965]`` (fp32) in ONE pass over the observation
     (``rover_policy_value_forward``): what a PPO rollout evaluates every step -- ``policy.act`` in the trainer loop
     (skrl_utils.py:139-142) and ``value.act`` in ``record_transition`` (models.py:89-102 + :151-162).  Bit-identical to
-    ``policy.compute`` / ``value.compute``."""
-    if not states.is_cuda or states.dtype != torch.float32 or states.dim() != 2 or states.shape[1] != OBS_COLS:
-        raise RuntimeError("policy_value_forward: states must be a CUDA fp32 [N,965] tensor")
-    if states.stride(1) != 1 or states.stride(0) % 4 != 0 or states.data_ptr() % 16 != 0:
-        buf = alloc_obs(states.shape[0], states.device)
-        buf.copy_(states)
-        states = buf
+    ``policy.compute`` / ``value.compute``.  bf16 states (``alloc_obs_bf16`` layout) take
+    ``rover_policy_value_forward_bf16``: one pass over the bf16 mirror, bit-identical to ``compute_bf16`` of both."""
+    bf16 = states.dtype == torch.bfloat16
+    if bf16:
+        _check_bf16_states(states, "policy_value_forward")
+    else:
+        if not states.is_cuda or states.dtype != torch.float32 or states.dim() != 2 or states.shape[1] != OBS_COLS:
+            raise RuntimeError("policy_value_forward: states must be a CUDA fp32 [N,965] tensor")
+        if states.stride(1) != 1 or states.stride(0) % 4 != 0 or states.data_ptr() % 16 != 0:
+            buf = alloc_obs(states.shape[0], states.device)
+            buf.copy_(states)
+            states = buf
     for net in (policy, value):
         if net._dirty:
             net._pack()
-    return torch.ops.rover_b200.policy_value_forward(states, policy._packed, value._packed)
+    op = torch.ops.rover_b200.policy_value_forward_bf16 if bf16 else torch.ops.rover_b200.policy_value_forward
+    return op(states, policy._packed, value._packed)
 
 
 class DeterministicNeuralNetwork(_RoverNetwork):

@@ -81,6 +81,7 @@ _SCHEMAS = {
     "policy_mlp_forward": "(Tensor enc, Tensor packed, bool value_head) -> Tensor",
     "policy_forward": "(Tensor obs, Tensor packed, bool value_head) -> Tensor",
     "policy_value_forward": "(Tensor obs, Tensor packed_policy, Tensor packed_value) -> (Tensor, Tensor)",
+    "policy_value_forward_bf16": "(Tensor obs, Tensor packed_policy, Tensor packed_value) -> (Tensor, Tensor)",
     "gaussian_act": "(Tensor mean, Tensor log_std, Tensor eps) -> (Tensor, Tensor)",
     "gaussian_act_out": "(Tensor mean, Tensor log_std, Tensor eps, Tensor(a!) actions, Tensor(b!) log_prob) -> ()",
     # ---- the forward pass with GaussianMixin.act in its last epilogue: noise keyed on (seed, step, env_offset + env)
@@ -88,6 +89,8 @@ _SCHEMAS = {
                   "Tensor(c!) actions, Tensor(d!) log_prob) -> ()",
     "policy_value_act": "(Tensor obs, Tensor packed_policy, Tensor packed_value, Tensor log_std, Tensor(a!) rng_state, "
                         "int env_offset, Tensor(b!) mean, Tensor(c!) value, Tensor(d!) actions, Tensor(e!) log_prob) -> ()",
+    "policy_value_act_bf16": "(Tensor obs, Tensor packed_policy, Tensor packed_value, Tensor log_std, Tensor(a!) rng_state, "
+                             "int env_offset, Tensor(b!) mean, Tensor(c!) value, Tensor(d!) actions, Tensor(e!) log_prob) -> ()",
     "action_noise": "(Tensor(a!) rng_state, int env_offset, int n_envs, bool advance) -> Tensor",
     # ---- PPO returns and advantages over the rollout memory (skrl PPO._update -> compute_gae)
     "ppo_gae": "(Tensor rewards, Tensor dones, Tensor values, Tensor last_values, float discount_factor, "
@@ -522,6 +525,35 @@ def _policy_value_forward(obs, packed_policy, packed_value):
     return mean, value
 
 
+def _bf16_obs(what, obs):
+    """The layout of ``policy.alloc_obs_bf16``: bf16 [N,965], unit inner stride, rows a multiple of 8 elements, 16-byte
+    aligned -- what the TMA tile of the bf16 passes reads."""
+    if (obs.dtype != torch.bfloat16 or obs.dim() != 2 or obs.shape[1] != 965 or obs.stride(1) != 1 or obs.stride(0) % 8 != 0
+            or obs.data_ptr() % 16 != 0):
+        raise RuntimeError(f"rover_b200::{what}: bf16 states must be a [N,965] view from alloc_obs_bf16()")
+
+
+def _packed_pair(what, obs, packed_policy, packed_value):
+    size = policy_packed_bytes()
+    for t in (packed_policy, packed_value):
+        if not t.is_cuda or t.device != obs.device or t.dtype != torch.uint8 or t.numel() != size or not t.is_contiguous():
+            raise RuntimeError(f"rover_b200::{what}: packed blobs must be contiguous uint8 [{size}] tensors on the states' "
+                               "device (policy_pack)")
+
+
+def _policy_value_forward_bf16(obs, packed_policy, packed_value):
+    _bf16_obs("policy_value_forward_bf16", obs)
+    if not obs.is_cuda:
+        raise RuntimeError("rover_b200::policy_value_forward_bf16: states must be a CUDA tensor")
+    _packed_pair("policy_value_forward_bf16", obs, packed_policy, packed_value)
+    n = obs.shape[0]
+    mean = torch.empty(n, 2, dtype=torch.float32, device=obs.device)
+    value = torch.empty(n, 1, dtype=torch.float32, device=obs.device)
+    _lib.check(_lib.load().rover_policy_value_forward_bf16(_p(obs), int(obs.stride(0)), n, _p(packed_policy), _p(packed_value),
+                                                           _p(mean), _p(value), _stream(obs)))
+    return mean, value
+
+
 def _gaussian_act_out(mean, log_std, eps, actions, log_prob):
     _f32("gaussian_act_out", mean, log_std, eps, actions, log_prob)
     n = mean.shape[0]
@@ -542,9 +574,8 @@ def _gaussian_act(mean, log_std, eps):
 def _act_checks(what, obs, log_std, rng_state, env_offset, mean, actions, log_prob, value=None):
     """The checks of the sampling operators: what the forward operators check on ``obs``, plus the sampling tensors."""
     n = obs.shape[0] if obs.dim() == 2 else -1
-    if obs.dtype == torch.bfloat16 and what == "policy_act":
-        if obs.dim() != 2 or obs.shape[1] != 965 or obs.stride(1) != 1 or obs.stride(0) % 8 != 0 or obs.data_ptr() % 16 != 0:
-            raise RuntimeError(f"rover_b200::{what}: bf16 states must be a [N,965] view from alloc_obs_bf16()")
+    if what == "policy_value_act_bf16" or (obs.dtype == torch.bfloat16 and what == "policy_act"):
+        _bf16_obs(what, obs)
     elif (obs.dtype != torch.float32 or obs.dim() != 2 or obs.shape[1] != 965 or obs.stride(1) != 1
             or obs.stride(0) % 4 != 0 or obs.data_ptr() % 16 != 0):
         raise RuntimeError(f"rover_b200::{what}: states must be fp32 [N,965] with 16-byte aligned rows")
@@ -578,6 +609,14 @@ def _policy_value_act(obs, packed_policy, packed_value, log_std, rng_state, env_
     _lib.check(_lib.load().rover_policy_value_act(_p(obs), int(obs.stride(0)), n, _p(packed_policy), _p(packed_value),
                                                   _p(log_std), _p(rng_state), int(env_offset), _p(mean), _p(value),
                                                   _p(actions), _p(log_prob), _stream(obs)))
+
+
+def _policy_value_act_bf16(obs, packed_policy, packed_value, log_std, rng_state, env_offset, mean, value, actions, log_prob):
+    n = _act_checks("policy_value_act_bf16", obs, log_std, rng_state, env_offset, mean, actions, log_prob, value)
+    _packed_pair("policy_value_act_bf16", obs, packed_policy, packed_value)
+    _lib.check(_lib.load().rover_policy_value_act_bf16(_p(obs), int(obs.stride(0)), n, _p(packed_policy), _p(packed_value),
+                                                       _p(log_std), _p(rng_state), int(env_offset), _p(mean), _p(value),
+                                                       _p(actions), _p(log_prob), _stream(obs)))
 
 
 def _action_noise(rng_state, env_offset, n_envs, advance):
@@ -680,6 +719,7 @@ _IMPLS = {
     "scan_encoder_fused": _scan_encoder_fused, "policy_mlp_forward": _policy_mlp_forward, "mesh_to_heightmap": _mesh_to_heightmap,
     "steep_mask": _steep_mask, "morph_box": _morph_box, "fill_holes": _fill_holes, "ppo_gae": _ppo_gae,
     "policy_act": _policy_act, "policy_value_act": _policy_value_act, "action_noise": _action_noise,
+    "policy_value_forward_bf16": _policy_value_forward_bf16, "policy_value_act_bf16": _policy_value_act_bf16,
 }
 for _name, _fn in _IMPLS.items():
     _IMPL.impl(_name, _fn)
@@ -728,6 +768,11 @@ def _(obs, packed_policy, packed_value):
     return obs.new_empty(obs.shape[0], 2, dtype=torch.float32), obs.new_empty(obs.shape[0], 1, dtype=torch.float32)
 
 
+@_fake("policy_value_forward_bf16")
+def _(obs, packed_policy, packed_value):
+    return obs.new_empty(obs.shape[0], 2, dtype=torch.float32), obs.new_empty(obs.shape[0], 1, dtype=torch.float32)
+
+
 @_fake("scan_encoder_fused")
 def _(pos_w, quat_w, ray_starts, pattern_box, grid, cells, max_distance, base_offset, obs, write_obs, packed_fused):
     return pos_w.new_empty(pos_w.shape[0], 64, dtype=torch.bfloat16)
@@ -769,7 +814,8 @@ def _fake_none(*args, **kwargs):
 
 for _name in ("height_scan_out", "ray_cast_out", "height_scan_obs", "height_scan_host", "ray_cast_obs", "ray_cast_host",
               "gaussian_act_out", "mdp_pre_step", "mdp_post_step", "mdp_step", "step_fused", "stats_read", "policy_pack",
-              "policy_pack_fused", "mesh_to_heightmap", "ppo_gae", "policy_act", "policy_value_act"):
+              "policy_pack_fused", "mesh_to_heightmap", "ppo_gae", "policy_act", "policy_value_act",
+              "policy_value_act_bf16"):
     torch.library.register_fake(f"{NS}::{_name}", _fake_none, lib=_DEF)
 
 OPS = tuple(_SCHEMAS)

@@ -143,8 +143,9 @@ class RolloutAgent(BaseAgent):
         ``record_transition`` on the states ``act`` just saw; here both networks run in ONE pass over the observation
         (``policy.policy_value_forward``) and the values are written to the memory's ``values`` tensor.
         ``action_rng`` (an ``ops.ActionRng``): the policy samples inside its forward pass with noise keyed on
-        (seed, step, env) instead of ``torch.randn`` -- one launch per ``act``, policy and value together on fp32 states
-        (``policy.policy_value_act``); without it ``act`` draws ``torch.randn`` as before."""
+        (seed, step, env) instead of ``torch.randn`` -- one launch per ``act``, policy and value together
+        (``policy.policy_value_act``); without it ``act`` draws ``torch.randn`` as before.  fp32 states and the bf16 mirror
+        (``alloc_obs_bf16`` layout, what ``RoverEnv(observation_dtype=torch.bfloat16)`` returns) take the same routes."""
         super().__init__()
         self.policy = policy
         self.value = value
@@ -163,14 +164,14 @@ class RolloutAgent(BaseAgent):
             memory.create_tensor("log_prob", 1)
 
     def act(self, states: torch.Tensor, timestep: int, timesteps: int):
-        if self.action_rng is not None and self.value is not None and states.dtype == torch.float32:
+        if self.action_rng is not None and self.value is not None:
             from .policy import policy_value_act
 
             actions, log_prob, self._values, mean = policy_value_act(self.policy, self.value, states, self.action_rng,
                                                                      out_actions=self.action_out)
             self._log_prob = log_prob
             return actions, log_prob, {"mean_actions": mean}
-        if self.value is None or states.dtype != torch.float32:
+        if self.value is None:
             extra = {"out_actions": self.action_out} if self.action_out is not None else {}  # (any skrl-style policy works)
             if self.action_rng is not None:
                 extra["rng"] = self.action_rng
