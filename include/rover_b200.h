@@ -449,7 +449,8 @@ typedef struct RoverPolicyWeights {
     int32_t in_dim[6], out_dim[6];  /* out_dim[5] = 2 (policy mean) or 1 (value) */
 } RoverPolicyWeights;
 
-/* returns the number of bytes the packed blob needs (when packed == NULL) or packs into it */
+/* returns the number of bytes the packed blob needs (when packed == NULL) or packs into it.  The encoder input width is
+ * R = in_dim[0] (1 <= R <= 4092; the layout of rover_policy_pass); weights == packed == NULL: the size for R = 961. */
 int64_t rover_policy_pack(const RoverPolicyWeights* weights /* host struct, device pointers */, void* packed,
                           void* stream);
 /* obs [N, obs_stride] fp32 (965 columns used), rows 16-byte aligned (obs_stride % 4 == 0); mean [N,2] fp32 */
@@ -537,6 +538,39 @@ int rover_policy_value_act(const float* obs, int32_t obs_stride, int32_t n_envs,
 int rover_policy_value_act_bf16(const uint16_t* obs_bf16, int32_t stride, int32_t n_envs, const void* packed_policy,
                                 const void* packed_value, const float* log_std, int64_t* rng_state, int32_t env_offset,
                                 float* mean, float* value, float* actions, float* log_prob, void* stream);
+/* Every forward / act form above for an encoder of any input width R (GaussianNeuralNetwork / DeterministicNeuralNetwork
+ * with encoder_input_size = R, models.py:24-36, 89-102, 151-162): the scan's R rays, an observation of 4 + R columns, the
+ * encoder reading s[:, 3:-1] = columns [3, 3 + R) (heading column in, last ray out, as the reference slices).  The MLP
+ * behind the encoder is the fixed one (80 -> 60, 64 -> 256 -> 160 -> 128 -> 2 | 1).  Blobs come from rover_policy_pack
+ * with in_dim[0] = R: W0 in ceil((3 + R) / 64) chunks of 10,240 B, then layers 1-5 and the biases (at R = 961 the blob
+ * of the entries above, byte for byte, and every result equals theirs bit for bit).
+ *   obs [n_envs, stride]: fp32 (obs_dtype ROVER_OBS_FP32, stride >= 4 + R, stride % 4 == 0) or the bf16 mirror
+ *     (ROVER_OBS_BF16, stride >= 3 + R, stride % 8 == 0), rows 16-byte aligned.  1 <= enc_in = R <= 4092.
+ *   out: mean [N,2] (tanh), or value [N] with value_head != 0.
+ *   packed_value != NULL: the value network in the same pass (value [N]; policy head only), as
+ *     rover_policy_value_forward; both blobs packed for the same R.
+ *   log_std, rng_state, actions all non-NULL: the pass samples as rover_policy_act (env_offset, log_prob optional);
+ *     all NULL: no sampling (log_prob must then be NULL). */
+#define ROVER_OBS_FP32 0
+#define ROVER_OBS_BF16 1
+typedef struct RoverPolicyPass {
+    const void* obs;
+    const void* packed;
+    const void* packed_value;  /* NULL: one network */
+    float* out;                /* mean [N,2] or value [N] */
+    float* value;              /* [N] with packed_value, else NULL */
+    const float* log_std;      /* [2]; sampling */
+    int64_t* rng_state;        /* {seed, step}; sampling */
+    float* actions;            /* [N,2]; sampling */
+    float* log_prob;           /* [N] or NULL; sampling */
+    int32_t obs_dtype;         /* ROVER_OBS_FP32 / ROVER_OBS_BF16 */
+    int32_t stride;            /* elements per observation row */
+    int32_t n_envs;
+    int32_t enc_in;            /* R */
+    int32_t value_head;
+    int32_t env_offset;        /* sampling: first env's index in the noise stream */
+} RoverPolicyPass;
+int rover_policy_pass(const RoverPolicyPass* pass /* host struct, device pointers */, void* stream);
 /* The eps [N,2] (8-byte aligned) that the next rover_policy_*act launch with rng_state and env_offset draws, computed on
  * the device with the same code (host libm's log / sin / cos round differently).  advance != 0: the step advances by one
  * as an act launch would; advance == 0 leaves rng_state unchanged.  Feed it to rover_gaussian_act to reproduce an act

@@ -32,7 +32,7 @@ SYMBOLS = ("rover_abi_version", "rover_last_error", "rover_height_scan", "rover_
            "rover_fill_holes", "rover_step_fused", "rover_ray_cast", "rover_ray_cast_obs", "rover_ray_cast_obs_bf16",
            "rover_ray_cast_host", "rover_ppo_gae", "rover_ppo_gae_work_bytes", "rover_mdp_math", "rover_policy_act",
            "rover_policy_act_bf16", "rover_policy_value_act", "rover_action_noise", "rover_policy_math",
-           "rover_policy_value_forward_bf16", "rover_policy_value_act_bf16")
+           "rover_policy_value_forward_bf16", "rover_policy_value_act_bf16", "rover_policy_pass")
 
 
 class ScanLevel(C.Structure):
@@ -106,6 +106,29 @@ class TerrainTables(C.Structure):
 
 class PolicyWeights(C.Structure):
     _fields_ = [("w", C.c_void_p * 6), ("b", C.c_void_p * 6), ("in_dim", C.c_int32 * 6), ("out_dim", C.c_int32 * 6)]
+
+
+OBS_FP32, OBS_BF16 = 0, 1
+ENC_IN = 961       # the shipped task's encoder input width (a 31 x 31 scan)
+ENC_IN_MAX = 4092  # observations of up to 4096 columns
+
+
+class PolicyPass(C.Structure):
+    """``RoverPolicyPass``: one forward / act pass of the policy (and value) network for encoder input width R."""
+
+    _fields_ = [("obs", C.c_void_p), ("packed", C.c_void_p), ("packed_value", C.c_void_p), ("out", C.c_void_p),
+                ("value", C.c_void_p), ("log_std", C.c_void_p), ("rng_state", C.c_void_p), ("actions", C.c_void_p),
+                ("log_prob", C.c_void_p), ("obs_dtype", C.c_int32), ("stride", C.c_int32), ("n_envs", C.c_int32),
+                ("enc_in", C.c_int32), ("value_head", C.c_int32), ("env_offset", C.c_int32)]
+
+
+def check_enc_in(enc_in) -> int:
+    """The encoder input width R (the scan's ray count) as an int, or ``ValueError`` outside ``[1, ENC_IN_MAX]``."""
+    r = int(enc_in)
+    if r != enc_in or not 1 <= r <= ENC_IN_MAX:
+        raise ValueError(f"encoder input width {enc_in!r} is outside [1, {ENC_IN_MAX}] (observations of 4 + R <= "
+                         f"{ENC_IN_MAX + 4} columns)")
+    return r
 
 
 _lib = None
@@ -241,6 +264,8 @@ def load() -> C.CDLL:
     lib.rover_action_noise.argtypes = [vp, i32, i32, vp, i32, vp]
     lib.rover_policy_math.restype = C.c_int
     lib.rover_policy_math.argtypes = [i32, vp, vp, vp, i32, vp]
+    lib.rover_policy_pass.restype = C.c_int
+    lib.rover_policy_pass.argtypes = [C.POINTER(PolicyPass), vp]
     _lib = lib
     return lib
 

@@ -291,11 +291,14 @@ struct PackArgs {
     int in_dim[6], out_dim[6];
 };
 
+// layer 0 reads R = in_dim[0] columns into w0_chunks(R) chunks; layers 1-5 and the biases follow w0_shift(R) bytes
+// further along than in the R = 961 layout (policy_common.cuh)
 __global__ void policy_pack_kernel(const __grid_constant__ PackArgs a, unsigned char* __restrict__ packed) {
     const int l = blockIdx.y;
-    const int k_pad = layer_k(l), n_pad = layer_n(l), k_real = layer_k_real(l), n_real = a.out_dim[l];
-    __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(packed + weight_offset(l));
-    const int total = (l == 0 ? kNumChunks * kChunkK : k_pad) * n_pad;
+    const int enc_in = a.in_dim[0], shift = l == 0 ? 0 : w0_shift(enc_in);
+    const int k_pad = layer_k(l), n_pad = layer_n(l), k_real = l == 0 ? enc_in : layer_k_real(l), n_real = a.out_dim[l];
+    __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(packed + shift + weight_offset(l));
+    const int total = (l == 0 ? w0_chunks(enc_in) * kChunkK : k_pad) * n_pad;
     for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += gridDim.x * blockDim.x) {
         // idx enumerates (plane-major) the packed image: [chunk][plane][n][8] for layer 0, [plane][n][8] otherwise
         const int j = idx & 7;
@@ -309,7 +312,7 @@ __global__ void policy_pack_kernel(const __grid_constant__ PackArgs a, unsigned 
         if (n < n_real && src_k >= 0 && src_k < k_real) v = a.w[l][(size_t)n * a.in_dim[l] + src_k];
         dst[idx] = __float2bfloat16_rn(v);
     }
-    float* bdst = reinterpret_cast<float*>(packed + bias_offset(l));
+    float* bdst = reinterpret_cast<float*>(packed + w0_shift(enc_in) + bias_offset(l));
     for (int n = blockIdx.x * blockDim.x + threadIdx.x; n < n_pad; n += gridDim.x * blockDim.x)
         bdst[n] = n < n_real ? a.b[l][n] : 0.f;
 }
@@ -366,23 +369,30 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
 
 int launch_policy_forward_ws(const void* obs, int obs_stride, int n_envs, const void* packed, float* out,
                              bool value_head, bool bf16_in, cudaStream_t stream, const void* packed2 = nullptr,
-                             float* value2 = nullptr, const SampleArgs* sample = nullptr);  // policy_ws.cu
+                             float* value2 = nullptr, const SampleArgs* sample = nullptr,
+                             int enc_in = kEncIn);  // policy_ws.cu
 
 }  // namespace rover
 
 extern "C" int64_t rover_policy_pack(const RoverPolicyWeights* weights, void* packed, void* stream) {
     using namespace rover;
-    if (packed == nullptr) return kPackedBytes;
+    if (packed == nullptr && weights == nullptr) return kPackedBytes;
     if (weights == nullptr) {
         fail("rover_policy_pack: weights is NULL");
         return -1;
     }
+    const int enc_in = weights->in_dim[0];  // R: the encoder input width
+    if (enc_in < 1 || enc_in > kEncInMax) {
+        fail("rover_policy_pack: encoder input width %d outside [1, %d]", enc_in, kEncInMax);
+        return -1;
+    }
+    if (packed == nullptr) return packed_bytes(enc_in);
     PackArgs a;
     for (int l = 0; l < 6; ++l) {
         const bool out_ok = weights->out_dim[l] == layer_n_real(l) || (l == 5 && weights->out_dim[l] == 1);  // value head
-        if (!weights->w[l] || !weights->b[l] || weights->in_dim[l] < layer_k_real(l) || !out_ok) {
+        if (!weights->w[l] || !weights->b[l] || (l > 0 && weights->in_dim[l] < layer_k_real(l)) || !out_ok) {
             fail("rover_policy_pack: layer %d has shape [%d,%d], expected [%d,%d]", l, weights->out_dim[l],
-                 weights->in_dim[l], layer_n_real(l), layer_k_real(l));
+                 weights->in_dim[l], layer_n_real(l), l == 0 ? enc_in : layer_k_real(l));
             return -1;
         }
         a.w[l] = weights->w[l];
@@ -391,7 +401,7 @@ extern "C" int64_t rover_policy_pack(const RoverPolicyWeights* weights, void* pa
         a.out_dim[l] = weights->out_dim[l];
     }
     policy_pack_kernel<<<dim3(64, 6), 256, 0, static_cast<cudaStream_t>(stream)>>>(a, static_cast<unsigned char*>(packed));
-    return check_launch("policy_pack_kernel") ? -1 : kPackedBytes;
+    return check_launch("policy_pack_kernel") ? -1 : packed_bytes(enc_in);
 }
 
 static int policy_or_value_forward(const float* obs, int32_t obs_stride, int32_t n_envs, const void* packed, float* mean,
@@ -597,6 +607,48 @@ extern "C" int rover_policy_value_act_bf16(const uint16_t* obs_bf16, int32_t str
     const SampleArgs s{log_std, reinterpret_cast<unsigned long long*>(rng_state), (uint32_t)env_offset, actions, log_prob};
     return launch_policy_forward_ws(obs_bf16, stride, n_envs, packed_policy, mean, false, true, static_cast<cudaStream_t>(stream),
                                     packed_value, value, &s);
+}
+
+// ---------------------------------------------------------------------------------------------------- any encoder width
+extern "C" int rover_policy_pass(const RoverPolicyPass* p, void* stream) {
+    using namespace rover;
+    ROVER_CHECK(p != nullptr, "rover_policy_pass: NULL descriptor");
+    ROVER_CHECK(p->n_envs >= 0, "rover_policy_pass: negative n_envs");
+    ROVER_CHECK(p->enc_in >= 1 && p->enc_in <= kEncInMax, "rover_policy_pass: encoder input width %d outside [1, %d]",
+                p->enc_in, kEncInMax);
+    ROVER_CHECK(p->obs_dtype == ROVER_OBS_FP32 || p->obs_dtype == ROVER_OBS_BF16,
+                "rover_policy_pass: obs_dtype must be ROVER_OBS_FP32 or ROVER_OBS_BF16");
+    if (p->n_envs == 0) return 0;
+    const bool bf16 = p->obs_dtype == ROVER_OBS_BF16, dual = p->packed_value != nullptr;
+    const bool sample = p->log_std != nullptr || p->rng_state != nullptr || p->actions != nullptr;
+    ROVER_CHECK(p->obs && p->packed && p->out, "rover_policy_pass: NULL argument");
+    // fp32: the map reads columns [0, 4 + R) (4 floats per 16 bytes); bf16: [0, 3 + R) (8 per 16 bytes)
+    const int min_stride = kEncInOffset + p->enc_in + (bf16 ? 0 : 1), align = bf16 ? 8 : 4;
+    ROVER_CHECK(p->stride >= min_stride && p->stride % align == 0 && (reinterpret_cast<uintptr_t>(p->obs) & 15) == 0,
+                "rover_policy_pass: observation rows must hold %d columns and be 16-byte aligned (stride >= %d, stride %% %d "
+                "== 0, got %d)", min_stride, min_stride, align, p->stride);
+    ROVER_CHECK((reinterpret_cast<uintptr_t>(p->packed) & 127) == 0, "rover_policy_pass: packed blob not 128B aligned");
+    ROVER_CHECK(p->value_head || (reinterpret_cast<uintptr_t>(p->out) & 7) == 0,
+                "rover_policy_pass: the mean output [N,2] must be 8-byte aligned");
+    if (dual) {
+        ROVER_CHECK(p->value != nullptr && !p->value_head, "rover_policy_pass: packed_value needs value and the policy head");
+        ROVER_CHECK((reinterpret_cast<uintptr_t>(p->packed_value) & 127) == 0, "rover_policy_pass: packed blob not 128B aligned");
+    } else {
+        ROVER_CHECK(p->value == nullptr, "rover_policy_pass: value is written only with packed_value");
+    }
+    if (!sample) {
+        ROVER_CHECK(p->log_prob == nullptr, "rover_policy_pass: log_prob is written only when sampling");
+        return launch_policy_forward_ws(p->obs, p->stride, p->n_envs, p->packed, p->out, p->value_head != 0, bf16,
+                                        static_cast<cudaStream_t>(stream), p->packed_value, p->value, nullptr, p->enc_in);
+    }
+    ROVER_CHECK(!p->value_head, "rover_policy_pass: sampling needs the policy head");
+    if (int rc = check_act_args("rover_policy_pass", p->n_envs, p->packed, p->log_std, p->rng_state, p->env_offset, p->out,
+                                p->actions))
+        return rc;
+    const SampleArgs s{p->log_std, reinterpret_cast<unsigned long long*>(p->rng_state), (uint32_t)p->env_offset, p->actions,
+                       p->log_prob};
+    return launch_policy_forward_ws(p->obs, p->stride, p->n_envs, p->packed, p->out, false, bf16,
+                                    static_cast<cudaStream_t>(stream), p->packed_value, p->value, &s, p->enc_in);
 }
 
 extern "C" int rover_action_noise(int64_t* rng_state, int32_t env_offset, int32_t n_envs, float* eps_out, int32_t advance,

@@ -45,6 +45,16 @@ __host__ __device__ constexpr int bias_offset(int l) {
 }
 constexpr int kPackedBytes = bias_offset(kNumLayers);
 
+// Encoder input width R (the scan's ray count; the encoder reads observation columns [3, 3 + R)) of the warp-specialised
+// kernel and of rover_policy_pass: W0 holds ceil((3 + R) / 64) chunks, and everything behind W0 moves by the difference
+// to the 16 chunks of R = 961 (the blob of R = 961 is the blob above, byte for byte).  4092: observations up to 4096
+// columns.
+constexpr int kEncInMax = 4092;
+__host__ __device__ constexpr int w0_chunks(int enc_in) { return (kEncInOffset + enc_in + kChunkK - 1) / kChunkK; }
+__host__ __device__ constexpr int w0_shift(int enc_in) { return (w0_chunks(enc_in) - kNumChunks) * kW0ChunkBytes; }
+__host__ __device__ constexpr int packed_bytes(int enc_in) { return kPackedBytes + w0_shift(enc_in); }
+static_assert(w0_chunks(kEncIn) == kNumChunks && packed_bytes(kEncIn) == kPackedBytes, "R = 961 is the fixed-width blob");
+
 // ---------------------------------------------------------------------------------------------------- PTX helpers
 __device__ __forceinline__ uint32_t sptr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mb_init(unsigned long long* b, uint32_t n) {

@@ -28,6 +28,12 @@
 // (the policy's four K = 16 MMAs into D0[buf] columns 0-79, then the value network's four into columns 80-159); 352
 // threads, no converter warps; the TMEM plan is the fp32 dual plan.  Shared memory: the 4-stage observation ring of the
 // dual layout, and a W0 ring of TWO 20 KB stages (both networks' 10 KB chunks) overlaid on a_bf16[] + w0[] (46 KB).
+//
+// Encoder width: `enc_in` = R (1 <= R <= kEncInMax) is a launch argument.  Layer 0 streams ceil((3 + R) / 32) fp32 or
+// ceil((3 + R) / 64) bf16 chunks of observation columns and as many W0 ring stages; the tensor map ends the observation
+// at column 4 + R (fp32; the converters zero columns outside [3, 3 + R)) or 3 + R (bf16) and zero-fills the tail chunk.
+// Layers 1-5 and the biases sit w0_shift(R) bytes further along the blob than at R = 961.  Nothing else depends on R:
+// W0 is streamed, so no stage, TMEM column or epilogue grows with it.
 #include "policy_common.cuh"
 
 #ifndef ROVER_POLICY_DBG
@@ -52,7 +58,6 @@ __device__ unsigned long long g_pol_cta[2][256];  // globaltimer (ns) at CTA sta
 constexpr int kWsThreads = 352;        // bf16 observations: warps 0-10
 constexpr int kWsThreadsF32 = 480;     // fp32 observations: + warps 11-14, a second converter warpgroup
 constexpr int kWsChunkK = 32;
-constexpr int kWsChunks = 31;  // observation columns [0, 992) cover the encoder input [3, 964)
 constexpr int kWsStagesF = 5;
 constexpr int kWsStagesFDual = 4;  // the second W0 image takes the shared memory of one observation stage
 constexpr int kWsStagesA = 2;
@@ -71,7 +76,6 @@ static_assert(kW0ChunkBytes == 2 * kWsW0Chunk, "a 32-column chunk is half of a p
 // rover_height_scan_obs), so a TMA tile of 64 columns x tile rows (128 B per row, SWIZZLE_128B) IS the A operand of
 // the MMA (canonical K-major SWIZZLE_128B layout) -- no conversion stage, half the HBM bytes.
 constexpr int kBfChunkK = 64;
-constexpr int kBfChunks = 16;                 // columns [0, 1024); beyond column 963 the tensor map zero-fills
 constexpr int kBfStagesW = 3;                 // 10 KB W0 chunks in the space of a_bf16[] + w0[]
 constexpr int kBfStagesWDual = 2;             // 2 x 10 KB (policy + value) W0 chunks in the same space of the dual layout
 
@@ -117,7 +121,7 @@ __global__ void __launch_bounds__(kBf16In ? kWsThreads : kWsThreadsF32, 1)
 policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const float* __restrict__ obs, int obs_stride,
                          int n_envs, int tile_rows, const unsigned char* __restrict__ packed, float* __restrict__ mean,
                          int value_head, const unsigned char* __restrict__ packed2, float* __restrict__ value2,
-                         const __grid_constant__ SampleArgs sample) {
+                         const __grid_constant__ SampleArgs sample, int enc_in) {
     using Smem = WsSmemT<kDual>;
     constexpr int kNets = Smem::kNets, kStagesFK = Smem::kStagesFT;
     constexpr uint32_t kColD0Stride = kDual ? kWsColD0StrideDual : kWsColD0Stride, kColAcc = kDual ? kWsColAccDual : kWsColAcc;
@@ -130,8 +134,10 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
     // rounds of the grid: 65536 envs on 148 SMs -> 586 tiles of 112 instead of 512 of 128 = 3.96 instead of 3.46 -> 4
     // rounds).  The MMAs stay M = 128; accumulator rows >= tile_rows hold garbage and are never stored.
     const int n_tiles = (n_envs + tile_rows - 1) / tile_rows;
-    constexpr int kChunks = kBf16In ? kBfChunks : kWsChunks;
     constexpr int kChunkK = kBf16In ? kBfChunkK : kWsChunkK;        // observation columns per chunk
+    const int n_chunks = (kEncInOffset + enc_in + kChunkK - 1) / kChunkK;  // layer-0 K chunks: columns [0, 3 + R)
+    const int w_shift = w0_shift(enc_in);                           // layers 1-5 and biases behind the W0 chunks
+    const int blob_bytes = kPackedBytes + w_shift;
     constexpr int kStagesW = kBf16In ? (kDual ? kBfStagesWDual : kBfStagesW) : kWsStagesW;
     constexpr int kW0Chunk = kBf16In ? kW0ChunkBytes : kWsW0Chunk;  // bytes of ONE packed W0 image per chunk
     constexpr int kW0Stage = kNets * kW0Chunk;                      // bytes of a W0 ring stage
@@ -158,7 +164,7 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
         // (common.cuh) everything above -- and the weight loads, the TMEM allocation of the other warps -- overlaps its tail
         grid_dependency_wait();
         if ((int)blockIdx.x < n_tiles)
-            for (int c = 0; c < kStagesFK; ++c) {
+            for (int c = 0; c < kStagesFK && c < n_chunks; ++c) {
                 mb_expect_tx(&sm.f_full[c], chunk_bytes);
                 tma_2d(sm.stage_f[c], &obs_map, c * kChunkK, blockIdx.x * tile_rows, &sm.f_full[c]);
             }
@@ -202,7 +208,7 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
             bool first = true;  // chunks 0 .. kStagesFK-1 of the first tile were issued in the prologue
             for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
                 const int row0 = tile * tile_rows;
-                for (int c = 0; c < kChunks; ++c) {
+                for (int c = 0; c < n_chunks; ++c) {
                     if (!(first && c < kStagesFK)) {
                         mb_wait(&sm.f_empty[sf], (pf & 1u) ^ 1u);
                         mb_expect_tx(&sm.f_full[sf], chunk_bytes);
@@ -221,7 +227,7 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
             int sw = 0;
             uint32_t pw = 0;
             for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-                for (int c = 0; c < kChunks; ++c) {
+                for (int c = 0; c < n_chunks; ++c) {
                     mb_wait(&sm.w0_empty[sw], (pw & 1u) ^ 1u);
                     mb_expect_tx(&sm.w0_full[sw], kW0Stage);
                     bulk_g2s(w0_ring + sw * kW0Stage, packed + (size_t)c * kW0Chunk, kW0Chunk, &sm.w0_full[sw]);
@@ -243,7 +249,7 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
                 mb_wait(&sm.d0_empty[buf], (((uint32_t)i >> 1) & 1u) ^ 1u);  // the layer group has drained D0[buf]
                 tc_fence_after();
                 const uint32_t d0 = tmem + kWsColD0 + buf * kColD0Stride;
-                for (int c = 0; c < kChunks; ++c) {
+                for (int c = 0; c < n_chunks; ++c) {
                     if (kBf16In) mb_wait(&sm.f_full[sa], pa & 1u);  // sa / pa walk the 5-stage TMA ring in this mode
                     else mb_wait(&sm.a_full[sa], pa & 1u);
                     mb_wait(&sm.w0_full[sw], pw & 1u);
@@ -285,7 +291,7 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
         }
     } else if (warp >= 4 && kBf16In) {
         // bf16-observation mode: no conversion stage; these warps only pull the packed weights into L2
-        for (int off = (tid - 128) * 128; off < kPackedBytes; off += 128 * 128) {
+        for (int off = (tid - 128) * 128; off < blob_bytes; off += 128 * 128) {
             asm volatile("prefetch.global.L2 [%0];" ::"l"(packed + off));
             if (kDual) asm volatile("prefetch.global.L2 [%0];" ::"l"(packed2 + off));
         }
@@ -298,7 +304,7 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
         // per scheduler -- which bounds the stream whenever the observation comes from L2 (the closed loop: 8.2 us per tile).
         const int half = warp >= 11 ? 1 : 0;
         const int row = half ? tid - kWsThreads : tid - 128;  // tile row
-        for (int off = (half * 128 + row) * 128; off < kPackedBytes; off += 256 * 128) {
+        for (int off = (half * 128 + row) * 128; off < blob_bytes; off += 256 * 128) {
             asm volatile("prefetch.global.L2 [%0];" ::"l"(packed + off));
             if (kDual) asm volatile("prefetch.global.L2 [%0];" ::"l"(packed2 + off));
         }
@@ -307,7 +313,7 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
         uint32_t pf = 0, pa = 0;
         int dbg_g = 0;
         for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-            for (int c = 0; c < kWsChunks; ++c) {
+            for (int c = 0; c < n_chunks; ++c) {
                 mb_wait(&sm.f_full[sf], pf & 1u);
                 if (tid == 128 && dbg_g < 128) PDBG(128 + dbg_g);
                 mb_wait(&sm.a_empty[sa], (pa & 1u) ^ 1u);
@@ -321,11 +327,11 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
                     const float4 lo = *reinterpret_cast<const float4*>(src + (((2 * plane) ^ sx) << 4));
                     const float4 hi = *reinterpret_cast<const float4*>(src + (((2 * plane + 1) ^ sx) << 4));
                     float v[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
-                    if (c == 0 || c == kWsChunks - 1) {  // encoder input = observation columns [3, 964) (models.py:95)
+                    if (c == 0 || c == n_chunks - 1) {  // encoder input = observation columns [3, 3 + R) (models.py:95)
 #pragma unroll
                         for (int j = 0; j < 8; ++j) {
                             const int col = c * kWsChunkK + plane * 8 + j;
-                            if (col < kEncInOffset || col >= kEncInOffset + kEncIn) v[j] = 0.f;
+                            if (col < kEncInOffset || col >= kEncInOffset + enc_in) v[j] = 0.f;
                         }
                     }
                     uint4 o;
@@ -358,7 +364,7 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
         // calls these
         auto load_w = [&](int net, int byte_offset, int bytes) {
             mb_expect_tx(&sm.w_full, (uint32_t)bytes);
-            bulk_g2s(sm.w, (kDual && net ? packed2 : packed) + byte_offset, (uint32_t)bytes, &sm.w_full);
+            bulk_g2s(sm.w, (kDual && net ? packed2 : packed) + w_shift + byte_offset, (uint32_t)bytes, &sm.w_full);
         };
         // D[128 x nn] (+)= A[planes plane0 ..] x W^T, k_steps MMAs of K = 16; then commit to acc_done.  The weight image in
         // the buffer has n_image rows per plane; the MMA uses rows n_row0 .. n_row0 + nn - 1 of it.
@@ -391,7 +397,7 @@ policy_forward_ws_kernel(const __grid_constant__ CUtensorMap obs_map, const floa
 #pragma unroll
                 for (int k = 0; k < kPer; ++k)
                     b[net][k] = tid + 128 * k < kWsBiasFloats
-                                    ? __ldg(reinterpret_cast<const float*>((kDual && net ? packed2 : packed) + kBiasOffset) + tid + 128 * k)
+                                    ? __ldg(reinterpret_cast<const float*>((kDual && net ? packed2 : packed) + w_shift + kBiasOffset) + tid + 128 * k)
                                     : 0.f;
 #pragma unroll
             for (int net = 0; net < kNets; ++net)
@@ -566,9 +572,10 @@ typedef CUresult (*WsEncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_
 // packed2 != nullptr: policy (`packed` -> mean [N, 2]) and value network (`packed2` -> value2 [N]) in one pass over the
 // observation (either dtype).
 // sample != nullptr (policy head): the pass also samples the actions (kSample).
+// enc_in: encoder width R (the callers check 1 <= R <= kEncInMax and obs_stride against it; blobs packed for R).
 int launch_policy_forward_ws(const void* obs, int obs_stride, int n_envs, const void* packed, float* mean,
                              bool value_head, bool bf16_in, cudaStream_t stream, const void* packed2, float* value2,
-                             const SampleArgs* sample) {
+                             const SampleArgs* sample, int enc_in) {
     static WsEncodeTiledFn encode = nullptr;
     static int n_sms = 0;
     constexpr int kSmemBytes = (int)sizeof(WsSmem) + 1024, kSmemBytesDual = (int)sizeof(WsSmemT<true>) + 1024;
@@ -605,10 +612,10 @@ int launch_policy_forward_ws(const void* obs, int obs_stride, int n_envs, const 
     tile_rows = ((tile_rows + 7) / 8) * 8;
     if (tile_rows > kTileM) tile_rows = kTileM;
     alignas(64) CUtensorMap map;
-    // fp32: columns [0, 965), the converter zeroes what lies outside [3, 964).  bf16: the tile is the MMA operand as
-    // it lands, so the map ends at column 964 (the ray the reference's slicing drops is zero-filled; columns 0..2 are
-    // finite and meet zero weights)
-    const cuuint64_t gdim[2] = {(cuuint64_t)(bf16_in ? kEncInOffset + kEncIn : kObsCols), (cuuint64_t)n_envs};
+    // fp32: columns [0, 4 + R), the converter zeroes what lies outside [3, 3 + R).  bf16: the tile is the MMA operand as
+    // it lands, so the map ends at column 3 + R (the ray the reference's slicing drops is zero-filled; columns 0..2 are
+    // finite and meet zero weights).  Beyond the map's end the tail chunk is zero-filled.
+    const cuuint64_t gdim[2] = {(cuuint64_t)(kEncInOffset + enc_in + (bf16_in ? 0 : 1)), (cuuint64_t)n_envs};
     const cuuint64_t gstride[1] = {(cuuint64_t)obs_stride * (bf16_in ? 2ull : 4ull)};
     const cuuint32_t box[2] = {(cuuint32_t)(bf16_in ? kBfChunkK : kWsChunkK), (cuuint32_t)tile_rows};
     const cuuint32_t estr[2] = {1u, 1u};
@@ -627,7 +634,7 @@ int launch_policy_forward_ws(const void* obs, int obs_stride, int n_envs, const 
         return launch_overlapped(kernel, dim3(grid), dim3(threads), (size_t)smem, stream, map, static_cast<const float*>(obs),
                                  obs_stride, n_envs, tile_rows, static_cast<const unsigned char*>(packed), mean,
                                  value_head ? 1 : 0, dual ? static_cast<const unsigned char*>(packed2) : no_net,
-                                 dual ? value2 : no_out, sa);
+                                 dual ? value2 : no_out, sa, enc_in);
     };
     if (dual && bf16_in && sample) ROVER_CUDA(launch(policy_forward_ws_kernel<true, true, true>, kWsThreads, kSmemBytesDual));
     else if (dual && bf16_in) ROVER_CUDA(launch(policy_forward_ws_kernel<true, true>, kWsThreads, kSmemBytesDual));

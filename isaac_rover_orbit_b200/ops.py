@@ -386,7 +386,11 @@ def height_scan_obs(pos_w: torch.Tensor, quat_w: torch.Tensor, rays, grid: ScanG
 def height_scan_encoder(pos_w: torch.Tensor, quat_w: torch.Tensor, rays, grid: ScanGridHandle, obs: torch.Tensor, net,
                         write_obs: bool = True, max_distance: float = 100.0, base_offset: float = 0.26878) -> torch.Tensor:
     """``height_scan_rover`` FUSED with the network's ``HeightmapEncoder`` (one launch): returns the encoder output
-    ``[N, 64]`` bf16 = ``[e(60), obs[:, 0:4]]``, the input of the MLP.  See ``height_scan_policy``."""
+    ``[N, 64]`` bf16 = ``[e(60), obs[:, 0:4]]``, the input of the MLP.  See ``height_scan_policy``.  The fused encoder
+    reads the 961-ray scan: a network with another ``encoder_input_size`` raises ``ValueError``."""
+    from .policy import _require_961
+
+    _require_961(net, "height_scan_encoder")
     if not isinstance(rays, RayPattern):
         rays = RayPattern(rays, pos_w.device)
     require_vertical("height_scan_encoder", rays)

@@ -14,6 +14,7 @@ they point into is owned by the Python handle objects of ``ops.py``.  Manager st
 from __future__ import annotations
 
 import ctypes as C
+import functools
 
 import torch
 from torch.library import Library
@@ -92,6 +93,10 @@ _SCHEMAS = {
     "policy_value_act_bf16": "(Tensor obs, Tensor packed_policy, Tensor packed_value, Tensor log_std, Tensor(a!) rng_state, "
                              "int env_offset, Tensor(b!) mean, Tensor(c!) value, Tensor(d!) actions, Tensor(e!) log_prob) -> ()",
     "action_noise": "(Tensor(a!) rng_state, int env_offset, int n_envs, bool advance) -> Tensor",
+    # ---- any of the forms above for encoder input width R (observations [N, 4 + R], fp32 or bf16)
+    "policy_pass": "(Tensor obs, int enc_in, Tensor packed, Tensor? packed_value, bool value_head, Tensor(a!) out, "
+                   "Tensor(b!)? value, Tensor? log_std, Tensor(c!)? rng_state, int env_offset, Tensor(d!)? actions, "
+                   "Tensor(e!)? log_prob) -> ()",
     # ---- PPO returns and advantages over the rollout memory (skrl PPO._update -> compute_gae)
     "ppo_gae": "(Tensor rewards, Tensor dones, Tensor values, Tensor last_values, float discount_factor, "
                "float lambda_coefficient, Tensor(a!) returns, Tensor(b!) advantages) -> ()",
@@ -443,6 +448,16 @@ def _stats_read(mailbox, world, out):
 
 # ----------------------------------------------------------------------------------------------------- policy
 def _policy_pack(weights, biases, packed):
+    # the blob's size follows W0's width (rover_policy_pack writes policy_packed_bytes(R) bytes): a shorter buffer would
+    # be written past its end.  (A width outside [1, 4092] is left to rover_policy_pack, which rejects it.)
+    r = int(weights[0].shape[1]) if len(weights) and weights[0].dim() == 2 else 0
+    if 1 <= r <= _lib.ENC_IN_MAX:
+        size = policy_packed_bytes(r)
+        if (not packed.is_cuda or packed.dtype != torch.uint8 or not packed.is_contiguous()
+                or packed.numel() < size):
+            raise RuntimeError(f"rover_b200::policy_pack: packed must be a contiguous CUDA uint8 tensor of at least {size} "
+                               f"bytes for an encoder input width of {r} (got {packed.numel() * packed.element_size()} "
+                               "bytes)")
     w = _lib.PolicyWeights()
     for l, (wt, bs) in enumerate(zip(weights, biases)):
         _f32("policy_pack", wt, bs)
@@ -487,17 +502,28 @@ def _scan_encoder_fused(pos_w, quat_w, ray_starts, pattern_box, grid, cells, max
 def _policy_mlp_forward(enc, packed, value_head):
     if enc.dtype != torch.bfloat16 or enc.dim() != 2 or enc.shape[1] != 64 or not enc.is_contiguous() or enc.data_ptr() % 128:
         raise RuntimeError("rover_b200::policy_mlp_forward: enc must be a contiguous bf16 [N,64] tensor, 128-byte aligned")
+    if packed.dtype != torch.uint8 or packed.numel() != policy_packed_bytes():
+        raise RuntimeError("rover_b200::policy_mlp_forward: packed must be the blob of a network with encoder input width "
+                           f"{_lib.ENC_IN} (uint8 [{policy_packed_bytes()}])")
     n = enc.shape[0]
     out = torch.empty(n, 1 if value_head else 2, dtype=torch.float32, device=enc.device)
     _lib.check(_lib.load().rover_policy_mlp_forward(_p(enc), n, _p(packed), _p(out), int(bool(value_head)), _stream(enc)))
     return out
 
 
-def policy_packed_bytes() -> int:
-    return int(_lib.load().rover_policy_pack(None, None, None))
+@functools.lru_cache(maxsize=None)
+def policy_packed_bytes(enc_in: int = _lib.ENC_IN) -> int:
+    """Bytes of the packed blob of a network with encoder input width ``enc_in`` (``rover_policy_pack``)."""
+    w = _lib.PolicyWeights()
+    w.in_dim[0] = _lib.check_enc_in(enc_in)
+    n = int(_lib.load().rover_policy_pack(C.byref(w), None, None))
+    if n < 0:
+        _lib.check(1)
+    return n
 
 
 def _policy_forward(obs, packed, value_head):
+    _packed_pair("policy_forward", obs, packed)
     n = obs.shape[0]
     out = torch.empty(n, 1 if value_head else 2, dtype=torch.float32, device=obs.device)
     if obs.dtype == torch.bfloat16:
@@ -517,6 +543,7 @@ def _policy_value_forward(obs, packed_policy, packed_value):
     if (obs.dtype != torch.float32 or obs.dim() != 2 or obs.shape[1] != 965 or obs.stride(1) != 1
             or obs.stride(0) % 4 != 0 or obs.data_ptr() % 16 != 0):
         raise RuntimeError("rover_b200::policy_value_forward: states must be fp32 [N,965] with 16-byte aligned rows")
+    _packed_pair("policy_value_forward", obs, packed_policy, packed_value)
     n = obs.shape[0]
     mean = torch.empty(n, 2, dtype=torch.float32, device=obs.device)
     value = torch.empty(n, 1, dtype=torch.float32, device=obs.device)
@@ -533,12 +560,13 @@ def _bf16_obs(what, obs):
         raise RuntimeError(f"rover_b200::{what}: bf16 states must be a [N,965] view from alloc_obs_bf16()")
 
 
-def _packed_pair(what, obs, packed_policy, packed_value):
+def _packed_pair(what, obs, *blobs):
+    """The blobs of the fixed-width operators: packed for R = 961 (policy_pack of a [80, 961] W0), on the states' device."""
     size = policy_packed_bytes()
-    for t in (packed_policy, packed_value):
+    for t in blobs:
         if not t.is_cuda or t.device != obs.device or t.dtype != torch.uint8 or t.numel() != size or not t.is_contiguous():
             raise RuntimeError(f"rover_b200::{what}: packed blobs must be contiguous uint8 [{size}] tensors on the states' "
-                               "device (policy_pack)")
+                               "device (policy_pack of an encoder input width of 961; other widths: policy_pass)")
 
 
 def _policy_value_forward_bf16(obs, packed_policy, packed_value):
@@ -579,7 +607,12 @@ def _act_checks(what, obs, log_std, rng_state, env_offset, mean, actions, log_pr
     elif (obs.dtype != torch.float32 or obs.dim() != 2 or obs.shape[1] != 965 or obs.stride(1) != 1
             or obs.stride(0) % 4 != 0 or obs.data_ptr() % 16 != 0):
         raise RuntimeError(f"rover_b200::{what}: states must be fp32 [N,965] with 16-byte aligned rows")
-    ts = [obs, log_std, rng_state, mean, actions, log_prob] + ([value] if value is not None else [])
+    return _sample_checks(what, obs, n, log_std, rng_state, env_offset, mean, actions, log_prob, value)
+
+
+def _sample_checks(what, obs, n, log_std, rng_state, env_offset, mean, actions, log_prob, value=None):
+    """The sampling tensors of an act operator (``log_prob`` may be None where the operator makes it optional)."""
+    ts = [t for t in (obs, log_std, rng_state, mean, actions, log_prob, value) if t is not None]
     if not all(t.is_cuda and t.device == obs.device for t in ts):
         raise RuntimeError(f"rover_b200::{what}: every tensor must be a CUDA tensor on the states' device")
     if rng_state.dtype != torch.int64 or rng_state.numel() != 2 or not rng_state.is_contiguous():
@@ -587,7 +620,8 @@ def _act_checks(what, obs, log_std, rng_state, env_offset, mean, actions, log_pr
     _f32(what, log_std, mean, actions, log_prob, value)
     if log_std.numel() != 2:
         raise RuntimeError(f"rover_b200::{what}: log_std must hold 2 values")
-    if mean.shape != (n, 2) or actions.shape != (n, 2) or log_prob.numel() != n or (value is not None and value.numel() != n):
+    if (mean.shape != (n, 2) or actions.shape != (n, 2) or (log_prob is not None and log_prob.numel() != n)
+            or (value is not None and value.numel() != n)):
         raise RuntimeError(f"rover_b200::{what}: mean / actions [N,2], log_prob [N]" + (", value [N]" if value is not None else "")
                            + " expected")
     if mean.data_ptr() % 8 or actions.data_ptr() % 8:
@@ -599,6 +633,7 @@ def _act_checks(what, obs, log_std, rng_state, env_offset, mean, actions, log_pr
 
 def _policy_act(obs, packed, log_std, rng_state, env_offset, mean, actions, log_prob):
     n = _act_checks("policy_act", obs, log_std, rng_state, env_offset, mean, actions, log_prob)
+    _packed_pair("policy_act", obs, packed)
     entry = _lib.load().rover_policy_act_bf16 if obs.dtype == torch.bfloat16 else _lib.load().rover_policy_act
     _lib.check(entry(_p(obs), int(obs.stride(0)), n, _p(packed), _p(log_std), _p(rng_state), int(env_offset), _p(mean),
                      _p(actions), _p(log_prob), _stream(obs)))
@@ -606,6 +641,7 @@ def _policy_act(obs, packed, log_std, rng_state, env_offset, mean, actions, log_
 
 def _policy_value_act(obs, packed_policy, packed_value, log_std, rng_state, env_offset, mean, value, actions, log_prob):
     n = _act_checks("policy_value_act", obs, log_std, rng_state, env_offset, mean, actions, log_prob, value)
+    _packed_pair("policy_value_act", obs, packed_policy, packed_value)
     _lib.check(_lib.load().rover_policy_value_act(_p(obs), int(obs.stride(0)), n, _p(packed_policy), _p(packed_value),
                                                   _p(log_std), _p(rng_state), int(env_offset), _p(mean), _p(value),
                                                   _p(actions), _p(log_prob), _stream(obs)))
@@ -617,6 +653,55 @@ def _policy_value_act_bf16(obs, packed_policy, packed_value, log_std, rng_state,
     _lib.check(_lib.load().rover_policy_value_act_bf16(_p(obs), int(obs.stride(0)), n, _p(packed_policy), _p(packed_value),
                                                        _p(log_std), _p(rng_state), int(env_offset), _p(mean), _p(value),
                                                        _p(actions), _p(log_prob), _stream(obs)))
+
+
+def _policy_pass(obs, enc_in, packed, packed_value, value_head, out, value, log_std, rng_state, env_offset, actions,
+                 log_prob):
+    """``rover_policy_pass``: obs ``[N, 4 + enc_in]`` fp32 (``alloc_obs`` layout) or bf16 (``alloc_obs_bf16``); ``out`` the
+    mean ``[N,2]`` (or the value ``[N]`` / ``[N,1]`` with ``value_head``); ``packed_value`` with ``value`` ``[N]`` / ``[N,1]``:
+    the value network in the same pass; ``log_std`` with ``rng_state``, ``actions`` (and optionally ``log_prob``): the
+    pass samples, as ``policy_act``."""
+    what = "rover_b200::policy_pass"
+    r = _lib.check_enc_in(enc_in)
+    bf16 = obs.dtype == torch.bfloat16
+    align = 8 if bf16 else 4
+    if (obs.dtype not in (torch.float32, torch.bfloat16) or obs.dim() != 2 or obs.shape[1] != 4 + r or obs.stride(1) != 1
+            or obs.stride(0) % align != 0 or obs.data_ptr() % 16 != 0):
+        raise RuntimeError(f"{what}: states must be fp32 or bf16 [N,{4 + r}] (4 + R columns, R = {r}) with 16-byte aligned "
+                           "rows (alloc_obs / alloc_obs_bf16)")
+    if not obs.is_cuda:
+        raise RuntimeError(f"{what}: states must be a CUDA tensor")
+    n = obs.shape[0]
+    size = policy_packed_bytes(r)
+    for t in (packed, packed_value):
+        if t is not None and (not t.is_cuda or t.device != obs.device or t.dtype != torch.uint8 or t.numel() != size
+                              or not t.is_contiguous()):
+            raise RuntimeError(f"{what}: packed blobs must be contiguous uint8 [{size}] tensors (packed for R = {r}) on the "
+                               "states' device")
+    if (packed_value is None) != (value is None):
+        raise RuntimeError(f"{what}: packed_value and value go together")
+    sample = log_std is not None or rng_state is not None or actions is not None
+    if sample:
+        if log_std is None or rng_state is None or actions is None or value_head:
+            raise RuntimeError(f"{what}: sampling needs log_std, rng_state and actions, and the policy head")
+        _sample_checks("policy_pass", obs, n, log_std, rng_state, env_offset, out, actions, log_prob, value)
+    elif log_prob is not None:
+        raise RuntimeError(f"{what}: log_prob is written only when sampling")
+    _f32("policy_pass", out, value)
+    if not all(t is None or (t.is_cuda and t.device == obs.device) for t in (out, value)):
+        raise RuntimeError(f"{what}: outputs must be CUDA tensors on the states' device")
+    if out.numel() != n * (1 if value_head else 2) or out.shape[0] != n or (value is not None and value.numel() != n):
+        raise RuntimeError(f"{what}: out must be [N,2] (mean) or [N] / [N,1] (value_head), value [N] / [N,1]")
+    if not value_head and out.data_ptr() % 8:  # the kernel stores each row's mean as one float2
+        raise RuntimeError(f"{what}: the mean output must be 8-byte aligned")
+    p = _lib.PolicyPass(obs=obs.data_ptr(), packed=packed.data_ptr(), out=out.data_ptr(),
+                        obs_dtype=_lib.OBS_BF16 if bf16 else _lib.OBS_FP32, stride=int(obs.stride(0)), n_envs=n, enc_in=r,
+                        value_head=int(bool(value_head)), env_offset=int(env_offset))
+    for name, t in (("packed_value", packed_value), ("value", value), ("log_std", log_std), ("rng_state", rng_state),
+                    ("actions", actions), ("log_prob", log_prob)):
+        if t is not None:
+            setattr(p, name, t.data_ptr())
+    _lib.check(_lib.load().rover_policy_pass(C.byref(p), _stream(obs)))
 
 
 def _action_noise(rng_state, env_offset, n_envs, advance):
@@ -720,6 +805,7 @@ _IMPLS = {
     "steep_mask": _steep_mask, "morph_box": _morph_box, "fill_holes": _fill_holes, "ppo_gae": _ppo_gae,
     "policy_act": _policy_act, "policy_value_act": _policy_value_act, "action_noise": _action_noise,
     "policy_value_forward_bf16": _policy_value_forward_bf16, "policy_value_act_bf16": _policy_value_act_bf16,
+    "policy_pass": _policy_pass,
 }
 for _name, _fn in _IMPLS.items():
     _IMPL.impl(_name, _fn)
@@ -815,7 +901,7 @@ def _fake_none(*args, **kwargs):
 for _name in ("height_scan_out", "ray_cast_out", "height_scan_obs", "height_scan_host", "ray_cast_obs", "ray_cast_host",
               "gaussian_act_out", "mdp_pre_step", "mdp_post_step", "mdp_step", "step_fused", "stats_read", "policy_pack",
               "policy_pack_fused", "mesh_to_heightmap", "ppo_gae", "policy_act", "policy_value_act",
-              "policy_value_act_bf16"):
+              "policy_value_act_bf16", "policy_pass"):
     torch.library.register_fake(f"{NS}::{_name}", _fake_none, lib=_DEF)
 
 OPS = tuple(_SCHEMAS)

@@ -137,16 +137,21 @@ class RolloutAgent(BaseAgent):
     (sampling + log-prob, SURVEY.md A.4) and ``record_transition`` = the ``RandomMemory`` rollout write.  The
     hooks the trainer calls around them exist and do what skrl's base ``Agent`` does (tracking), nothing more."""
 
-    def __init__(self, policy, memory: RolloutMemory | None = None, observation_size: int = 965, action_size: int = 2,
-                 value=None, action_out: torch.Tensor | None = None, action_rng=None):
+    def __init__(self, policy, memory: RolloutMemory | None = None, observation_size: int | None = None,
+                 action_size: int = 2, value=None, action_out: torch.Tensor | None = None, action_rng=None):
         """``value``: the PPO value network (``DeterministicNeuralNetwork``).  skrl's PPO evaluates it in
         ``record_transition`` on the states ``act`` just saw; here both networks run in ONE pass over the observation
         (``policy.policy_value_forward``) and the values are written to the memory's ``values`` tensor.
         ``action_rng`` (an ``ops.ActionRng``): the policy samples inside its forward pass with noise keyed on
         (seed, step, env) instead of ``torch.randn`` -- one launch per ``act``, policy and value together
         (``policy.policy_value_act``); without it ``act`` draws ``torch.randn`` as before.  fp32 states and the bf16 mirror
-        (``alloc_obs_bf16`` layout, what ``RoverEnv(observation_dtype=torch.bfloat16)`` returns) take the same routes."""
+        (``alloc_obs_bf16`` layout, what ``RoverEnv(observation_dtype=torch.bfloat16)`` returns) take the same routes.
+        ``observation_size``: the width of the memory's ``states``; by default ``4 + policy.encoder_input_size`` for a
+        policy that has one (965 for the shipped 961-ray scan), else 965."""
         super().__init__()
+        if observation_size is None:
+            r = getattr(policy, "encoder_input_size", None)
+            observation_size = 965 if r is None else 4 + int(r)
         self.policy = policy
         self.value = value
         self.action_rng = action_rng
@@ -222,10 +227,11 @@ class PPORolloutAgent(RolloutAgent):
     as in skrl 1.1.0: a truncated step bootstraps from the next row's value.  The optimisation epochs are not provided."""
 
     def __init__(self, policy, value, memory: RolloutMemory, discount_factor: float = 0.99, lambda_: float = 0.95,
-                 action_out: torch.Tensor | None = None, action_rng=None):
+                 action_out: torch.Tensor | None = None, action_rng=None, observation_size: int | None = None):
         if value is None or memory is None:
             raise ValueError("PPORolloutAgent needs a value network and a memory")
-        super().__init__(policy, memory, value=value, action_out=action_out, action_rng=action_rng)
+        super().__init__(policy, memory, observation_size=observation_size, value=value, action_out=action_out,
+                         action_rng=action_rng)
         self.discount_factor = float(discount_factor)
         self.lambda_ = float(lambda_)
         self._rollout = 0
